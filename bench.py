@@ -4,7 +4,8 @@
   python bench.py [--gpus N] [--steps K] [--warmup W] [--envs E] [--agents A] [--beams B]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
   python bench.py --impl reference ...      # the CPU arm: oracle port on all host cores
-  python bench.py --config c4|c5 ...        # BASELINE configs 4 / 5 (not the driver's line, which is C3)
+  python bench.py --config c4|c5 ...        # BASELINE configs 4 / 5 (the default is C3)
+  python bench.py --dump-outputs DIR ...    # also write what the last timed step returned, DIR/<name>.npy
 
 Workload (config C3 of BASELINE.json / SURVEY 8d): E = 4096 single-agent envs per GPU on the Shanghai map
 (2000x2000 cells, 0.06505 m), 1080-beam 270-degree lidar, RK4 single-track dynamics, start poses spread over
@@ -55,7 +56,11 @@ def parse():
                     "(a small first chunk starts the downloads sooner)")
     ap.add_argument("--pipe-chunks", type=int, default=4, help="env chunks of the e2e send/recv (cross-step pipelined) figure")
     ap.add_argument("--no-flush", action="store_true", help="do not flush L2 between timed steps")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the arrays the last timed step returned as DIR/<name>.npy "
+                    "(rank 0's envs; a seeded sample of them above 64 MiB, see dump_outputs)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if a.config == "c5":
         a.agents = 2
@@ -311,17 +316,20 @@ def main():
     stream = torch.cuda.current_stream(dev)
 
     def run(env, first, n, per_step_events=None, flush_buf=None):
+        """-> what the last of the n steps returned."""
+        result = None
         for k in range(first, first + n):
             if flush_buf is not None:
                 flush_buf.fill_(k & 0xFF)          # evict L2 (252 MiB written) before every timed step
             if per_step_events is not None:
                 per_step_events[k - first][0].record(stream)
             if ro is not None:
-                ro.step()
+                result = ro.step()
             else:
-                env.step(acts[k])
+                result = env.step(acts[k])
             if per_step_events is not None:
                 per_step_events[k - first][1].record(stream)
+        return result
 
     # ---- warm-up, then the timed region: K steps, device-timed per step so the flush is not counted
     run(env, 0, W, None, flush)
@@ -333,13 +341,15 @@ def main():
     launches0 = env.backend.kernel_launches
     torch.cuda.synchronize()
     t_wall0 = time.perf_counter()
-    run(env, W, K, ev, flush)
+    last = run(env, W, K, ev, flush)
     torch.cuda.synchronize()
     t_wall = time.perf_counter() - t_wall0
     launches = env.backend.kernel_launches - launches0
     step_ms = [a.elapsed_time(b) for a, b in ev]
     dev_ms = float(sum(step_ms))
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last, torch)       # before kernel_breakdown steps this env again
     if world > 1:
         dist.barrier()
         t = torch.tensor([dev_ms], dtype=torch.float64, device=dev)
@@ -461,6 +471,34 @@ def main():
     }
     emit(line)
     return 0
+
+
+DUMP_BYTES = 64 * 10 ** 6      # all files of a dump together, headers included
+NPY_HEADER_BYTES = 4096        # bound on one .npy header (128 bytes for the short shapes written here)
+
+
+def dump_outputs(directory, result, torch):
+    """One step's return value -- (obs, reward, terminated, truncated, info) of F110VecEnv.step or DeviceRollout.step -- as
+    <directory>/<name>.npy: obs, reward, terminated, truncated and every other tensor of info, float64 where the step
+    computes float64, float32 otherwise.  Rows are envs.  When all of them would exceed DUMP_BYTES, a sample of envs drawn
+    from a fixed seed is kept instead, so that two builds run with the same arguments write the same rows;
+    env_index.npy names the rows written."""
+    obs, reward, terminated, truncated, info = result
+    arrays = dict(obs=obs, reward=reward, terminated=terminated, truncated=truncated)
+    arrays.update((k, v) for k, v in info.items() if k not in arrays)
+    n = obs.shape[0]
+    row_bytes = 8 + sum((8 if v.dtype == torch.float64 else 4) * (v.numel() // n) for v in arrays.values())
+    budget = DUMP_BYTES - NPY_HEADER_BYTES * (len(arrays) + 1)
+    rows = np.arange(n)
+    if n * row_bytes > budget:
+        rows = np.sort(np.random.default_rng(0).choice(n, budget // row_bytes, replace=False))
+    idx = torch.from_numpy(rows).to(obs.device)
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "env_index.npy"), rows.astype(np.float64))
+    for k, v in arrays.items():
+        v = v.index_select(0, idx)
+        v = v if v.dtype == torch.float64 else v.to(torch.float32)
+        np.save(os.path.join(directory, k + ".npy"), v.cpu().numpy())
 
 
 def kernel_breakdown(env, acts, first, n, flush, torch):

@@ -1,8 +1,8 @@
 """Generate the committed golden fixtures from the UNMODIFIED reference.
 
-Run in the build container only (needs /root/reference):  python tests/golden/make_golden.py
-Writes tests/golden/*.npz.  The fixtures are what travels to the GPU box; nothing under
-tests/ reads /root/reference at test time.
+Needs a checkout of the reference:  F110_REFERENCE_ROOT=<dir> python tests/golden/make_golden.py
+Writes tests/golden/*.npz.  The tests read these fixtures; only the optional differential
+tests read the reference itself.
 
 What is recorded
   maps.npz         binarised occupancy (bit-packed, after the reference's flip+threshold,
@@ -231,13 +231,14 @@ def make_reward_golden():
                                           wall_quantile=0.05)   # defaults otherwise: exercises lead / bubble / flank terms
     cl = np.loadtxt(csv, delimiter=',', comments='#')
     rng = np.random.default_rng(21)
-    obs_all, rew_all, rew2_all, first = [], [], [], []
+    obs_all, rew_all, rew2_all, first, acts_all, poses_all = [], [], [], [], [], []
     for ep, (i0, gap, kspeed) in enumerate([(0, 30, 1.6), (2500, 14, 1.2), (5200, 9, 2.2), (900, 12, 0.8)]):
         def pose(i):
             j = (i + 1) % len(cl)
             return [cl[i, 0], cl[i, 1], np.arctan2(cl[j, 1] - cl[i, 1], cl[j, 0] - cl[i, 0])]
         rfn.reset(); rfn2.reset()
-        obs, info = env.reset(options=np.array([pose(i0), pose((i0 + gap) % len(cl))], np.float32))
+        poses_all.append(np.array([pose(i0), pose((i0 + gap) % len(cl))], np.float32).astype(np.float64))
+        obs, info = env.reset(options=poses_all[-1])
         for t in range(260):
             ego = gap_follow_action(info['scans'][0]).astype(np.float32)
             ego[1] *= kspeed
@@ -245,14 +246,19 @@ def make_reward_golden():
             if ep == 3 and t > 120:
                 ego[0] = np.float32(0.35)        # drive it into the wall: crash penalty path
             opp = gap_follow_action(info['scans'][1]).astype(np.float32)
-            obs, _, term, trunc, info = env.step(np.stack([ego, opp]).astype(np.float32))
+            acts_all.append(np.stack([ego, opp]).astype(np.float32))
+            obs, _, term, trunc, info = env.step(acts_all[-1])
             obs_all.append(obs.copy()); rew_all.append(float(rfn(obs))); rew2_all.append(float(rfn2(obs)))
             first.append(1 if t == 0 else 0)
             if term and t > 150:
                 break
-    np.savez_compressed(os.path.join(HERE, 'reward.npz'), obs=np.stack(obs_all), reward=np.array(rew_all),
-                        reward_alt=np.array(rew2_all), episode_start=np.array(first, np.uint8),
-                        centerline=cl, s=P.s, L=np.float64(P.L))
+    # the observations themselves (3 MB of noisy scans) are not stored: tests/helpers.py:reward_recording replays the
+    # rollout from its poses, actions and noise seed (F110Env's default, 42) and checks each against its SHA-256
+    sha = np.stack([np.frombuffer(hashlib.sha256(np.ascontiguousarray(o, np.float32).tobytes()).digest(), np.uint8)
+                    for o in obs_all])
+    np.savez_compressed(os.path.join(HERE, 'reward.npz'), actions=np.stack(acts_all), poses=np.stack(poses_all),
+                        seed=np.int64(42), obs_sha256=sha, reward=np.array(rew_all), reward_alt=np.array(rew2_all),
+                        episode_start=np.array(first, np.uint8), centerline=cl)
     print('reward.npz', len(rew_all), 'steps; reward range', min(rew_all), max(rew_all), 'alt', min(rew2_all), max(rew2_all))
 
 

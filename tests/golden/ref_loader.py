@@ -1,9 +1,8 @@
 """Loader for the UNMODIFIED reference (test infrastructure only).
 
-Works only where /root/reference exists (the build container).  Nothing that runs on the
-GPU box imports this module: it is used by ``make_golden.py`` to generate the committed
-fixtures and by the optional ``-m "not gpu"`` differential tests (skipped when the reference
-tree is absent).
+Works only where the environment variable F110_REFERENCE_ROOT names a checkout of the
+reference.  It is used by ``make_golden.py`` to generate the committed fixtures and by the
+optional differential tests (skipped when F110_REFERENCE_ROOT is unset).
 
 The reference imports ``gymnasium`` and ``pyglet`` at module top
 (f110_gymnasium/gym/f110_gym/envs/f110_env.py:27-45, f110_gym/__init__.py:1); neither is
@@ -14,13 +13,13 @@ import os
 import sys
 import types
 
-REF_ROOT = os.environ.get("F110_REFERENCE_ROOT", "/root/reference")
+REF_ROOT = os.environ.get("F110_REFERENCE_ROOT", "")
 REF_GYM = os.path.join(REF_ROOT, "f110_gymnasium", "gym")
 REF_MAPS = os.path.join(REF_ROOT, "rl_training", "maps") + "/"
 
 
 def reference_available():
-    return os.path.isdir(os.path.join(REF_GYM, "f110_gym", "envs"))
+    return bool(REF_ROOT) and os.path.isdir(os.path.join(REF_GYM, "f110_gym", "envs"))
 
 
 def _install_stubs():
@@ -60,8 +59,11 @@ def _install_stubs():
 
 def load_reference():
     """Return a namespace with the reference's own classes / njit kernels."""
+    if not REF_ROOT:
+        raise SystemExit("set F110_REFERENCE_ROOT to a checkout of the reference (the directory holding f110_gymnasium/ "
+                         "and rl_training/)")
     if not reference_available():
-        raise RuntimeError("reference tree not present at %s" % REF_ROOT)
+        raise SystemExit("F110_REFERENCE_ROOT=%s holds no f110_gymnasium/gym/f110_gym/envs" % REF_ROOT)
     os.environ.setdefault("NUMBA_CACHE_DIR", "/tmp/f110_numba_cache")
     _install_stubs()
     if REF_GYM not in sys.path:

@@ -85,6 +85,36 @@ def noise_stream(seed, steps, beams=1080, expect_sha=None):
     return out
 
 
+@functools.lru_cache(maxsize=None)
+def reward_recording():
+    """reward.npz with its flat observations 'obs' [T, 1088] f32.  The file keeps what the recorded reference rollout was
+    driven with (start poses per episode, the actions applied, the lidar noise seed) and the SHA-256 of every observation
+    the reference returned; the oracle, whose env reproduces the reference's bit for bit (test_env_rollouts), replays the
+    rollout here and every observation must hash to the recorded one."""
+    from oracle.f110_oracle import Oracle
+    g = dict(load('reward'))
+    o = Oracle(1, 2)
+    s, c, a, bc, sd = tables()
+    o.set_tables(s, c)
+    o.set_beam_tables(a, bc, sd)
+    o.set_map_arrays(*golden_map('Shanghai_map'))
+    obs, episode = [], -1
+    for k in range(len(g['actions'])):
+        if g['episode_start'][k]:
+            # F110Env.reset restarts the noise stream of every agent and draws one scan (the reset observation)
+            episode += 1
+            rng = np.random.default_rng(int(g['seed']))
+            nz = rng.normal(0., 0.01, size=1080)
+            o.reset(g['poses'][episode][None], noise=np.stack([nz, nz])[None])
+        nz = rng.normal(0., 0.01, size=1080)
+        ob = np.array(o.step(g['actions'][k][None], noise=np.stack([nz, nz])[None])['obs'][0], np.float32)   # a copy
+        assert hashlib.sha256(ob.tobytes()).digest() == g['obs_sha256'][k].tobytes(), \
+            ("replayed observation differs from the reference's", k)
+        obs.append(ob)
+    g['obs'] = np.stack(obs)
+    return g
+
+
 ROLLOUT_MAP = {
     'rollout_c2_shanghai': 'Shanghai_map', 'rollout_const_shanghai': 'Shanghai_map',
     'rollout_circles_open': 'open_square', 'rollout_headon_open': 'open_square',

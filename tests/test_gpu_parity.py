@@ -449,7 +449,8 @@ def test_constructor_parameters_vs_oracle(kw):
 
 def test_per_agent_params_vs_oracle():
     """update_params on one agent (heavier, longer, wider car; the oracle is pinned to the reference for this in
-    test_reference_differential): dynamics and ray-cast use the agent's parameters, GJK the Simulator's."""
+    test_reference_differential, and to its recording in test_differential_golden): dynamics and ray-cast use the
+    agent's parameters, GJK the Simulator's."""
     from oracle.f110_oracle import DEFAULT_PARAMS
     N, A = 16, 3
     p1 = dict(DEFAULT_PARAMS)
@@ -894,7 +895,7 @@ def test_consumers_survive_non_finite_inputs():
     torch = _torch()
     from f110_gymnasium_ros2_jazzy_b200 import ShapedReward, gap_follow_actions
     from tests.test_oracle_golden import REWARD_KW
-    g, r = H.load('gap_follow'), H.load('reward')
+    g, r = H.load('gap_follow'), H.reward_recording()
     scans = g['scans'][:64].copy()
     bad = scans.copy()
     bad[5] = np.nan
@@ -1132,7 +1133,7 @@ def test_shaped_reward_kernel_matches_reference_and_oracle(form, monkeypatch):
     from f110_gymnasium_ros2_jazzy_b200 import ShapedReward
     from oracle.f110_oracle import RewardOracle
     from tests.test_oracle_golden import REWARD_ALT_KW, REWARD_KW
-    g = H.load('reward')
+    g = H.reward_recording()
     obs, starts = g['obs'], g['episode_start']
     T = len(obs)
     for kw, key in ((REWARD_KW, 'reward'), (REWARD_ALT_KW, 'reward_alt')):

@@ -154,6 +154,34 @@ def test_bench_reference_arm_runs_on_cpu():
     assert line['cpu_baseline']['kind'] == 'port' and line['e2e']['h2d_bytes_per_step'] == 0
 
 
+def test_bench_dump_outputs_writes_every_returned_array(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: each array of a step's return value as <name>.npy, float64 kept, the rest as float32, and
+    above the size cap the same seeded sample of envs from every array, named by env_index.npy."""
+    import torch
+    import bench
+    n = 50
+    obs, rew = torch.rand((n, 12)), torch.rand(n)
+    term, trunc = (torch.arange(n) % 3 == 0).to(torch.uint8), torch.zeros(n, dtype=torch.uint8)
+    info = {'obs': obs, 'reward': rew, 'terminated': term, 'state': torch.rand((n, 2, 7), dtype=torch.float64),
+            'toggles': torch.arange(2 * n, dtype=torch.int32).reshape(n, 2)}
+    bench.dump_outputs(str(tmp_path / 'all'), (obs, rew, term, trunc, info), torch)
+    got = {f[:-4]: np.load(str(tmp_path / 'all' / f)) for f in os.listdir(str(tmp_path / 'all'))}
+    assert sorted(got) == ['env_index', 'obs', 'reward', 'state', 'terminated', 'toggles', 'truncated']
+    assert got['state'].dtype == np.float64 and np.array_equal(got['state'], info['state'].numpy())
+    assert got['toggles'].dtype == np.float32 and np.array_equal(got['toggles'], info['toggles'].numpy())
+    assert np.array_equal(got['terminated'], term.numpy()) and np.array_equal(got['env_index'], np.arange(n))
+    row = 8 + 4 * 12 + 4 + 4 + 4 + 8 * 14 + 4 * 2
+    cap = 20 * row + 7 * bench.NPY_HEADER_BYTES           # 7 files
+    monkeypatch.setattr(bench, 'DUMP_BYTES', cap)
+    for d in ('a', 'b'):
+        bench.dump_outputs(str(tmp_path / d), (obs, rew, term, trunc, info), torch)
+    keep = np.load(str(tmp_path / 'a' / 'env_index.npy')).astype(int)
+    assert len(keep) == 20 and np.array_equal(keep, np.load(str(tmp_path / 'b' / 'env_index.npy')))
+    assert sum(os.path.getsize(str(tmp_path / 'a' / f)) for f in os.listdir(str(tmp_path / 'a'))) <= cap
+    assert np.array_equal(np.load(str(tmp_path / 'a' / 'obs.npy')), obs.numpy()[keep])
+    assert np.array_equal(np.load(str(tmp_path / 'a' / 'state.npy')), info['state'].numpy()[keep])
+
+
 def test_bind_host_to_gpu_uses_the_gpus_numa_node(tmp_path):
     """bind_host_to_gpu reads <sysfs>/bus/pci/devices/<id>/numa_node and node<N>/cpulist; here against a fake sysfs."""
     import os
@@ -213,6 +241,11 @@ def test_device_replay_buffer_ring_and_per_formulas():
         small.sample()
     small.add(*batch(2, 1))
     assert small.sample()[0].shape == (4,)                    # fewer than a batch stored: with replacement
+    # clamping (replay_buffer.py:120-135): +inf -> float32 max, tiny -> 1e-8; the probabilities stay finite
+    small.update_priorities([0, 1], [float('inf'), 1e-12])
+    assert float(small.priority[0]) == np.finfo(np.float32).max and float(small.priority[1]) == float(np.float32(1e-8))
+    p = small.probabilities().numpy()
+    assert np.isfinite(p).all() and abs(p.sum() - 1.0) < 1e-12 and p[0] > 0.999
 
 
 def test_f110_gym_alias_resolves_like_gymnasium():

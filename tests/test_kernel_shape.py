@@ -4,19 +4,22 @@ DESIGN.md section 3 rests on properties of the generated code that a harmless-lo
 test failing: the hot loop of the ray-march must contain no call (5 % of the kernel, DESIGN section 9) and no local-memory
 traffic and stay short (it is the dependent chain of every lookup), and the kernel must fit the 40 registers that keep 12
 CTAs of 128 threads resident per SM (32 for the 16-CTA variant)."""
+import os
 import re
 import shutil
 import subprocess
 
 import pytest
+from torch.utils.cpp_extension import CUDA_HOME
 
 from f110_gymnasium_ros2_jazzy_b200 import _lib
 
-pytestmark = pytest.mark.skipif(shutil.which("cuobjdump") is None, reason="cuobjdump not on PATH")
+CUOBJDUMP = shutil.which("cuobjdump") or (CUDA_HOME and shutil.which("cuobjdump", path=os.path.join(CUDA_HOME, "bin")))
+pytestmark = pytest.mark.skipif(not CUOBJDUMP, reason="cuobjdump neither on PATH nor under CUDA_HOME")
 
 
 def _functions(args):
-    out = subprocess.check_output(["cuobjdump"] + args + [_lib.LIB_PATH], stderr=subprocess.DEVNULL).decode()
+    out = subprocess.check_output([CUOBJDUMP] + args + [_lib.LIB_PATH], stderr=subprocess.DEVNULL).decode()
     fns, name = {}, None
     for line in out.splitlines():
         m = re.search(r"Function\s*:?\s*(\S+)", line)

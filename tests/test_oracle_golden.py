@@ -189,7 +189,7 @@ def test_shaped_reward_oracle_matches_reference():
     """rewards.py:185-355 + track_progress.py over 754 recorded steps (4 episodes incl. a crash), two parameter sets:
     within 1e-12 of the reference's float (BLAS dots / libm ulps), and the float32 quantile path bit-exact."""
     from oracle.f110_oracle import RewardOracle
-    g = H.load('reward')
+    g = H.reward_recording()
     for kw, key in ((REWARD_KW, 'reward'), (REWARD_ALT_KW, 'reward_alt')):
         o = RewardOracle(1, g['centerline'], **kw)
         got = np.array([o(g['obs'][k], np.array([g['episode_start'][k]], np.uint8))[0] for k in range(len(g[key]))])

@@ -1,5 +1,5 @@
-"""Differential tests of the oracle against the LIVE reference (only where /root/reference exists, i.e. the build
-container; skipped on the GPU box).  The committed golden fixtures pin fixed scenarios; these draw fresh ones."""
+"""Differential tests of the oracle against the LIVE reference (only where F110_REFERENCE_ROOT names a checkout of it;
+skipped otherwise).  The committed golden fixtures pin fixed scenarios; these draw fresh ones."""
 import os
 import sys
 import warnings
@@ -10,7 +10,7 @@ import pytest
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden'))
 from ref_loader import REF_MAPS, fresh_statics, load_reference, reference_available  # noqa: E402
 
-pytestmark = pytest.mark.skipif(not reference_available(), reason="reference tree not present")
+pytestmark = pytest.mark.skipif(not reference_available(), reason="F110_REFERENCE_ROOT does not name a checkout of the reference")
 
 
 @pytest.fixture(scope="module")

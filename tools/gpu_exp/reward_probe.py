@@ -3,7 +3,7 @@ import numpy as np, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
 from f110_gymnasium_ros2_jazzy_b200 import ShapedReward
 from tests import helpers as H
-g = H.load('reward')
+g = H.reward_recording()
 N = 8192
 obs = torch.from_numpy(g['obs'][np.arange(N) % len(g['obs'])]).cuda().contiguous()
 rw = ShapedReward(N, g['centerline'], w_prog=5.0, alive_bonus=0.5, grace_steps_wall=25, grace_steps_opp=175, wall_quantile=0.10)
