@@ -98,7 +98,7 @@ void layout_state(Arena& a, SimState& st, int N, int NA) {
     st.near_start = a.take<uint8_t>(NA); st.collisions = a.take<uint8_t>(NA);
 }
 
-void layout_scratch(Arena& a, StepScratch& sc, int NA, int B, bool timeline) {
+void layout_scratch(Arena& a, StepScratch& sc, int NA, int B, bool timeline, unsigned homes) {
     sc.scan_x = a.take<double>(NA); sc.scan_y = a.take<double>(NA); sc.pre_yaw = a.take<double>(NA);
     sc.head = a.take<double>((size_t)NA * 4);
     sc.ttc_hit = a.take<int32_t>(NA);
@@ -108,11 +108,16 @@ void layout_scratch(Arena& a, StepScratch& sc, int NA, int B, bool timeline) {
     // capacities of the three heavy-unit lists (classes >= 96 / 48 / 24 lookups); a list that overflows sends the rest of
     // its class to the light region, which costs order, never correctness
     sc.cap[0] = sc.num_units / 16 + 8; sc.cap[1] = sc.num_units / 8 + 8; sc.cap[2] = sc.num_units / 4 + 8;
-    sc.ctrl = a.take<unsigned>(F110_CTRL_WORDS);
+    // home segments of equal size (the last may be short), none empty
+    homes = homes < 1u ? 1u : (homes > sc.num_units ? sc.num_units : homes);
+    sc.seg_units = (sc.num_units + homes - 1u) / homes;
+    sc.homes = (sc.num_units + sc.seg_units - 1u) / sc.seg_units;
+    sc.ctrl = a.take<unsigned>(ctrl_words(sc.homes));
     const size_t ncap = (size_t)sc.cap[0] + sc.cap[1] + sc.cap[2];
     sc.list[0] = a.take<unsigned>(ncap); sc.list[1] = a.take<unsigned>(ncap);
     sc.cls[0] = a.take<unsigned>(sc.num_units); sc.cls[1] = a.take<unsigned>(sc.num_units);
     sc.timeline = (timeline && sc.num_units <= (1u << 22)) ? a.take<uint4>(sc.num_units) : nullptr;
+    sc.home_of_sm = a.take<unsigned>(F110_SMID_TABLE);
 }
 
 FastDiv make_fast_div(uint32_t d) {
@@ -224,8 +229,24 @@ int f110_create(const F110Config* cfg, const double* params, F110Sim** out) {
     Arena measure;
     layout_state(measure, sim->st, N, NA);
     sim->state_bytes = (measure.used + 255) & ~size_t(255);
+    // Longest-first order for launches of up to 48 units per resident warp; larger ones get home segments, one per SM
+    // (F110_LIDAR_HOMES=n forces n segments, and natural order with them).  SM ids are not contiguous, so a wave of probe
+    // CTAs finds the ones in use and home k goes to the SMs of rank k * homes / SMs.
+    unsigned char seen[F110_SMID_TABLE];
+    if (probe_sm_ids(seen) != cudaSuccess) {
+        cudaGetLastError();
+        delete sim;
+        return fail(F110_ERR_CUDA, "cannot probe the device's SM ids");
+    }
+    unsigned nsm = 0;
+    for (int k = 0; k < F110_SMID_TABLE; ++k) nsm += seen[k];
+    if (nsm == 0) { delete sim; return fail(F110_ERR_CUDA, "the SM id probe saw no SM"); }
+    const size_t units = (size_t)NA * ((B + 31) / 32);
+    bool ordered = units <= (size_t)48 * 4 * (size_t)sim->lidar_blocks;
+    unsigned homes = ordered ? 1u : nsm;
+    { const char* h = getenv("F110_LIDAR_HOMES"); if (h && atoi(h) > 0) { homes = (unsigned)atoi(h); ordered = ordered && homes == 1u; } }
     Arena measure2;
-    layout_scratch(measure2, sim->sc, NA, B, sim->count_lookups);
+    layout_scratch(measure2, sim->sc, NA, B, sim->count_lookups, homes);
     sim->scratch_bytes = (measure2.used + 255) & ~size_t(255);
     const size_t ntab = (size_t)A * F110_NUM_PARAMS + F110_NUM_PARAMS + 2 * (size_t)cfg->theta_dis + 3 * (size_t)B;
 
@@ -252,13 +273,19 @@ int f110_create(const F110Config* cfg, const double* params, F110Sim** out) {
         return F110_ERR_CUDA;
     }
     Arena a; a.base = sim->state_blob; layout_state(a, sim->st, N, NA);
-    Arena b; b.base = sim->scratch_blob; layout_scratch(b, sim->sc, NA, B, sim->count_lookups);
-    sim->sc.ordered = (size_t)sim->sc.num_units <= (size_t)48 * 4 * (size_t)(sim->lidar_blocks > 0 ? sim->lidar_blocks : 1) ? 1u : 0u;
+    Arena b; b.base = sim->scratch_blob; layout_scratch(b, sim->sc, NA, B, sim->count_lookups, homes);
+    sim->sc.ordered = ordered ? 1u : 0u;
     // before the first step no unit is on a list: every unit is class 3 (light, natural order)
     {
         const std::vector<unsigned> light(sim->sc.num_units, 3u);
         e = cudaMemcpy(sim->sc.cls[0], light.data(), light.size() * sizeof(unsigned), cudaMemcpyHostToDevice);
         if (e == cudaSuccess) e = cudaMemcpy(sim->sc.cls[1], light.data(), light.size() * sizeof(unsigned), cudaMemcpyHostToDevice);
+        std::vector<unsigned> table(F110_SMID_TABLE);
+        for (unsigned k = 0, rank = 0; k < F110_SMID_TABLE; ++k) {
+            table[k] = seen[k] ? (unsigned)((size_t)rank * sim->sc.homes / nsm) : k % sim->sc.homes;
+            rank += seen[k];
+        }
+        if (e == cudaSuccess) e = cudaMemcpy((void*)sim->sc.home_of_sm, table.data(), table.size() * sizeof(unsigned), cudaMemcpyHostToDevice);
     }
     if (e != cudaSuccess) {
         fail(F110_ERR_CUDA, "scratch initialisation failed: %s", cudaGetErrorString(e));

@@ -501,6 +501,14 @@ constexpr unsigned LIDAR_CHUNK = LIDAR_CHUNK_OVERRIDE;   // queue positions a wa
 // * The queue is one atomic counter (same-address atomics retire at about one per ns on this part: one fetch per unit
 //   costs 45 % at 32 768 envs); a fetch takes up to LIDAR_CHUNK positions at a time in the bulk of the light region, one
 //   near the ends, and is issued after the march of the chunk's last unit, so that its latency hides behind the epilogue.
+// * Home segments, in launches without the longest-first order (more than 48 units per resident warp).  The units are cut
+//   into sc.homes contiguous segments, one per SM, each with its own counter; a warp serves the segment of its SM (%smid
+//   through sc.home_of_sm) and, once that is drained, the nearest one that is not (home + 1, home - 1, home + 2, ...: 32
+//   looked at per round trip), and ends when every segment is drained.  Env order is track order (workloads.start_poses;
+//   auto-reset returns a car to its own start), so the cars of a segment see the same walls and the map lines its warps
+//   march stay in the SM's L1 (tools/locality_study.py).  Where the CTAs land only changes the order.  With one segment
+//   the queue is the one above.  Smaller launches keep one: a warp's first position then costs no fetch, and at the end
+//   no warp looks through other segments (DESIGN.md section 9).
 // MODE 0: opponents follow (A >= 2); 1: single agent, the scan goes straight to the outputs; 2: single agent and the float32
 // observation is the only scan output, noise from the device stream, no mask of active envs -- the bulk throughput case
 // (BASELINE configs 3 / 4) -- without the unit's tests and address arithmetic for what is not there; 3: opponents, likewise
@@ -522,14 +530,16 @@ lidar_kernel(const __grid_constant__ SimConst c, const __grid_constant__ MapView
     const unsigned done = 4u + ((epoch >> 1) & 1u);
     // list ends (K1 may have pushed the third count past its capacity)
     const unsigned n0 = sc.ctrl[CTRL_CUR], n1 = n0 + sc.ctrl[CTRL_CUR + 1], n2 = n1 + min(sc.ctrl[CTRL_CUR + 2], sc.cap[2]);
-    const unsigned npos = n2 + sc.num_units;
     const unsigned cap0 = sc.cap[0], cap1 = sc.cap[1], cap2 = sc.cap[2];
     const unsigned* __restrict__ cur_list = sc.list[par];
     unsigned* cur_cls = sc.cls[par];
     unsigned* __restrict__ next_list = sc.list[par ^ 1u];
     unsigned* __restrict__ next_cls = sc.cls[par ^ 1u];
-    unsigned* qpos = sc.ctrl + CTRL_POS;
     unsigned cnt_look = 0, cnt_rays = 0, cnt_max = 0, cnt_redone = 0;
+
+    // The segment the warp serves and the end of its positions: the heavy lists (one segment only), then its units.
+    unsigned g = 0, npos = 0;
+    auto seg_end = [&](unsigned seg) { return n2 + min(sc.seg_units, sc.num_units - seg * sc.seg_units); };
 
     // position -> unit: an entry of list b, valid if b is still the unit's class (a unit can have been entered on a lighter
     // list before a neighbour raised it to a heavier one), or, in the light region, the unit itself if its class is light
@@ -541,28 +551,78 @@ lidar_kernel(const __grid_constant__ SimConst c, const __grid_constant__ MapView
             unit = cur_list[k];
             skip = cur_cls[unit] != b;
         } else if (p < npos) {
-            unit = p - n2;
+            unit = g * sc.seg_units + (p - n2);
             skip = false;
             if (sc.ordered) { const unsigned v = cur_cls[unit]; skip = v < 3u || v == done; }
         }
     };
 
-    // the first position of every warp is its own index: the counter starts at 0 and a fetch returns old + nwarps
-    unsigned pos = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, end = pos + 1u;
     unsigned f = 0, take = 1u;
     // guided self-scheduling: half of an even share of what is left, between LIDAR_MIN_TAKE and LIDAR_CHUNK positions; one at a
     // time in the heavy lists, where a unit is long and balance matters most.  Not one at a time at the end of the light
     // region: a fetch is an L2 atomic's round trip plus the class lookup behind it (1.9 us when every unit pays it: unit
     // timeline with LIDAR_CHUNK 1), a light unit is 3.3 us, and all 7 104 warps asking after every unit is more than the
     // one counter serves (about 1.4 fetches per ns) -- two at a time costs 1.6 us of balance and was 3 % faster at 4096 envs.
+    // with one segment the first position of every warp is its own index: the counter starts at 0 and a fetch returns
+    // old + nwarps; with several, a warp's first position is a fetch from its home
+    const bool one = sc.homes == 1u;
+    const unsigned share = one ? nwarps : max(nwarps / sc.homes, 1u);     // warps per segment
     auto fetch = [&](unsigned at) {
-        take = (npos - at) / (2u * nwarps);
+        take = (npos - at) / (2u * share);
         take = at < n1 ? 1u : at < n2 ? LIDAR_LIST2_TAKE : take < LIDAR_MIN_TAKE ? LIDAR_MIN_TAKE : (take > (sc.ordered ? LIDAR_CHUNK : 2u * LIDAR_CHUNK) ? (sc.ordered ? LIDAR_CHUNK : 2u * LIDAR_CHUNK) : take);
-        if (lane == 0) f = atomicAdd(qpos, take) + nwarps;
+        if (lane == 0) f = atomicAdd(sc.ctrl + CTRL_SEG + g * SEG_STRIDE, take) + (one ? nwarps : 0u);
     };
+    unsigned pos, end;
+    // The warp's segment is drained: claim a chunk of the nearest segment that is not, in the order home, home + 1,
+    // home - 1, home + 2, ...; false once every segment is drained (counters only grow, so that is final).
+    auto steal = [&]() -> bool {
+        const unsigned Q = sc.homes;
+        if (Q == 1u) return false;                 // the one queue's fetch has just come back empty
+        unsigned smid;
+        asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
+        const unsigned h = sc.home_of_sm[smid & (F110_SMID_TABLE - 1u)];
+        for (;;) {
+            bool found = false;
+            for (unsigned v0 = 0; v0 < Q && !found; v0 += 32u) {
+                const unsigned v = v0 + lane, off = (v + 1u) >> 1;
+                unsigned seg = (v & 1u) ? h + off : h + Q - off, at = 0u;
+                seg = seg >= Q ? seg - Q : seg;
+                bool open = false;
+                if (v < Q) { at = __ldcg(sc.ctrl + CTRL_SEG + seg * SEG_STRIDE); open = at < seg_end(seg); }
+                const unsigned m = __ballot_sync(0xffffffffu, open);
+                if (m) {
+                    found = true;
+                    g = __shfl_sync(0xffffffffu, seg, __ffs(m) - 1);
+                    npos = seg_end(g);
+                    fetch(__shfl_sync(0xffffffffu, at, __ffs(m) - 1));
+                }
+            }
+            if (!found) return false;
+            pos = __shfl_sync(0xffffffffu, f, 0);
+            end = pos + take;
+            if (pos < npos) return true;
+        }
+    };
+    if (one) {
+        npos = seg_end(0u);
+        pos = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+        end = pos + 1u;
+    } else {
+        unsigned smid;
+        asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
+        g = sc.home_of_sm[smid & (F110_SMID_TABLE - 1u)];
+        npos = seg_end(g);
+        fetch(0u);
+        pos = __shfl_sync(0xffffffffu, f, 0);
+        end = pos + take;
+    }
     unsigned unit; bool skip;
     resolve(pos, unit, skip);
-    while (pos < npos) {
+    for (;;) {
+        if (pos >= npos) {
+            if (!steal()) break;
+            resolve(pos, unit, skip);
+        }
         unsigned nlook = 0;
         bool live = false, redone_here = false;
         unsigned npos_next, nunit; bool nskip;
@@ -913,12 +973,14 @@ lidar_tile_kernel(const __grid_constant__ SimConst c, const __grid_constant__ Ma
 
 // ---------------------------------------------------------------- K3: post
 
-// End of a step's lidar bookkeeping, done by one thread of the post kernel: latch the recorded counts, flip the parity and
-// rewind the queue.  Everything it touches was written by the lidar kernel, which is complete before the post kernel's
-// first instruction (cudaGridDependencySynchronize), and is next read by the following step's kernels, which wait for
-// this grid in the same way -- no fence, no ticket.
+// End of a step's lidar bookkeeping, done by the post kernel: its threads rewind the segments' queues (one each), thread 0
+// latches the recorded counts and flips the parity.  Everything it touches was written by the lidar kernel, which is
+// complete before the post kernel's first instruction (cudaGridDependencySynchronize), and is next read by the following
+// step's kernels, which wait for this grid in the same way -- no fence, no ticket.
 __device__ __forceinline__ void latch_launch_order(const StepScratch& sc) {
-    if (blockIdx.x != 0 || threadIdx.x != 0) return;
+    const unsigned t = blockIdx.x * blockDim.x + threadIdx.x;
+    for (unsigned g = t; g < sc.homes; g += gridDim.x * blockDim.x) sc.ctrl[CTRL_SEG + g * SEG_STRIDE] = 0u;
+    if (t != 0) return;
 #pragma unroll
     for (int b = 0; b < 3; ++b) {
         const unsigned n = sc.ctrl[CTRL_NEXT + b * CTRL_NEXT_STRIDE];
@@ -926,7 +988,6 @@ __device__ __forceinline__ void latch_launch_order(const StepScratch& sc) {
         sc.ctrl[CTRL_CUR + b] = n < sc.cap[b] ? n : sc.cap[b];
     }
     sc.ctrl[CTRL_EPOCH] += 1u;
-    sc.ctrl[CTRL_POS] = 0u;
 }
 
 // get_trmtx + get_vertices, collision_models.py:218-260; order rl, rr, fr, fl
@@ -1529,6 +1590,27 @@ int lidar_resident_blocks(bool single_agent) {
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, lidar_variant(21, false, single_agent ? 1 : 0), LIDAR_THREADS, 0) != cudaSuccess)
         return -1;
     return sms * per_sm;
+}
+
+namespace {
+__global__ void smid_probe_kernel(unsigned char* seen) {
+    unsigned smid;
+    asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
+    if (threadIdx.x == 0) seen[smid & (F110_SMID_TABLE - 1u)] = 1;
+}
+}  // namespace
+
+cudaError_t probe_sm_ids(unsigned char* seen) {
+    int dev = 0, sms = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    unsigned char* d = nullptr;
+    if (e == cudaSuccess) e = cudaMalloc(&d, F110_SMID_TABLE);
+    if (e == cudaSuccess) e = cudaMemset(d, 0, F110_SMID_TABLE);
+    if (e == cudaSuccess) { smid_probe_kernel<<<sms * 8, 128>>>(d); e = cudaPeekAtLastError(); }
+    if (e == cudaSuccess) e = cudaMemcpy(seen, d, F110_SMID_TABLE, cudaMemcpyDeviceToHost);
+    cudaFree(d);
+    return e;
 }
 
 typedef void (*LidarTileKernel)(SimConst, MapView, SimState, StepScratch, F110StepIO);

@@ -73,14 +73,20 @@ struct StepScratch {
     unsigned num_units;        // NA * ceil(B / 32) warp-sized work units (32 consecutive beams of one scan)
     unsigned ordered;          // 1: longest-first launch order kept (batches of up to 48 units per resident warp; beyond that the
                                //    tail it saves is below 2 % of the launch and the list atomics cost more), 0: natural order
+    unsigned homes;            // segments of the unit range, each with its own queue: one per SM for launches without the
+                               //   longest-first order, else one (see lidar_kernel)
+    unsigned seg_units;        // units per segment: segment g is units [g seg_units, (g + 1) seg_units) (the last one may be short)
+    const unsigned* home_of_sm;  // [F110_SMID_TABLE] home segment of the warps that run on SM smid (f110_create probes the ids)
     unsigned cap[3];           // capacity of the three heavy-unit lists
-    unsigned* ctrl;            // [F110_CTRL_WORDS]: queue position, parity, latched counts, counts being recorded
+    unsigned* ctrl;            // [ctrl_words(homes)]: counts being recorded, parity, latched counts, the segments' queue positions
     unsigned* list[2];         // [parity][cap0 + cap1 + cap2] unit ids, heaviest class first
     unsigned* cls[2];          // [parity][num_units] class of each unit: 0..2 = on that list, >= 3 = light (natural order); 4 / 5 =
                                //   processed, alternating every second step (see lidar_kernel)
 };
-// the four words atomics hit (queue position, the three counts being recorded) sit on 128-byte lines of their own
-enum { CTRL_POS = 0, CTRL_NEXT = 32, CTRL_NEXT_STRIDE = 32, CTRL_EPOCH = 128, CTRL_CUR = 129, F110_CTRL_WORDS = 160 };
+// the words atomics hit (the three counts being recorded, each segment's queue position) sit on 128-byte lines of their own
+enum { CTRL_NEXT = 32, CTRL_NEXT_STRIDE = 32, CTRL_EPOCH = 128, CTRL_CUR = 129, CTRL_SEG = 160, SEG_STRIDE = 32,
+       F110_SMID_TABLE = 1024 };
+inline size_t ctrl_words(unsigned homes) { return CTRL_SEG + (size_t)homes * SEG_STRIDE; }
 
 struct FastDiv { uint32_t mul, sh1, sh2; };   // n / d == (t + ((n - t) >> sh1)) >> sh2 with t = umulhi(n, mul)
 
@@ -113,6 +119,8 @@ struct SimConst {
 
 cudaError_t launch_dynamics(const SimConst& c, const MapView& m, const SimState& st, const StepScratch& sc, const F110StepIO& io, cudaStream_t s);
 int lidar_resident_blocks(bool single_agent);
+// seen[k] = 1 for every SM id k < F110_SMID_TABLE a wave of the device's CTAs ran on (host array); synchronises
+cudaError_t probe_sm_ids(unsigned char* seen);
 cudaError_t launch_lidar(const SimConst& c, const MapView& m, const SimState& st, const StepScratch& sc, const F110StepIO& io,
                          bool count_lookups, int resident_blocks, bool tile_experiment, cudaStream_t s);
 // smallest positive value of a dense device map (set_map time); synchronises the stream

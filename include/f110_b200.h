@@ -136,6 +136,9 @@ int f110_abi_version(void);
  * Environment switches read here (development / test aids, none changes a result):
  *   F110_DEBUG_SYNC=1   synchronise after every kernel of a step and name the one that faulted
  *   F110_LIDAR_TILE=1   single-agent handles run the shared-memory tile experiment of the lidar kernel (DESIGN.md section 3)
+ *   F110_LIDAR_HOMES=n  the lidar kernel's units are cut into n home segments with a queue each, in natural order, instead
+ *                       of one per SM for launches above 48 units per resident warp and one below (n is clamped to
+ *                       [1, units]; changes the order units run in, never a result)
  * and by f110_set_map_image:
  *   F110_EDT_WIDE=1     force the general form of the device EDT on a map the 16-bit form would take */
 int f110_create(const F110Config* cfg, const double* params, F110Sim** out);

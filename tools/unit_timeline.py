@@ -57,13 +57,16 @@ def main():
     print("last units to finish:")
     for u in last:
         print("  unit %7d pos %6d sm %3d lookups %4d  start %7.1f end %7.1f" % (u, pos[u], sm[u], look[u], s[u], e[u]))
+    for q in (1, 10, 50):
+        print("  units started by %.1f us: %d%%" % (np.percentile(s, q), q))
     for q in (50, 90, 99, 100):
         print("  units ended by %.1f us: %d%%" % (np.percentile(e, q), q))
     # light units: duration vs lookups
     for lo, hi in ((0, 4), (4, 8), (8, 16), (16, 24), (24, 48), (48, 96), (96, 1000)):
         sel = (look >= lo) & (look < hi)
         if sel.any():
-            print("  lookups [%3d,%4d): %6d units, mean %.2f us, start median %.1f us" % (lo, hi, sel.sum(), dur[sel].mean(), np.median(s[sel])))
+            print("  lookups [%3d,%4d): %6d units, mean %.2f us (%.0f ns/lookup), start median %.1f us"
+                  % (lo, hi, sel.sum(), dur[sel].mean(), 1e3 * dur[sel].sum() / max(look[sel].sum(), 1), np.median(s[sel])))
     r = redo > 0
     if r.any():
         print("units with rays redone in exact arithmetic: %d, mean %.2f us (%.0f ns/lookup) against %.2f us (%.0f ns/lookup) for the others below 24 lookups"
