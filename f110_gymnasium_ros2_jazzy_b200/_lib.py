@@ -16,13 +16,15 @@ F110_MAX_AGENTS = 16
 F110_FLAG_COUNT_LOOKUPS = 1
 F110_FLAG_NARROW_FRACTION = 2
 F110_HOST_MERGE_ADJACENT = 1
+F110_MAX_MAPS = 256
 
 F110_OK = 0
 F110_ERR_INVALID, F110_ERR_MAP_NOT_SET, F110_ERR_CUDA, F110_ERR_INDEX = -1, -2, -3, -4
 F110_ERR_POSE_COUNT, F110_ERR_INTEGRATOR, F110_ERR_NO_DEVICE = -5, -6, -7
 
 # every symbol include/f110_b200.h declares
-EXPORTS = ["f110_last_error", "f110_abi_version", "f110_create", "f110_destroy", "f110_set_map", "f110_set_map_image", "f110_get_map", "f110_set_tables",
+EXPORTS = ["f110_last_error", "f110_abi_version", "f110_create", "f110_destroy", "f110_set_map", "f110_set_map_image", "f110_get_map", "f110_set_maps",
+           "f110_map_count", "f110_get_map_slot", "f110_set_env_maps", "f110_set_env_maps_host", "f110_get_env_maps", "f110_set_tables",
            "f110_set_beam_tables", "f110_set_params", "f110_sim_reset", "f110_sim_reset_host", "f110_step", "f110_step_host", "f110_step_host_async", "f110_host_sync", "f110_step_host_multi",
            "f110_state_nbytes", "f110_get_state", "f110_set_state", "f110_get_stats", "f110_get_lookup_count",
            "f110_kernel_launches", "f110_max_lookups", "f110_redone_rays", "f110_map_generation", "f110_debug_unit_timeline", "f110_set_kernel_timing", "f110_get_kernel_timing", "f110_gap_follow", "f110_gather_probe", "f110_edt_kernel_ms", "f110_reward_create", "f110_reward_destroy",
@@ -45,6 +47,12 @@ class F110StepIO(C.Structure):
                 ("obs", C.c_void_p), ("reward", C.c_void_p), ("terminated", C.c_void_p), ("scans_f64", C.c_void_p),
                 ("scans_f32", C.c_void_p), ("state", C.c_void_p), ("collisions", C.c_void_p), ("toggles", C.c_void_p),
                 ("lap_times", C.c_void_p), ("lap_counts", C.c_void_p), ("time", C.c_void_p), ("agent_poses", C.c_void_p)]
+
+
+class F110MapDesc(C.Structure):
+    _fields_ = [("dt", C.c_void_p), ("free_mask", C.c_void_p), ("height", C.c_int32), ("width", C.c_int32),
+                ("resolution", C.c_double), ("orig_x", C.c_double), ("orig_y", C.c_double), ("orig_cos", C.c_double),
+                ("orig_sin", C.c_double)]
 
 
 class F110RewardConfig(C.Structure):
@@ -76,6 +84,13 @@ def load():
     L.f110_set_map.argtypes = [vp, vp, C.c_int32, C.c_int32] + [C.c_double] * 5
     L.f110_set_map_image.argtypes = [vp, vp, C.c_int32, C.c_int32] + [C.c_double] * 5
     L.f110_get_map.argtypes = [vp, vp, C.c_int64]
+    L.f110_set_maps.argtypes = [vp, C.POINTER(F110MapDesc), C.c_int32]
+    L.f110_map_count.argtypes = [vp]
+    L.f110_map_count.restype = C.c_int32
+    L.f110_get_map_slot.argtypes = [vp, C.c_int32, vp, C.c_int64]
+    L.f110_set_env_maps.argtypes = [vp, vp, vp, vp]
+    L.f110_set_env_maps_host.argtypes = [vp, vp, vp]
+    L.f110_get_env_maps.argtypes = [vp, vp, vp]
     L.f110_set_tables.argtypes = [vp, vp, vp]
     L.f110_set_beam_tables.argtypes = [vp, vp, vp, vp]
     L.f110_set_params.argtypes = [vp, vp, C.c_int32]

@@ -114,6 +114,7 @@ class BatchSim(object):
                                          float(resolution), float(origin[0]), float(origin[1]),
                                          float(np.cos(origin[2])), float(np.sin(origin[2]))))
         self.map_shape = dt.shape
+        self.map_shapes = None
 
     def set_map_image(self, free_mask, resolution, origin):
         """Map from the binarised image (non-zero = free, row 0 = bottom row): the EDT runs on the device
@@ -123,15 +124,83 @@ class BatchSim(object):
                                                float(resolution), float(origin[0]), float(origin[1]),
                                                float(np.cos(origin[2])), float(np.sin(origin[2]))))
         self.map_shape = m.shape
+        self.map_shapes = None
 
     def edt_kernel_ms(self):
         """Device time of the EDT kernels of the last set_map_image call (CUDA events)."""
         return float(self.lib.f110_edt_kernel_ms(self.h))
 
-    def get_map(self):
-        dt = np.empty(self.map_shape, np.float64)
-        _lib.check(self.lib.f110_get_map(self.h, dt.ctypes.data_as(C.c_void_p), dt.size))
+    def get_map(self, slot=0):
+        """The fp64 map of `slot` (0 for a single map) as the device holds it."""
+        shape = self.map_shapes[slot] if getattr(self, 'map_shapes', None) else self.map_shape
+        dt = np.empty(shape, np.float64)
+        _lib.check(self.lib.f110_get_map_slot(self.h, int(slot), dt.ctypes.data_as(C.c_void_p), dt.size))
         return dt
+
+    @property
+    def num_maps(self):
+        """Maps installed: 1 for a single map, K after set_maps with K maps, 0 before any."""
+        return int(self.lib.f110_map_count(self.h))
+
+    def set_maps(self, specs, edt='host', map_ext='.png'):
+        """Installs a map set (f110_set_maps): env e then drives on map floor(e * K / N) until set_env_maps says otherwise.
+        Each spec is a yaml path (loaded like set_map: scipy's EDT on the host, or the device EDT with edt='device'), a
+        (dt float64 [H, W], resolution, origin) tuple, or a (free_mask bool / uint8 [H, W], resolution, origin) tuple (device
+        EDT).  The shaped reward keeps one centerline per handle: it does not follow the slots."""
+        from .maps import load_map_image
+        descs, keep, shapes = (_lib.F110MapDesc * len(specs))(), [], []
+        for k, spec in enumerate(specs):
+            if isinstance(spec, (str, bytes)) or hasattr(spec, '__fspath__'):
+                spec = load_map_image(spec, map_ext) if edt == 'device' else load_map(spec, map_ext)
+                if edt == 'device':
+                    spec = (spec[0].astype(bool),) + tuple(spec[1:])
+            arr, res, origin = spec
+            arr = np.asarray(arr)
+            d = descs[k]
+            if arr.dtype == np.float64:
+                a = np.ascontiguousarray(arr)
+                d.dt = a.ctypes.data
+            elif arr.dtype in (np.bool_, np.uint8):
+                a = np.ascontiguousarray(arr != 0, np.uint8)
+                d.free_mask = a.ctypes.data
+            else:
+                raise ValueError("map %d: a distance transform must be float64, a free mask bool or uint8 (got %s)" % (k, arr.dtype))
+            keep.append(a)
+            d.height, d.width = a.shape
+            # orig_s / orig_c are numpy-evaluated on the host like laser_models.py:421-422
+            d.resolution, d.orig_x, d.orig_y = float(res), float(origin[0]), float(origin[1])
+            d.orig_cos, d.orig_sin = float(np.cos(origin[2])), float(np.sin(origin[2]))
+            shapes.append(a.shape)
+        _lib.check(self.lib.f110_set_maps(self.h, descs, len(specs)))
+        self.map_shapes = shapes
+        self.map_shape = shapes[0]
+
+    def set_env_maps(self, slots, env_mask=None):
+        """Each (masked) env's map slot.  numpy / list input: validated on the host first -- a slot outside
+        [0, num_maps) raises IndexError and changes nothing.  CUDA tensors: stream-ordered on the current stream (capturable;
+        entries out of range leave that env's slot unchanged).  A slot change is not a reset: see F110VecEnv.reassign."""
+        if torch.is_tensor(slots) and slots.is_cuda:
+            sl = slots.to(device=self.device, dtype=torch.int32).contiguous()
+            m = None if env_mask is None else env_mask.to(device=self.device, dtype=torch.uint8).contiguous()
+            if sl.numel() != self.N or (m is not None and m.numel() != self.N):
+                raise ValueError("slots and env_mask need %d entries" % self.N)
+            self._keep_slots = (sl, m)
+            _lib.check(self.lib.f110_set_env_maps(self.h, _ptr(sl), _ptr(m), self._stream()))
+            return
+        sl = np.ascontiguousarray(np.asarray(slots.cpu() if torch.is_tensor(slots) else slots), np.int32).reshape(-1)
+        m = None
+        if env_mask is not None:
+            m = np.ascontiguousarray(np.asarray(env_mask.cpu() if torch.is_tensor(env_mask) else env_mask) != 0, np.uint8).reshape(-1)
+        if sl.size != self.N or (m is not None and m.size != self.N):
+            raise ValueError("slots and env_mask need %d entries" % self.N)
+        _lib.check(self.lib.f110_set_env_maps_host(self.h, sl.ctypes.data_as(C.c_void_p),
+                                                   None if m is None else m.ctypes.data_as(C.c_void_p)))
+
+    def env_maps(self):
+        """Device int32 [N]: each env's map slot (all 0 for a single map), valid in stream order."""
+        out = torch.empty(self.N, dtype=torch.int32, device=self.device)
+        _lib.check(self.lib.f110_get_env_maps(self.h, _ptr(out), self._stream()))
+        return out
 
     def set_map(self, map_path, map_ext, edt='host'):
         """edt='host': scipy on the host, as the reference; edt='device': f110_set_map_image."""

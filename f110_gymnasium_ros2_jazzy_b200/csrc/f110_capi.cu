@@ -59,7 +59,11 @@ struct F110Sim {
     StepScratch sc;
     MapView map;
     bool map_set = false;
-    int64_t map_generation = 0;   // bumped by every set_map: a CUDA graph captured before holds the old map by value
+    int64_t map_generation = 0;   // bumped by every set_map / set_maps: a CUDA graph captured before holds the old map by value
+    int32_t map_count = 0;        // maps installed: 0 before any, 1 for a single map, K for a set
+    bool maps_mode = false;       // a set of K >= 2 maps is installed: the *_maps kernels run, `map` is the set's common view
+    MapSet ms;                    // the set's device descriptors (valid while maps_mode)
+    std::vector<MapView> h_views; // [K] host copies of ms.views: the direction tables are rebuilt from them
     bool count_lookups = false;
     bool narrow_fraction = false;
     bool debug_sync = false;
@@ -68,8 +72,11 @@ struct F110Sim {
     char* state_blob = nullptr;   size_t state_bytes = 0;    // checkpointable
     char* scratch_blob = nullptr; size_t scratch_bytes = 0;
     double* d_tables = nullptr;   // params[A][18], sim_params[18], sines, cosines, scan_angles, beam_cos, side_dist
-    double* d_map = nullptr;
+    double* d_map = nullptr;      // the padded map, or the K padded maps of a set back to back
     double2* d_lidar_tables = nullptr;   // beam_tt[B], dir_fx[theta_dis]
+    MapView* d_views = nullptr;   // [K] a set's per-slot views
+    double2* d_map_dir = nullptr; // [K][theta_dis] a set's direction tables
+    int32_t* d_env_map = nullptr; // [N] slot of each env (all 0 unless a set is installed)
     std::vector<double> h_sines, h_cosines;   // host copies: dir_fx is rebuilt from them whenever the map changes
     // host-buffer path (f110_step_host)
     cudaStream_t host_stream = nullptr;
@@ -166,10 +173,11 @@ int run_step(F110Sim* sim, const F110StepIO& io, cudaStream_t s) {
         const cudaError_t de = cudaStreamSynchronize(s);                                                           \
         if (de != cudaSuccess) return fail(F110_ERR_CUDA, "%s: %s", name, cudaGetErrorString(de));                 \
     }
-    CUDA_TRY(launch_dynamics(sim->c, sim->map, sim->st, sim->sc, io, s));
+    const MapSet* ms = sim->maps_mode ? &sim->ms : nullptr;
+    CUDA_TRY(launch_dynamics(sim->c, sim->map, sim->st, sim->sc, io, ms, s));
     DEBUG_SYNC("dynamics_kernel")
     if (sim->timing) CUDA_TRY(cudaEventRecord(e[1], s));
-    CUDA_TRY(launch_lidar(sim->c, sim->map, sim->st, sim->sc, io, sim->count_lookups, sim->lidar_blocks, sim->lidar_tile, s));
+    CUDA_TRY(launch_lidar(sim->c, sim->map, sim->st, sim->sc, io, ms, sim->count_lookups, sim->lidar_blocks, sim->lidar_tile, s));
     DEBUG_SYNC("lidar_kernel")
     if (sim->timing) CUDA_TRY(cudaEventRecord(e[2], s));
     CUDA_TRY(launch_post(sim->c, sim->st, sim->sc, io, s));
@@ -258,6 +266,8 @@ int f110_create(const F110Config* cfg, const double* params, F110Sim** out) {
     if (e == cudaSuccess) e = cudaMemset(sim->d_tables, 0, ntab * sizeof(double));
     if (e == cudaSuccess) e = cudaMalloc(&sim->d_lidar_tables, ((size_t)B + cfg->theta_dis) * sizeof(double2));
     if (e == cudaSuccess) e = cudaMemset(sim->d_lidar_tables, 0, ((size_t)B + cfg->theta_dis) * sizeof(double2));
+    if (e == cudaSuccess) e = cudaMalloc(&sim->d_env_map, (size_t)N * sizeof(int32_t));
+    if (e == cudaSuccess) e = cudaMemset(sim->d_env_map, 0, (size_t)N * sizeof(int32_t));
     if (e == cudaSuccess) {
         // host_stream_rank r > 0: the r-th highest stream priority the device offers, so that a caller pipelining several
         // handles (f110_step_host_multi) gets handle 1's kernels finished -- and its download started -- first
@@ -341,42 +351,82 @@ void f110_destroy(F110Sim* sim) {
     Guard g(sim->cfg.device);
     if (sim->host_stream) { cudaStreamSynchronize(sim->host_stream); cudaStreamDestroy(sim->host_stream); }
     cudaFree(sim->state_blob); cudaFree(sim->scratch_blob); cudaFree(sim->d_tables); cudaFree(sim->d_map); cudaFree(sim->d_lidar_tables);
+    cudaFree(sim->d_views); cudaFree(sim->d_map_dir); cudaFree(sim->d_env_map);
     cudaFree(sim->io_blob);
     edt_scratch_free(&sim->edt);
     for (cudaEvent_t e : sim->tev) cudaEventDestroy(e);
     delete sim;
 }
 
-// The lidar kernel's direction table: table direction k rotated into the map frame and scaled to fixed-point cells per
-// metre.  Depends on the sin / cos tables and on the map (origin yaw, resolution, fraction bits): rebuilt by both setters.
-static int refresh_direction_table(F110Sim* sim) {
-    if (!sim->map_set) return F110_OK;
-    const MapView& m = sim->map;
+// The lidar kernel's direction table of one map: table direction k rotated into the map frame and scaled to fixed-point
+// cells per metre.  Depends on the sin / cos tables and on the map (origin yaw, resolution, fraction bits).
+static void direction_table(const F110Sim* sim, const MapView& m, double2* dir) {
     const size_t n = sim->h_sines.size();
-    std::vector<double2> dir(n);
     for (size_t k = 0; k < n; ++k) {
         const double cs = sim->h_cosines[k], sn = sim->h_sines[k];
         dir[k].x = (cs * m.oc + sn * m.os) * m.inv_fx;
         dir[k].y = (-cs * m.os + sn * m.oc) * m.inv_fx;
     }
+}
+
+// Rebuilds the direction table of the map, or of every map of a set (both setters call it).
+static int refresh_direction_table(F110Sim* sim) {
+    if (!sim->map_set) return F110_OK;
+    const size_t n = sim->h_sines.size();
+    if (sim->maps_mode) {
+        std::vector<double2> dir(n * sim->h_views.size());
+        for (size_t k = 0; k < sim->h_views.size(); ++k) direction_table(sim, sim->h_views[k], dir.data() + k * n);
+        CUDA_TRY(cudaMemcpy(sim->d_map_dir, dir.data(), dir.size() * sizeof(double2), cudaMemcpyHostToDevice));
+        return F110_OK;
+    }
+    std::vector<double2> dir(n);
+    direction_table(sim, sim->map, dir.data());
     CUDA_TRY(cudaMemcpy(const_cast<double2*>(sim->c.dir_fx), dir.data(), n * sizeof(double2), cudaMemcpyHostToDevice));
     return F110_OK;
+}
+
+// Fixed-point format of the lidar kernel's fast march for a map whose larger side is `side_cells`: as many fraction bits as
+// a 32-bit coordinate leaves beside the cell index (+ 1: the map is stored one cell in from the padded array's corner).
+// Fills fx_bits, guard, guard_mask, prows, pitch and fx_off.
+static void fixed_point_format(const F110Sim* sim, unsigned side_cells, MapView& m) {
+    auto bit_length = [](unsigned v) { unsigned b = 0; while ((v >> b) != 0u) ++b; return b; };
+    const unsigned side = side_cells + 1u;
+    m.fx_bits = 32u - bit_length(side) > 24u ? 24u : 32u - bit_length(side);
+    m.guard = sim->narrow_fraction ? (1u << (m.fx_bits - 5u)) : 2u;     // F110_FLAG_NARROW_FRACTION: 1/16 of every cell undecided
+    m.guard_mask = ((1u << m.fx_bits) - 1u) & ~(2u * m.guard - 1u);
+    m.prows = 1 << (32u - m.fx_bits);
+    m.pitch = m.prows + 16;
+    m.fx_off = (double)(1u << m.fx_bits) - (double)m.guard;
+}
+
+// The per-map fields of a view in format `m` (dt, size, resolution, origin)
+static void place_map(MapView& m, double* padded, int height, int width, double resolution,
+                      double orig_x, double orig_y, double orig_cos, double orig_sin) {
+    m.dt = padded; m.H = height; m.W = width;
+    m.last = (height - 1) * width + (width - 1);
+    m.res = resolution;
+    m.inv_fx = (1.0 / resolution) * (double)(1u << m.fx_bits);
+    m.ox = orig_x; m.oy = orig_y; m.oc = orig_cos; m.os = orig_sin;
+    m.wres = width * resolution; m.hres = height * resolution;   // laser_models.py:79
+}
+
+// Leaves set mode (after a single map replaced the set): frees the set's descriptors, every env back on slot 0
+static void drop_map_set(F110Sim* sim) {
+    cudaFree(sim->d_views); sim->d_views = nullptr;
+    cudaFree(sim->d_map_dir); sim->d_map_dir = nullptr;
+    sim->h_views.clear();
+    memset(&sim->ms, 0, sizeof(sim->ms));
+    if (sim->maps_mode) cudaMemset(sim->d_env_map, 0, (size_t)sim->c.N * sizeof(int32_t));
+    sim->maps_mode = false;
 }
 
 // Installs a DENSE device map [H][W] as the handle's padded map (see MapView) and frees `dense`.
 static int install_map(F110Sim* sim, double* dense, int height, int width, double resolution,
                        double orig_x, double orig_y, double orig_cos, double orig_sin) {
-    // fixed-point format of the lidar kernel's fast march: as many fraction bits as a 32-bit coordinate leaves beside the
-    // cell index of the larger side (+ 1: the map is stored one cell in from the padded array's corner)
-    auto bit_length = [](unsigned v) { unsigned b = 0; while ((v >> b) != 0u) ++b; return b; };
     MapView m;
     memset(&m, 0, sizeof(m));
-    const unsigned side = (unsigned)(width > height ? width : height) + 1u;
-    m.fx_bits = 32u - bit_length(side) > 24u ? 24u : 32u - bit_length(side);
-    m.guard = sim->narrow_fraction ? (1u << (m.fx_bits - 5u)) : 2u;     // F110_FLAG_NARROW_FRACTION: 1/16 of every cell undecided
-    m.guard_mask = ((1u << m.fx_bits) - 1u) & ~(2u * m.guard - 1u);
-    const size_t prows = (size_t)1 << (32u - m.fx_bits);
-    const size_t pitch = prows + 16;
+    fixed_point_format(sim, (unsigned)(width > height ? width : height), m);
+    const size_t prows = (size_t)m.prows, pitch = (size_t)m.pitch;
     if ((double)prows * (double)pitch >= 2147483648.0) { cudaFree(dense); return fail(F110_ERR_INVALID, "map too large once padded (%zu x %zu cells)", prows, pitch); }
     if (map_min_positive(dense, (size_t)height * width, &m.min_positive, sim->host_stream) != cudaSuccess) {
         cudaFree(dense); cudaGetLastError();
@@ -390,15 +440,11 @@ static int install_map(F110Sim* sim, double* dense, int height, int width, doubl
     if (e != cudaSuccess) { cudaFree(padded); cudaGetLastError(); return fail(F110_ERR_CUDA, "map padding: %s", cudaGetErrorString(e)); }
     cudaFree(sim->d_map);
     sim->d_map = padded;
-    m.dt = padded; m.H = height; m.W = width; m.pitch = (int)pitch; m.prows = (int)prows;
-    m.last = (height - 1) * width + (width - 1);
-    m.res = resolution;
-    m.inv_fx = (1.0 / resolution) * (double)(1u << m.fx_bits);
-    m.fx_off = (double)(1u << m.fx_bits) - (double)m.guard;
-    m.ox = orig_x; m.oy = orig_y; m.oc = orig_cos; m.os = orig_sin;
-    m.wres = width * resolution; m.hres = height * resolution;   // laser_models.py:79
+    drop_map_set(sim);
+    place_map(m, padded, height, width, resolution, orig_x, orig_y, orig_cos, orig_sin);
     sim->map = m;
     sim->map_set = true;
+    sim->map_count = 1;
     sim->map_generation += 1;
     return refresh_direction_table(sim);
 }
@@ -418,16 +464,12 @@ int f110_set_map(F110Sim* sim, const double* dt, int32_t height, int32_t width, 
     return install_map(sim, d, height, width, resolution, orig_x, orig_y, orig_cos, orig_sin);
 }
 
-int f110_set_map_image(F110Sim* sim, const uint8_t* free_mask, int32_t height, int32_t width, double resolution,
-                       double orig_x, double orig_y, double orig_cos, double orig_sin) {
-    if (!sim || !free_mask || height < 1 || width < 1 || !(resolution > 0)) return fail(F110_ERR_INVALID, "bad map arguments");
-    if ((double)height * width >= 2147483648.0 || height >= 65536 || width >= 65536)
-        return fail(F110_ERR_INVALID, "map too large (need H*W < 2^31 and H, W < 65536)");
-    Guard g(sim->cfg.device);
-    CUDA_TRY(cudaDeviceSynchronize());
+// The dense fp64 map of a mask through the device EDT: DEVICE [H][W] in *out (caller frees), or an error code
+static int dense_from_mask(F110Sim* sim, const uint8_t* free_mask, int32_t height, int32_t width, double resolution, double** out) {
     const size_t cells = (size_t)height * width;
     uint8_t* d_mask = nullptr;
     double* d = nullptr;
+    *out = nullptr;
     CUDA_TRY(cudaMalloc(&d_mask, cells));
     cudaError_t e = cudaMalloc(&d, cells * sizeof(double));
     if (e == cudaSuccess) e = cudaMemcpy(d_mask, free_mask, cells, cudaMemcpyHostToDevice);
@@ -435,21 +477,163 @@ int f110_set_map_image(F110Sim* sim, const uint8_t* free_mask, int32_t height, i
     if (e == cudaSuccess) rc = edt_device(d_mask, height, width, resolution, d, &sim->edt, sim->host_stream);
     cudaFree(d_mask);
     if (e != cudaSuccess || rc != 0) { cudaFree(d); cudaGetLastError(); return fail(F110_ERR_CUDA, "device EDT failed"); }
+    *out = d;
+    return F110_OK;
+}
+
+int f110_set_map_image(F110Sim* sim, const uint8_t* free_mask, int32_t height, int32_t width, double resolution,
+                       double orig_x, double orig_y, double orig_cos, double orig_sin) {
+    if (!sim || !free_mask || height < 1 || width < 1 || !(resolution > 0)) return fail(F110_ERR_INVALID, "bad map arguments");
+    if ((double)height * width >= 2147483648.0 || height >= 65536 || width >= 65536)
+        return fail(F110_ERR_INVALID, "map too large (need H*W < 2^31 and H, W < 65536)");
+    Guard g(sim->cfg.device);
+    CUDA_TRY(cudaDeviceSynchronize());
+    double* d = nullptr;
+    const int rc = dense_from_mask(sim, free_mask, height, width, resolution, &d);
+    if (rc != F110_OK) return rc;
     return install_map(sim, d, height, width, resolution, orig_x, orig_y, orig_cos, orig_sin);
 }
 
 float f110_edt_kernel_ms(const F110Sim* sim) { return sim ? sim->edt.kernel_ms : -1.f; }
 
-int f110_get_map(F110Sim* sim, double* dt_host, int64_t capacity_cells) {
-    if (!sim || !dt_host) return fail(F110_ERR_INVALID, "null argument");
-    if (!sim->map_set) return fail(F110_ERR_MAP_NOT_SET, "Map is not set for scan simulator.");
-    const size_t cells = (size_t)sim->map.H * sim->map.W;
-    if ((size_t)capacity_cells < cells) return fail(F110_ERR_INVALID, "buffer too small for %d x %d cells", sim->map.H, sim->map.W);
+int f110_set_maps(F110Sim* sim, const F110MapDesc* maps, int32_t count) {
+    if (!sim || !maps) return fail(F110_ERR_INVALID, "null argument");
+    if (count < 1 || count > F110_MAX_MAPS) return fail(F110_ERR_INVALID, "a map set holds 1 to %d maps, not %d", F110_MAX_MAPS, count);
+    unsigned side = 0;
+    for (int k = 0; k < count; ++k) {
+        const F110MapDesc& d = maps[k];
+        if ((!d.dt && !d.free_mask) || d.height < 1 || d.width < 1 || !(d.resolution > 0))
+            return fail(F110_ERR_INVALID, "bad arguments for map %d of the set", k);
+        if ((double)d.height * d.width >= 2147483648.0 || d.height >= 65536 || d.width >= 65536)
+            return fail(F110_ERR_INVALID, "map %d too large (need H*W < 2^31 and H, W < 65536)", k);
+        const unsigned s = (unsigned)(d.width > d.height ? d.width : d.height);
+        side = s > side ? s : side;
+    }
+    if (count == 1) {   // a set of one map is that map
+        const F110MapDesc& d = maps[0];
+        return d.dt ? f110_set_map(sim, d.dt, d.height, d.width, d.resolution, d.orig_x, d.orig_y, d.orig_cos, d.orig_sin)
+                    : f110_set_map_image(sim, d.free_mask, d.height, d.width, d.resolution, d.orig_x, d.orig_y, d.orig_cos, d.orig_sin);
+    }
+    // one fixed-point format for the whole set, that of its largest side; every map padded to it, at a fixed stride
+    MapView common;
+    memset(&common, 0, sizeof(common));
+    fixed_point_format(sim, side, common);
+    const size_t stride = (size_t)common.prows * (size_t)common.pitch;
+    if ((double)stride * count >= 2147483648.0)
+        return fail(F110_ERR_INVALID, "map set too large: %d maps padded to %d x %d cells each (the largest side is %u) exceed 2^31 cells",
+                    count, common.prows, common.pitch, side);
     Guard g(sim->cfg.device);
     CUDA_TRY(cudaDeviceSynchronize());
-    (void)cells;
-    CUDA_TRY(cudaMemcpy2D(dt_host, (size_t)sim->map.W * sizeof(double), sim->d_map + sim->map.pitch + 1, (size_t)sim->map.pitch * sizeof(double),
-                          (size_t)sim->map.W * sizeof(double), (size_t)sim->map.H, cudaMemcpyDeviceToHost));
+    double* padded = nullptr;
+    MapView* d_views = nullptr;
+    double2* d_dir = nullptr;
+    const size_t nt = sim->h_sines.size();
+    cudaError_t e = cudaMalloc(&padded, stride * count * sizeof(double));
+    if (e == cudaSuccess) e = cudaMalloc(&d_views, (size_t)count * sizeof(MapView));
+    if (e == cudaSuccess) e = cudaMalloc(&d_dir, (size_t)count * nt * sizeof(double2));
+    auto undo = [&]() { cudaFree(padded); cudaFree(d_views); cudaFree(d_dir); cudaGetLastError(); };
+    if (e != cudaSuccess) { undo(); return fail(F110_ERR_CUDA, "map set allocation (%d x %zu cells): %s", count, stride, cudaGetErrorString(e)); }
+    std::vector<MapView> views(count, common);
+    double min_positive = INFINITY;
+    for (int k = 0; k < count; ++k) {
+        const F110MapDesc& d = maps[k];
+        const size_t cells = (size_t)d.height * d.width;
+        double* dense = nullptr;
+        if (d.dt) {
+            e = cudaMalloc(&dense, cells * sizeof(double));
+            if (e == cudaSuccess) e = cudaMemcpy(dense, d.dt, cells * sizeof(double), cudaMemcpyHostToDevice);
+            if (e != cudaSuccess) { cudaFree(dense); undo(); return fail(F110_ERR_CUDA, "upload of map %d: %s", k, cudaGetErrorString(e)); }
+        } else {
+            const int rc = dense_from_mask(sim, d.free_mask, d.height, d.width, d.resolution, &dense);
+            if (rc != F110_OK) { undo(); return rc; }
+        }
+        MapView& v = views[k];
+        double* block = padded + (size_t)k * stride;
+        e = map_min_positive(dense, cells, &v.min_positive, sim->host_stream);
+        if (e == cudaSuccess) e = launch_pad_map(dense, d.height, d.width, block, common.prows, common.pitch, sim->host_stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(sim->host_stream);
+        cudaFree(dense);
+        if (e != cudaSuccess) { undo(); return fail(F110_ERR_CUDA, "padding of map %d: %s", k, cudaGetErrorString(e)); }
+        place_map(v, block, d.height, d.width, d.resolution, d.orig_x, d.orig_y, d.orig_cos, d.orig_sin);
+        min_positive = v.min_positive < min_positive ? v.min_positive : min_positive;
+    }
+    std::vector<double2> dir(nt * count);
+    for (int k = 0; k < count; ++k) direction_table(sim, views[k], dir.data() + (size_t)k * nt);
+    e = cudaMemcpy(d_views, views.data(), views.size() * sizeof(MapView), cudaMemcpyHostToDevice);
+    if (e == cudaSuccess) e = cudaMemcpy(d_dir, dir.data(), dir.size() * sizeof(double2), cudaMemcpyHostToDevice);
+    // every env to its contiguous block: env e drives on slot floor(e K / N)
+    std::vector<int32_t> slots(sim->c.N);
+    for (int n = 0; n < sim->c.N; ++n) slots[n] = (int32_t)((int64_t)n * count / sim->c.N);
+    if (e == cudaSuccess) e = cudaMemcpy(sim->d_env_map, slots.data(), slots.size() * sizeof(int32_t), cudaMemcpyHostToDevice);
+    if (e != cudaSuccess) { undo(); return fail(F110_ERR_CUDA, "map set upload: %s", cudaGetErrorString(e)); }
+    // commit
+    cudaFree(sim->d_map); cudaFree(sim->d_views); cudaFree(sim->d_map_dir);
+    sim->d_map = padded; sim->d_views = d_views; sim->d_map_dir = d_dir;
+    sim->h_views = views;
+    sim->map = views[0];
+    sim->map.min_positive = min_positive;
+    sim->ms.env_map = sim->d_env_map;
+    sim->ms.views = d_views;
+    sim->ms.dir_fx = d_dir;
+    sim->ms.stride = stride;
+    sim->maps_mode = true;
+    sim->map_set = true;
+    sim->map_count = count;
+    sim->map_generation += 1;
+    return F110_OK;
+}
+
+int32_t f110_map_count(const F110Sim* sim) { return sim ? sim->map_count : 0; }
+
+int f110_get_map_slot(F110Sim* sim, int32_t slot, double* dt_host, int64_t capacity_cells) {
+    if (!sim || !dt_host) return fail(F110_ERR_INVALID, "null argument");
+    if (!sim->map_set) return fail(F110_ERR_MAP_NOT_SET, "Map is not set for scan simulator.");
+    if (slot < 0 || slot >= sim->map_count) return fail(F110_ERR_INDEX, "map slot %d out of range (%d maps)", slot, sim->map_count);
+    const MapView& m = sim->maps_mode ? sim->h_views[slot] : sim->map;
+    const size_t cells = (size_t)m.H * m.W;
+    if ((size_t)capacity_cells < cells) return fail(F110_ERR_INVALID, "buffer too small for %d x %d cells", m.H, m.W);
+    Guard g(sim->cfg.device);
+    CUDA_TRY(cudaDeviceSynchronize());
+    CUDA_TRY(cudaMemcpy2D(dt_host, (size_t)m.W * sizeof(double), m.dt + m.pitch + 1, (size_t)m.pitch * sizeof(double),
+                          (size_t)m.W * sizeof(double), (size_t)m.H, cudaMemcpyDeviceToHost));
+    return F110_OK;
+}
+
+int f110_get_map(F110Sim* sim, double* dt_host, int64_t capacity_cells) { return f110_get_map_slot(sim, 0, dt_host, capacity_cells); }
+
+int f110_set_env_maps(F110Sim* sim, const int32_t* slots, const uint8_t* env_mask, void* stream) {
+    if (!sim || !slots) return fail(F110_ERR_INVALID, "null argument");
+    Guard g(sim->cfg.device);
+    CUDA_TRY(launch_set_env_maps(sim->d_env_map, slots, env_mask, sim->c.N, sim->map_count, (cudaStream_t)stream));
+    sim->launches += 1;
+    return F110_OK;
+}
+
+int f110_set_env_maps_host(F110Sim* sim, const int32_t* slots, const uint8_t* env_mask) {
+    if (!sim || !slots) return fail(F110_ERR_INVALID, "null argument");
+    const int N = sim->c.N;
+    for (int n = 0; n < N; ++n)
+        if ((!env_mask || env_mask[n]) && (slots[n] < 0 || slots[n] >= sim->map_count))
+            return fail(F110_ERR_INDEX, "env %d: map slot %d out of range (%d maps)", n, slots[n], sim->map_count);
+    Guard g(sim->cfg.device);
+    CUDA_TRY(cudaDeviceSynchronize());
+    int32_t* d = nullptr;
+    CUDA_TRY(cudaMalloc(&d, (size_t)N * sizeof(int32_t) + N));
+    uint8_t* d_mask = env_mask ? reinterpret_cast<uint8_t*>(d + N) : nullptr;
+    cudaStream_t s = sim->host_stream;
+    cudaError_t e = cudaMemcpyAsync(d, slots, (size_t)N * sizeof(int32_t), cudaMemcpyHostToDevice, s);
+    if (e == cudaSuccess && env_mask) e = cudaMemcpyAsync(d_mask, env_mask, N, cudaMemcpyHostToDevice, s);
+    if (e == cudaSuccess) e = launch_set_env_maps(sim->d_env_map, d, d_mask, N, sim->map_count, s);
+    if (e == cudaSuccess) { sim->launches += 1; e = cudaStreamSynchronize(s); }
+    cudaFree(d);
+    if (e != cudaSuccess) return fail(F110_ERR_CUDA, "f110_set_env_maps_host: %s", cudaGetErrorString(e));
+    return F110_OK;
+}
+
+int f110_get_env_maps(F110Sim* sim, int32_t* slots_out, void* stream) {
+    if (!sim || !slots_out) return fail(F110_ERR_INVALID, "null argument");
+    Guard g(sim->cfg.device);
+    CUDA_TRY(cudaMemcpyAsync(slots_out, sim->d_env_map, (size_t)sim->c.N * sizeof(int32_t), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
     return F110_OK;
 }
 

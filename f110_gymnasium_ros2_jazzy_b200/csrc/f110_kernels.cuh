@@ -36,6 +36,17 @@ struct MapView {
     double wres, hres;  // W*res, H*res
 };
 
+// A map set (f110_set_maps): K maps in one handle, each env on the map of its slot.  Every map is padded to the set's
+// common fixed-point format (fx_bits of the largest side, so prows, pitch and guard_mask are shared) and the K padded
+// blocks lie back to back at a stride of prows * pitch cells: a slot's cells start at the set MapView's dt + slot * stride.
+// What differs per slot is in views[slot] (origin, resolution, inv_fx, H, W, dt of its own block) and in its direction table.
+struct MapSet {
+    const int32_t* env_map;   // [N] slot of each env
+    const MapView* views;     // [K] per-slot descriptors
+    const double2* dir_fx;    // [K][theta_dis] slot k's direction table (as SimConst::dir_fx for a single map)
+    size_t stride;            // cells between the blocks of two consecutive slots
+};
+
 // Persistent simulation state: one arena, SoA over s = env*A + agent (coalesced for one thread
 // per vehicle) and over env.  Everything a checkpoint needs lives between arena and arena+nbytes.
 struct SimState {
@@ -117,12 +128,16 @@ struct SimConst {
                                //   ((cos*oc + sin*os) * inv_fx, (-cos*os + sin*oc) * inv_fy); rebuilt by set_map / set_tables
 };
 
-cudaError_t launch_dynamics(const SimConst& c, const MapView& m, const SimState& st, const StepScratch& sc, const F110StepIO& io, cudaStream_t s);
+// ms == nullptr: the handle holds one map (m); otherwise m is the set's common view (slot 0's, min_positive over the set)
+cudaError_t launch_dynamics(const SimConst& c, const MapView& m, const SimState& st, const StepScratch& sc, const F110StepIO& io,
+                            const MapSet* ms, cudaStream_t s);
 int lidar_resident_blocks(bool single_agent);
 // seen[k] = 1 for every SM id k < F110_SMID_TABLE a wave of the device's CTAs ran on (host array); synchronises
 cudaError_t probe_sm_ids(unsigned char* seen);
 cudaError_t launch_lidar(const SimConst& c, const MapView& m, const SimState& st, const StepScratch& sc, const F110StepIO& io,
-                         bool count_lookups, int resident_blocks, bool tile_experiment, cudaStream_t s);
+                         const MapSet* ms, bool count_lookups, int resident_blocks, bool tile_experiment, cudaStream_t s);
+// env_map[e] = slots[e] for every env e with (mask == nullptr || mask[e]) and 0 <= slots[e] < count (all DEVICE pointers)
+cudaError_t launch_set_env_maps(int32_t* env_map, const int32_t* slots, const uint8_t* mask, int N, int count, cudaStream_t s);
 // smallest positive value of a dense device map (set_map time); synchronises the stream
 cudaError_t map_min_positive(const double* dense, size_t cells, double* out, cudaStream_t s);
 cudaError_t launch_post(const SimConst& c, const SimState& st, const StepScratch& sc, const F110StepIO& io, cudaStream_t s);

@@ -219,12 +219,18 @@ class F110VecEnv(object):
     The returned tensors are persistent buffers rewritten by the next step.  With ``auto_reset=True`` an env
     that terminated is reset to its start poses by the NEXT step call, which is then that env's zero-action
     reset step (gymnasium's next-step autoreset; F110Env.reset semantics f110_env.py:425-472).
+
+    ``maps=[spec, ...]`` instead of ``map=`` / ``map_arrays=`` installs a map set (BatchSim.set_maps): every env drives on
+    the map of its slot, env e on slot floor(e * K / N) unless ``env_maps`` (int [N]) says otherwise; ``reassign`` moves envs
+    to other maps at their next reset.  The shaped reward (ShapedReward, DeviceRollout) stays single-centerline.
     """
 
     def __init__(self, num_envs, map_dir=None, map=None, map_ext='.png', num_agents=2, params=None, seed=42,
                  timestep=0.01, ego_idx=0, integrator=Integrator.RK4, lidar_dist=0.0, device=None, auto_reset=True,
                  outputs=FAST_OUTPUTS, noise_std=0.01, num_beams=1080, fov=4.7, count_lookups=False, map_arrays=None,
-                 cuda_graph=False):
+                 cuda_graph=False, maps=None, env_maps=None):
+        if maps is not None and (map is not None or map_arrays is not None):
+            raise ValueError("give either maps= (a map set) or map= / map_arrays= (one map), not both")
         self.num_envs, self.num_agents = num_envs, num_agents
         self.timestep = timestep
         self.auto_reset = auto_reset
@@ -232,7 +238,11 @@ class F110VecEnv(object):
         self.backend = BatchSim(num_envs, num_agents, params=params, seed=seed, timestep=timestep, integrator=integrator,
                                 ego_idx=ego_idx, lidar_dist=lidar_dist, noise_std=noise_std, device=device, outputs=outs,
                                 num_beams=num_beams, fov=fov, count_lookups=count_lookups)
-        if map_arrays is not None:
+        if maps is not None:
+            self.backend.set_maps(maps, map_ext=map_ext)
+            if env_maps is not None:
+                self.backend.set_env_maps(env_maps)
+        elif map_arrays is not None:
             self.backend.set_map_arrays(*map_arrays)
         else:
             self.backend.set_map(map_dir + map + '.yaml', map_ext)
@@ -298,6 +308,36 @@ class F110VecEnv(object):
         self.backend.set_map_arrays(dt, resolution, origin)
         self._drop_graph()
 
+    def set_maps(self, specs, edt='host', map_ext='.png'):
+        """Installs a map set for the whole batch (BatchSim.set_maps; env e on slot floor(e * K / N)); like set_map it drops a
+        captured CUDA graph."""
+        self.backend.set_maps(specs, edt=edt, map_ext=map_ext)
+        self._drop_graph()
+
+    def reassign(self, env_mask, slots, start_poses):
+        """Moves the masked envs to map `slots` with new start poses, effective at their reset on the next step: sets their
+        slots (BatchSim.set_env_maps) and start poses and ORs the mask into `terminated`, the next step's reset mask.  All
+        three are in-place, stream-ordered device writes, so a captured CUDA graph replays them without re-capture.
+        env_mask [N] (non-zero = move), slots int [N] (or one int), start_poses [N, A, 3] (or [A, 3]); entries of unmasked
+        envs are ignored.  Needs auto_reset=True (without it nothing would reset the envs)."""
+        if not self.auto_reset:
+            raise ValueError("reassign needs auto_reset=True: the moved envs are reset by the next step")
+        if self.start_poses is None:
+            raise ValueError("reset() the batch before reassign()")
+        N = self.num_envs
+        m = torch.as_tensor(np.asarray(env_mask) if not torch.is_tensor(env_mask) else env_mask).to(self.device)
+        m = (m.reshape(N) != 0)
+        sl = torch.as_tensor(np.asarray(slots) if not torch.is_tensor(slots) else slots).to(self.device, torch.int32)
+        sl = sl.expand(N).contiguous() if sl.ndim == 0 else sl.reshape(N).contiguous()
+        p = torch.as_tensor(np.asarray(start_poses, np.float64) if not torch.is_tensor(start_poses) else start_poses,
+                            dtype=torch.float64).to(self.device)
+        if p.ndim == 2:
+            p = p[None].expand(N, -1, -1)
+        self.backend.set_env_maps(sl, m.to(torch.uint8))
+        self.start_poses.copy_(torch.where(m[:, None, None], p, self.start_poses))
+        term = self.backend.out['terminated']
+        term.bitwise_or_(m.to(torch.uint8))
+
     def _drop_graph(self):
         self._graph = None
         self._steps_eager = 0
@@ -308,10 +348,13 @@ class F110VecEnv(object):
         BatchSim.state_dict), plus what lives on this side of the C ABI -- the terminated flags (the next step's reset mask
         under auto-reset) and the start poses."""
         return {'backend': self.backend.state_dict(), 'terminated': self.backend.out['terminated'].clone(),
-                'start_poses': None if self.start_poses is None else self.start_poses.clone(), 'auto_reset': self.auto_reset}
+                'start_poses': None if self.start_poses is None else self.start_poses.clone(), 'auto_reset': self.auto_reset,
+                'env_maps': self.backend.env_maps().clone()}
 
     def load_state_dict(self, sd):
         self.backend.load_state_dict(sd['backend'])
+        if sd.get('env_maps') is not None:
+            self.backend.set_env_maps(sd['env_maps'].cpu().numpy())      # host form: a slot this env's maps lack raises
         self.backend.out['terminated'].copy_(sd['terminated'].to(self.device))
         self.start_poses = None if sd['start_poses'] is None else sd['start_poses'].to(self.device).contiguous()
         self._drop_graph()          # a captured step holds the old start-pose tensor
@@ -335,8 +378,13 @@ class F110HostVecEnv(object):
     """
 
     def __init__(self, num_envs, chunks=2, map_arrays=None, map_dir=None, map=None, map_ext='.png', num_agents=1,
-                 seed=42, device=None, outputs=FAST_OUTPUTS, num_beams=1080, **kw):
+                 seed=42, device=None, outputs=FAST_OUTPUTS, num_beams=1080, maps=None, env_maps=None, **kw):
+        if maps is not None and (map is not None or map_arrays is not None):
+            raise ValueError("give either maps= (a map set) or map= / map_arrays= (one map), not both")
         self.num_envs, self.num_agents, self.num_beams = num_envs, num_agents, num_beams
+        if maps is not None:
+            # the whole batch's assignment (F110VecEnv's default: env e on slot floor(e K / N)); each chunk gets its slice
+            slots = (np.arange(num_envs) * len(maps)) // num_envs if env_maps is None else np.asarray(env_maps, np.int32)
         if isinstance(chunks, int):
             chunks = max(1, min(chunks, num_envs))
             self.bounds = [(num_envs * k) // chunks for k in range(chunks + 1)]
@@ -349,7 +397,10 @@ class F110HostVecEnv(object):
             n = self.bounds[k + 1] - self.bounds[k]
             b = BatchSim(n, num_agents, seed=seed + 7919 * k, device=device, outputs=('obs',), num_beams=num_beams,
                          host_stream_rank=k + 1, **kw)
-            if map_arrays is not None:
+            if maps is not None:
+                b.set_maps(maps, map_ext=map_ext)
+                b.set_env_maps(slots[self.bounds[k]:self.bounds[k + 1]])
+            elif map_arrays is not None:
                 b.set_map_arrays(*map_arrays)
             else:
                 b.set_map(map_dir + map + '.yaml', map_ext)

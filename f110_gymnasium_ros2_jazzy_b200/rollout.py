@@ -63,7 +63,8 @@ class Actor(torch.nn.Module):
 class DeviceRollout(object):
     """ego = policy(obs), opponent = gap-follow on its own scan, env.step -- no host round trip per step.
 
-    ``reward_fn`` (optional, e.g. ShapedReward) replaces the env's constant reward, as train_ddpg.py:179 does.
+    ``reward_fn`` (optional, e.g. ShapedReward) replaces the env's constant reward, as train_ddpg.py:179 does.  Its
+    centerline is one track's: with a map set (F110VecEnv(maps=...)) the reward does not follow the envs' slots.
     ``replay`` (optional, e.g. DeviceReplayBuffer) receives every transition (obs, ego action, reward, next obs, done)
     except the auto-reset steps (see step).
     ``env`` is an F110VecEnv with num_agents == 2 and 'scans_f32' among its outputs; ``policy`` maps the observation
@@ -239,6 +240,7 @@ REWARD_DEFAULTS = dict(dt=0.01, w_prog=1.2, forward_sign=+1.0, alive_bonus=0.02,
 class ShapedReward(object):
     """Batched CenterlineSafetyProgressReward (rewards.py:185-355) on a CenterlineProgress (track_progress.py): one
     independent reward object per env, evaluated by ``f110_reward_compute`` straight from the observation tensor.
+    One centerline for all envs: under a map set (F110VecEnv(maps=...)) it is the centerline of one of the maps only.
 
     ``centerline``: [n, 2] (x_m, y_m) or [n, 4] (+ w_tr_right_m, w_tr_left_m), the CSV train_ddpg.py loads.  Keyword
     arguments are the reference constructor's.  ``__call__(obs, reset_mask=None)`` returns a float64 CUDA tensor [N];

@@ -135,7 +135,8 @@ int f110_abi_version(void);
 /* params: F110_NUM_PARAMS doubles applied to every agent (Simulator.__init__, base_classes.py:504-510).
  * Environment switches read here (development / test aids, none changes a result):
  *   F110_DEBUG_SYNC=1   synchronise after every kernel of a step and name the one that faulted
- *   F110_LIDAR_TILE=1   single-agent handles run the shared-memory tile experiment of the lidar kernel (DESIGN.md section 3)
+ *   F110_LIDAR_TILE=1   single-agent handles run the shared-memory tile experiment of the lidar kernel (DESIGN.md section 3);
+ *                       ignored while a map set of two or more maps is installed (the experiment is single-map only)
  *   F110_LIDAR_HOMES=n  the lidar kernel's units are cut into n home segments with a queue each, in natural order, instead
  *                       of one per SM for launches above 48 units per resident warp and one below (n is clamped to
  *                       [1, units]; changes the order units run in, never a result)
@@ -155,8 +156,42 @@ int f110_set_map_image(F110Sim* sim, const uint8_t* free_mask, int32_t height, i
                        double orig_x, double orig_y, double orig_cos, double orig_sin);
 /* Device time of the EDT kernels of the last f110_set_map_image call on this handle, in ms (CUDA events); 0 before any. */
 float f110_edt_kernel_ms(const F110Sim* sim);
-/* Reads the handle's fp64 map back into dt_host (capacity in cells). */
+/* Reads the handle's fp64 map back into dt_host (capacity in cells).  On a map set: slot 0's map. */
 int f110_get_map(F110Sim* sim, double* dt_host, int64_t capacity_cells);
+
+/* ---- map sets: several maps in one handle, each env driving on the map of its SLOT (DESIGN.md section 10) ----
+ * Every env's dynamics, lidar, iTTC, collisions and observation are exactly what a handle holding only that env's map would
+ * produce, bit for bit.  All maps of a set are padded to ONE fixed-point format, the one the largest side in the set gets
+ * alone (see f110_set_map), and lie back to back in one allocation: each member costs as much device memory as the largest
+ * would.  A set that contains one 8000 x 8000 map pads every member to 8208 x 8192 cells = 538 MB.  The set's padded cells
+ * in all must stay below 2^31 (31 maps when the largest is 8000^2, 127 at 4000^2, 508 at 2000^2).
+ * The shaped reward (f110_reward_*) keeps one centerline per reward object: it does not know about slots. */
+#define F110_MAX_MAPS 256
+typedef struct F110MapDesc {
+    const double*  dt;         /* HOST [height][width] fp64 as f110_set_map takes it, or NULL */
+    const uint8_t* free_mask;  /* HOST [height][width] as f110_set_map_image takes it; used when dt == NULL (device EDT) */
+    int32_t height, width;
+    double resolution, orig_x, orig_y, orig_cos, orig_sin;
+} F110MapDesc;
+/* Installs `count` (1 .. F110_MAX_MAPS) maps at once; maps may differ in size, resolution and origin.  Afterwards env e
+ * drives on slot floor(e * count / N) (contiguous blocks, which keep the lidar kernel's home-segment locality).  Atomic: on
+ * any failure (F110_ERR_INVALID for bad arguments or a set too large, F110_ERR_CUDA for out of memory) the handle keeps
+ * the map or maps it had.  Bumps f110_map_generation.  A set of one map is f110_set_map / f110_set_map_image of that map,
+ * and f110_set_map / f110_set_map_image on a handle holding a set replace the set with that one map. */
+int f110_set_maps(F110Sim* sim, const F110MapDesc* maps, int32_t count);
+/* Maps installed: 1 for a single map, 0 before any. */
+int32_t f110_map_count(const F110Sim* sim);
+/* Reads map `slot` back like f110_get_map; slot outside [0, f110_map_count) -> F110_ERR_INDEX. */
+int f110_get_map_slot(F110Sim* sim, int32_t slot, double* dt_host, int64_t capacity_cells);
+/* Slot assignment, stream-ordered (capturable into a CUDA graph; does NOT bump f110_map_generation).  slots DEVICE int32
+ * [N], env_mask DEVICE uint8 [N] or NULL (= all); entries outside [0, count) leave that env's slot unchanged.  An env whose
+ * slot changes without a reset goes on from the same coordinates on the other map (as the reference's update_map does);
+ * reset it in the same step to start it anew.  The assignment is not part of the f110_get_state blob. */
+int f110_set_env_maps(F110Sim* sim, const int32_t* slots, const uint8_t* env_mask, void* stream);
+/* The same from HOST arrays: validates first (an entry out of range -> F110_ERR_INDEX, nothing changed), copies, synchronises. */
+int f110_set_env_maps_host(F110Sim* sim, const int32_t* slots, const uint8_t* env_mask);
+/* slots_out: DEVICE int32 [N] <- each env's slot, stream-ordered. */
+int f110_get_env_maps(F110Sim* sim, int32_t* slots_out, void* stream);
 /* HOST [theta_dis] tables (laser_models.py:379-381). */
 int f110_set_tables(F110Sim* sim, const double* sines, const double* cosines);
 /* HOST [B] tables (base_classes.py:125-158).  scan_angles must be strictly increasing. */
@@ -215,7 +250,7 @@ int64_t f110_redone_rays(const F110Sim* sim);
  * both the low half of %globaltimer; longest ray in lookups | lanes redone exactly << 24; sm << 24 | queue position).  out == NULL returns the number
  * of units (0 when no timeline is kept); otherwise copies [units][4] words and returns the count, or a negative error. */
 int64_t f110_debug_unit_timeline(F110Sim* sim, uint32_t* out, int64_t capacity_units);
-/* Incremented by every successful f110_set_map / f110_set_map_image.  The step kernels receive the map descriptor by
+/* Incremented by every successful f110_set_map / f110_set_map_image / f110_set_maps (not by f110_set_env_maps).  The step kernels receive the map descriptor by
  * value, so a CUDA graph captured from f110_step before a map change still holds the old (freed) map: re-capture when
  * this number has changed (F110VecEnv does). */
 int64_t f110_map_generation(const F110Sim* sim);
