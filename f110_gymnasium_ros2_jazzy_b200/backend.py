@@ -400,6 +400,13 @@ class BatchSim(object):
         self.redone_rays = int(self.lib.f110_redone_rays(self.h))
         return a.value, b.value
 
+    def lidar_variant(self):
+        """The lidar kernel variant the last step ran (f110_get_lidar_variant): dict with fraction_bits, template_fb (0 =
+        generic), mode (0..3), maps (a map set's kernel) and tile (the tile kernel)."""
+        v = np.zeros(5, np.int32)
+        _lib.check(self.lib.f110_get_lidar_variant(self.h, v.ctypes.data_as(C.c_void_p)))
+        return dict(zip(('fraction_bits', 'template_fb', 'mode', 'maps', 'tile'), (int(x) for x in v)))
+
     @property
     def kernel_launches(self):
         return int(self.lib.f110_kernel_launches(self.h))

@@ -86,6 +86,8 @@ struct F110Sim {
     unsigned long long max_lookups = 0;   // longest ray (lookups) seen, refreshed by f110_get_lookup_count
     unsigned long long redone_rays = 0;   // rays the lidar kernel redid in exact arithmetic, refreshed likewise
     int lidar_blocks = 0;         // CTAs of one resident wave of the lidar kernel (persistent warps)
+    int32_t lidar_variant[5] = {0, 0, 0, 0, 0};   // what the last launch_lidar selected (f110_get_lidar_variant)
+    bool lidar_ran = false;
     std::vector<cudaEvent_t> tev;   // 4 events per timed step
     uint64_t ckpt_header_words[8] = {0};   // host staging of the checkpoint header (see f110_get_state)
     EdtScratch edt;               // f110_set_map_image's device scratch, kept between calls
@@ -177,7 +179,9 @@ int run_step(F110Sim* sim, const F110StepIO& io, cudaStream_t s) {
     CUDA_TRY(launch_dynamics(sim->c, sim->map, sim->st, sim->sc, io, ms, s));
     DEBUG_SYNC("dynamics_kernel")
     if (sim->timing) CUDA_TRY(cudaEventRecord(e[1], s));
-    CUDA_TRY(launch_lidar(sim->c, sim->map, sim->st, sim->sc, io, ms, sim->count_lookups, sim->lidar_blocks, sim->lidar_tile, s));
+    CUDA_TRY(launch_lidar(sim->c, sim->map, sim->st, sim->sc, io, ms, sim->count_lookups, sim->lidar_blocks, sim->lidar_tile,
+                          sim->lidar_variant, s));
+    sim->lidar_ran = true;
     DEBUG_SYNC("lidar_kernel")
     if (sim->timing) CUDA_TRY(cudaEventRecord(e[2], s));
     CUDA_TRY(launch_post(sim->c, sim->st, sim->sc, io, s));
@@ -934,6 +938,12 @@ int f110_get_kernel_timing(F110Sim* sim, double* ms3, int64_t* steps) {
 
 int64_t f110_max_lookups(const F110Sim* sim) { return sim ? (int64_t)sim->max_lookups : 0; }
 int64_t f110_redone_rays(const F110Sim* sim) { return sim ? (int64_t)sim->redone_rays : 0; }
+int f110_get_lidar_variant(const F110Sim* sim, int32_t out[5]) {
+    if (!sim || !out) return fail(F110_ERR_INVALID, "null argument");
+    if (!sim->lidar_ran) return fail(F110_ERR_INVALID, "no step has run on this handle yet");
+    memcpy(out, sim->lidar_variant, sizeof(sim->lidar_variant));
+    return F110_OK;
+}
 int64_t f110_map_generation(const F110Sim* sim) { return sim ? sim->map_generation : 0; }
 
 int64_t f110_kernel_launches(const F110Sim* sim) { return sim ? sim->launches : 0; }

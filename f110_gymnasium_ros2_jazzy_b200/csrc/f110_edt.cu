@@ -30,8 +30,9 @@ namespace {
 
 constexpr int BAND = 64;
 
+// any_obstacle: set to 1 when the band holds an obstacle (the caller clears it)
 __global__ void __launch_bounds__(128) edt_band_masks_kernel(const uint8_t* __restrict__ freemask, int H, int W,
-                                                             unsigned long long* __restrict__ words) {
+                                                             unsigned long long* __restrict__ words, unsigned* __restrict__ any_obstacle) {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= W) return;
     const int r0 = blockIdx.y * BAND;
@@ -42,6 +43,8 @@ __global__ void __launch_bounds__(128) edt_band_masks_kernel(const uint8_t* __re
         if (r < H && freemask[(size_t)r * W + c] == 0) m |= 1ull << j;
     }
     words[(size_t)blockIdx.y * W + c] = m;
+    const unsigned active = __activemask();
+    if (__any_sync(active, m != 0ull) && (threadIdx.x & 31u) == (unsigned)(__ffs(active) - 1)) *any_obstacle = 1u;
 }
 
 // g(row, column) = distance along the column to the nearest obstacle (0 on one), `inf` if the column has none
@@ -127,13 +130,22 @@ __global__ void __launch_bounds__(32) edt_envelope_kernel(const uint16_t* __rest
 
 constexpr int FILL_THREADS = 256;
 
+// A mask without any obstacle: scipy's distance_transform_edt then measures every pixel from a virtual obstacle at
+// (-1, 0), just outside the first row (checked against scipy 1.18 at several shapes): d2 = (row + 1)^2 + column^2.
+__device__ __forceinline__ void edt_fill_row_without_obstacle(int r, int W, int x0, int step, double resolution, double* out) {
+    for (int x = x0; x < W; x += step)
+        out[x] = resolution * sqrt((double)((long long)(r + 1) * (r + 1) + (long long)x * x));
+}
+
 // marks -> owning entry of every cell (running maximum along the row: stack indices grow with t) -> distance
 __global__ void __launch_bounds__(FILL_THREADS) edt_fill_kernel(const uint2* __restrict__ stacks, const uint16_t* __restrict__ marks,
-                                                                int W, int Wp, double resolution, double* __restrict__ dt) {
+                                                                int W, int Wp, double resolution, const unsigned* __restrict__ any_obstacle,
+                                                                double* __restrict__ dt) {
     const int r = blockIdx.x;
     const uint2* st = stacks + (size_t)r * W;
     const uint16_t* mk = marks + (size_t)r * Wp;
     double* out = dt + (size_t)r * W;
+    if (*any_obstacle == 0u) { edt_fill_row_without_obstacle(r, W, threadIdx.x, FILL_THREADS, resolution, out); return; }
     __shared__ unsigned s_warp[FILL_THREADS / 32];
     __shared__ unsigned s_carry;
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
@@ -176,7 +188,8 @@ __global__ void __launch_bounds__(FILL_THREADS) edt_fill_kernel(const uint2* __r
 }
 
 // ---- the general form for maps beyond the 16-bit fast path (H + W + 1 > 32767): one thread per column, then one per row
-__global__ void edt_columns_wide_kernel(const uint8_t* __restrict__ freemask, int H, int W, int* __restrict__ g, int inf) {
+__global__ void edt_columns_wide_kernel(const uint8_t* __restrict__ freemask, int H, int W, int* __restrict__ g, int inf,
+                                        unsigned* __restrict__ any_obstacle) {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= W) return;
     int d = inf;
@@ -184,6 +197,7 @@ __global__ void edt_columns_wide_kernel(const uint8_t* __restrict__ freemask, in
         d = freemask[(size_t)r * W + c] ? (d < inf ? d + 1 : inf) : 0;
         g[(size_t)r * W + c] = d;
     }
+    if (d < inf) *any_obstacle = 1u;    // the column holds an obstacle
     d = inf;
     for (int r = H - 1; r >= 0; --r) {
         d = freemask[(size_t)r * W + c] ? (d < inf ? d + 1 : inf) : 0;
@@ -195,9 +209,10 @@ __global__ void edt_columns_wide_kernel(const uint8_t* __restrict__ freemask, in
 __device__ __forceinline__ long long parab(long long x, long long i, long long gi) { return (x - i) * (x - i) + gi * gi; }
 
 __global__ void edt_rows_wide_kernel(const int* __restrict__ g, int H, int W, int* __restrict__ s_all, int* __restrict__ t_all,
-                                     double resolution, double* __restrict__ dt) {
+                                     double resolution, const unsigned* __restrict__ any_obstacle, double* __restrict__ dt) {
     const int r = blockIdx.x * blockDim.x + threadIdx.x;
     if (r >= H) return;
+    if (*any_obstacle == 0u) { edt_fill_row_without_obstacle(r, W, 0, 1, resolution, dt + (size_t)r * W); return; }
     const int* gr = g + (size_t)r * W;
     int* s = s_all + (size_t)r * W;
     int* t = t_all + (size_t)r * W;
@@ -249,6 +264,8 @@ int edt_device(const uint8_t* freemask, int H, int W, double resolution, double*
     } else {
         need = 3 * cells * sizeof(int);
     }
+    const size_t off_any = align_up(need, 256);   // one word: does the mask hold any obstacle
+    need = off_any + sizeof(unsigned);
     if (sc->bytes < need) {
         if (sc->base) cudaFree(sc->base);
         sc->base = nullptr; sc->bytes = 0;
@@ -261,7 +278,9 @@ int edt_device(const uint8_t* freemask, int H, int W, double resolution, double*
         sc->ev0 = a; sc->ev1 = b;
     }
     char* base = static_cast<char*>(sc->base);
+    unsigned* any_obstacle = reinterpret_cast<unsigned*>(base + off_any);
     cudaEventRecord((cudaEvent_t)sc->ev0, stream);
+    cudaMemsetAsync(any_obstacle, 0, sizeof(unsigned), stream);
     if (narrow) {
         unsigned long long* words = reinterpret_cast<unsigned long long*>(base + off_words);
         uint16_t* gT = reinterpret_cast<uint16_t*>(base + off_g);
@@ -269,16 +288,16 @@ int edt_device(const uint8_t* freemask, int H, int W, double resolution, double*
         uint16_t* marks = reinterpret_cast<uint16_t*>(base + off_marks);
         const unsigned inf = (unsigned)(H + W + 1);    // larger than any real distance
         cudaMemsetAsync(marks, 0, (size_t)H * Wp * sizeof(uint16_t), stream);
-        edt_band_masks_kernel<<<dim3((W + 127) / 128, NB), 128, 0, stream>>>(freemask, H, W, words);
+        edt_band_masks_kernel<<<dim3((W + 127) / 128, NB), 128, 0, stream>>>(freemask, H, W, words, any_obstacle);
         edt_columns_kernel<<<dim3((W + 127) / 128, NB), 128, 0, stream>>>(words, W, NB, Hp, inf, gT);
         edt_envelope_kernel<<<(H + 31) / 32, 32, 0, stream>>>(gT, H, W, Hp, Wp, stacks, marks);
-        edt_fill_kernel<<<H, FILL_THREADS, 0, stream>>>(stacks, marks, W, Wp, resolution, dt);
+        edt_fill_kernel<<<H, FILL_THREADS, 0, stream>>>(stacks, marks, W, Wp, resolution, any_obstacle, dt);
     } else {
         int* g = reinterpret_cast<int*>(base);
         int* s = g + cells;
         int* t = s + cells;
-        edt_columns_wide_kernel<<<(W + 127) / 128, 128, 0, stream>>>(freemask, H, W, g, H + W + 1);
-        edt_rows_wide_kernel<<<(H + 63) / 64, 64, 0, stream>>>(g, H, W, s, t, resolution, dt);
+        edt_columns_wide_kernel<<<(W + 127) / 128, 128, 0, stream>>>(freemask, H, W, g, H + W + 1, any_obstacle);
+        edt_rows_wide_kernel<<<(H + 63) / 64, 64, 0, stream>>>(g, H, W, s, t, resolution, any_obstacle, dt);
     }
     cudaEventRecord((cudaEvent_t)sc->ev1, stream);
     const cudaError_t e = cudaStreamSynchronize(stream);

@@ -1367,12 +1367,18 @@ cudaError_t probe_sm_ids(unsigned char* seen) {
 typedef void (*LidarTileKernel)(SimConst, MapView, SimState, StepScratch, F110StepIO);
 
 cudaError_t launch_lidar(const SimConst& c, const MapView& m, const SimState& st, const StepScratch& sc, const F110StepIO& io,
-                         const MapSet* ms, bool count_lookups, int resident_blocks, bool tile_experiment, cudaStream_t s) {
+                         const MapSet* ms, bool count_lookups, int resident_blocks, bool tile_experiment, int32_t* variant,
+                         cudaStream_t s) {
     // TUNED variant: compile-time fraction bits, d > 0 for d > eps, max_range 30, the observation's division by 30 through its
     // reciprocal.  For a map set m carries the set's common fraction bits and the smallest positive cell over all its maps.
     const bool tuned = m.guard == 2u && c.obs_fast_div && c.max_range == 30.0 && c.eps > 0.0 && m.min_positive > c.eps &&
                        m.fx_bits >= 19u && m.fx_bits <= 22u;
-    if (tile_experiment && tuned && c.A == 1 && !count_lookups && !ms) {   // the tile experiment is single-map only
+    const bool lean = !io.noise && !io.scans_f64 && !io.active_mask;
+    const int mode = c.A != 1 ? (lean ? 3 : 0) : (lean && io.obs && !io.scans_f32) ? 2 : 1;
+    const bool tile = tile_experiment && tuned && c.A == 1 && !count_lookups && !ms;   // the tile experiment is single-map only
+    variant[0] = (int32_t)m.fx_bits; variant[1] = tuned ? (int32_t)m.fx_bits : 0; variant[2] = mode;
+    variant[3] = ms ? 1 : 0; variant[4] = tile ? 1 : 0;
+    if (tile) {
         LidarTileKernel k = m.fx_bits == 19u ? lidar_tile_kernel<19> : m.fx_bits == 20u ? lidar_tile_kernel<20> :
                             m.fx_bits == 21u ? lidar_tile_kernel<21> : lidar_tile_kernel<22>;
         int dev = 0, sms = 148;
@@ -1384,8 +1390,6 @@ cudaError_t launch_lidar(const SimConst& c, const MapView& m, const SimState& st
     // one wave of persistent warps, or fewer when there are not that many units
     const unsigned want = (sc.num_units + LIDAR_THREADS / 32 - 1) / (LIDAR_THREADS / 32);
     const unsigned blocks = want < (unsigned)resident_blocks ? want : (unsigned)resident_blocks;
-    const bool lean = !io.noise && !io.scans_f64 && !io.active_mask;
-    const int mode = c.A != 1 ? (lean ? 3 : 0) : (lean && io.obs && !io.scans_f32) ? 2 : 1;
     if (ms)
         return launch_pdl(lidar_maps_variant(tuned ? (int)m.fx_bits : 0, count_lookups, mode), dim3(blocks ? blocks : 1u),
                           dim3(LIDAR_THREADS), 0, s, c, m, st, sc, io, *ms);

@@ -246,6 +246,12 @@ int64_t f110_max_lookups(const F110Sim* sim);
 /* Rays the lidar kernel redid in the reference's own arithmetic because its fixed-point march met a lookup it could not
  * decide (cell-edge guard band, map border and beyond, non-finite pose), as of the last f110_get_lookup_count call. */
 int64_t f110_redone_rays(const F110Sim* sim);
+/* The lidar kernel variant the last step selected (host-side record, no synchronisation): out[0] the fraction bits of
+ * the map (of the set's common format), out[1] the template fraction bits (19..22 for a tuned variant, 0 for the generic
+ * one), out[2] the mode (0 opponents, 1 single agent, 2 single agent lean, 3 opponents lean; for the tile kernel the
+ * single-agent mode the launch had), out[3] 1 when a map set's kernel ran, out[4] 1 when the tile kernel ran.
+ * F110_ERR_INVALID before the first step. */
+int f110_get_lidar_variant(const F110Sim* sim, int32_t out[5]);
 /* Development aid (requires F110_FLAG_COUNT_LOOKUPS): per work unit of the last lidar launch, 4 words (start ns, end ns,
  * both the low half of %globaltimer; longest ray in lookups | lanes redone exactly << 24; sm << 24 | queue position).  out == NULL returns the number
  * of units (0 when no timeline is kept); otherwise copies [units][4] words and returns the count, or a negative error. */

@@ -74,6 +74,89 @@ def tables():
     return m['sines'], m['cosines'], m['scan_angles'], m['beam_cosines'], m['side_distances']
 
 
+FOV, THETA_DIS = 4.7, 2000
+# Yaws whose np.cos / np.sin equal libm's: the handle gets the origin's cos / sin from numpy, the oracle from libm
+SYNTH_YAWS = (0.0, 0.3, np.pi / 2, -1.5708, np.pi, 2.5)
+# Thin synthetic maps at both ends of every fixed-point width of the lidar kernel's march, 32 - bit_length(side + 1)
+# capped at 24 (f110_capi.cu fixed_point_format): name -> (long side, short side, resolution, long side vertical, origin)
+SYNTH_MAPS = {
+    'w24_200': (200, 48, 0.05, False, (-3.0, 2.0, 0.0)),
+    'w23_254': (254, 64, 0.1, True, (4.5e5, 5.4e6, 0.3)),
+    'w22_511': (511, 48, 0.025, False, (-12.0, -1.0, np.pi / 2)),
+    'w22_1022': (1022, 80, 0.04, True, (100.0, -250.0, -1.5708)),
+    'w21_1500': (1500, 96, 0.05, False, (4.5e5, 5.4e6, np.pi)),
+    'w20_4094': (4094, 56, 0.05, False, (-40.0, 7.5, 2.5)),
+    'w19_4095': (4095, 48, 0.1, True, (0.0, 0.0, 0.0)),
+    'w19_8190': (8190, 64, 0.025, False, (4.5e5, 5.4e6, 0.3)),
+    'w18_8191': (8191, 48, 0.05, True, (-7.0, 3.0, np.pi / 2)),
+    'w17_16383': (16383, 48, 0.1, False, (4.5e5, 5.4e6, 2.5)),
+    'w17_20000': (20000, 48, 0.03, True, (-1.0e3, 2.0e3, np.pi)),
+}
+
+
+def fraction_bits(side):
+    """The lidar march's fixed-point fraction bits for a map (or map set) whose larger side is `side` cells."""
+    return min(24, 32 - int(side + 1).bit_length())
+
+
+@functools.lru_cache(maxsize=None)
+def synthetic_map(name):
+    """-> (free mask bool [H, W], dt fp64 [H, W] = resolution * scipy EDT, resolution, origin).  Border walls with a gap in
+    the far end wall (rays leave the map through it), boxes and single-cell obstacles in the first 40 % of the long axis,
+    and a free run after them (rays reach max_range where the map is long enough)."""
+    from scipy.ndimage import distance_transform_edt
+    side, thick, res, vertical, origin = SYNTH_MAPS[name]
+    rng = np.random.default_rng(side)
+    free = np.ones((thick, side), bool)
+    free[0, :] = free[-1, :] = free[:, 0] = free[:, -1] = False
+    free[thick // 3:2 * thick // 3, -1] = True
+    region = max(8, int(0.4 * side))
+    for _ in range(max(2, side // 150)):
+        h, w = rng.integers(2, thick // 4), rng.integers(2, 12)
+        r, c = rng.integers(2, thick - 2 - h), rng.integers(2, region - w)
+        free[r:r + h, c:c + w] = False
+    for _ in range(max(4, side // 60)):
+        free[rng.integers(2, thick - 2), rng.integers(2, region)] = False
+    if vertical:
+        free = np.ascontiguousarray(free.T)
+    dt = res * distance_transform_edt(np.where(free, 255., 0.))
+    return free, dt, res, tuple(origin)
+
+
+def synthetic_poses(name, n_free=6, seed=0):
+    """World-frame poses [n, 3] on synthetic map `name`: exact cell corners and edge midpoints in the map frame, free cells,
+    an obstacle cell, the map border, outside the map on every side and beyond the far corner, and headings on exact
+    theta-table indices; yaws from SYNTH_YAWS otherwise."""
+    free, _, res, origin = synthetic_map(name)
+    H, W = free.shape
+    rng = np.random.default_rng(seed)
+    ok = free.copy()
+    ok[:-1] &= free[1:]; ok[:, :-1] &= free[:, 1:]; ok[1:] &= free[:-1]; ok[:, 1:] &= free[:, :-1]
+    cells = np.argwhere(ok)
+    pick = cells[rng.integers(0, len(cells), n_free)]
+    m = []                                             # map-frame (x, y)
+    for k, (r, c) in enumerate(pick):
+        m.append((c * res, r * res) if k % 3 == 0 else (c * res + 0.5 * res, r * res) if k % 3 == 1 else
+                 (c * res + rng.uniform(0, res), r * res + rng.uniform(0, res)))
+    occ = np.argwhere(~free[1:-1, 1:-1]) + 1
+    r, c = occ[len(occ) // 2]
+    m.append(((c + 0.5) * res, (r + 0.5) * res))       # inside an obstacle
+    m += [(0.0, H * res / 2), (W * res / 2, 0.0), (0.5 * res, 0.5 * res)]          # on the border
+    m += [(-0.5, H * res / 2), (W * res + 0.5, H * res / 2), (W * res / 2, -0.5), (W * res / 2, H * res + 0.5),
+          (W * res + 1.0, H * res + 1.0)]              # outside, every side, and beyond the far corner
+    yaws = [SYNTH_YAWS[k % len(SYNTH_YAWS)] for k in range(len(m))]
+    # the free run, looking along the long axis towards the gap in the end wall: from its start and from near its end
+    for f in (0.42, 0.97):
+        m.append((f * W * res, (H / 2 + 0.25) * res) if W > H else ((W / 2 + 0.25) * res, f * H * res))
+        yaws.append(0.0 if W > H else np.pi / 2)
+    m, yaws = np.array(m, np.float64), np.array(yaws)
+    co, so = np.cos(origin[2]), np.sin(origin[2])
+    out = np.stack([origin[0] + co * m[:, 0] - so * m[:, 1], origin[1] + so * m[:, 0] + co * m[:, 1], yaws + origin[2]], 1)
+    # headings on exact theta-table indices: theta_dis * (yaw - fov / 2) / (2 pi) an integer
+    out[1::4, 2] = FOV / 2 + 2 * np.pi * rng.integers(0, THETA_DIS, len(out[1::4])) / THETA_DIS
+    return out
+
+
 def noise_stream(seed, steps, beams=1080, expect_sha=None):
     """The reference's lidar noise: one Generator.normal(0, 0.01, beams) per agent per step, every agent
     seeded identically (base_classes.py:204, laser_models.py:450-452) -> [steps, beams]."""
