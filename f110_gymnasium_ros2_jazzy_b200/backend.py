@@ -402,10 +402,10 @@ class BatchSim(object):
 
     def lidar_variant(self):
         """The lidar kernel variant the last step ran (f110_get_lidar_variant): dict with fraction_bits, template_fb (0 =
-        generic), mode (0..3), maps (a map set's kernel) and tile (the tile kernel)."""
-        v = np.zeros(5, np.int32)
+        generic), mode (0..3) and maps (a map set's kernel)."""
+        v = np.zeros(4, np.int32)
         _lib.check(self.lib.f110_get_lidar_variant(self.h, v.ctypes.data_as(C.c_void_p)))
-        return dict(zip(('fraction_bits', 'template_fb', 'mode', 'maps', 'tile'), (int(x) for x in v)))
+        return dict(zip(('fraction_bits', 'template_fb', 'mode', 'maps'), (int(x) for x in v)))
 
     @property
     def kernel_launches(self):

@@ -67,7 +67,6 @@ struct F110Sim {
     bool count_lookups = false;
     bool narrow_fraction = false;
     bool debug_sync = false;
-    bool lidar_tile = false;      // F110_LIDAR_TILE=1: the shared-memory tile experiment of the lidar kernel (see lidar_tile_kernel)
     // device memory
     char* state_blob = nullptr;   size_t state_bytes = 0;    // checkpointable
     char* scratch_blob = nullptr; size_t scratch_bytes = 0;
@@ -86,7 +85,7 @@ struct F110Sim {
     unsigned long long max_lookups = 0;   // longest ray (lookups) seen, refreshed by f110_get_lookup_count
     unsigned long long redone_rays = 0;   // rays the lidar kernel redid in exact arithmetic, refreshed likewise
     int lidar_blocks = 0;         // CTAs of one resident wave of the lidar kernel (persistent warps)
-    int32_t lidar_variant[5] = {0, 0, 0, 0, 0};   // what the last launch_lidar selected (f110_get_lidar_variant)
+    int32_t lidar_variant[4] = {0, 0, 0, 0};   // what the last launch_lidar selected (f110_get_lidar_variant)
     bool lidar_ran = false;
     std::vector<cudaEvent_t> tev;   // 4 events per timed step
     uint64_t ckpt_header_words[8] = {0};   // host staging of the checkpoint header (see f110_get_state)
@@ -179,8 +178,7 @@ int run_step(F110Sim* sim, const F110StepIO& io, cudaStream_t s) {
     CUDA_TRY(launch_dynamics(sim->c, sim->map, sim->st, sim->sc, io, ms, s));
     DEBUG_SYNC("dynamics_kernel")
     if (sim->timing) CUDA_TRY(cudaEventRecord(e[1], s));
-    CUDA_TRY(launch_lidar(sim->c, sim->map, sim->st, sim->sc, io, ms, sim->count_lookups, sim->lidar_blocks, sim->lidar_tile,
-                          sim->lidar_variant, s));
+    CUDA_TRY(launch_lidar(sim->c, sim->map, sim->st, sim->sc, io, ms, sim->count_lookups, sim->lidar_blocks, sim->lidar_variant, s));
     sim->lidar_ran = true;
     DEBUG_SYNC("lidar_kernel")
     if (sim->timing) CUDA_TRY(cudaEventRecord(e[2], s));
@@ -229,7 +227,6 @@ int f110_create(const F110Config* cfg, const double* params, F110Sim** out) {
     sim->count_lookups = (cfg->flags & F110_FLAG_COUNT_LOOKUPS) != 0;
     sim->narrow_fraction = (cfg->flags & F110_FLAG_NARROW_FRACTION) != 0;
     sim->debug_sync = getenv("F110_DEBUG_SYNC") != nullptr;
-    { const char* t = getenv("F110_LIDAR_TILE"); sim->lidar_tile = t && t[0] == '1'; }
     sim->lidar_blocks = lidar_resident_blocks(A == 1);
     sim->sc.ordered = 0;   // set below, once the unit count is known
     if (sim->lidar_blocks < 1) {
@@ -938,7 +935,7 @@ int f110_get_kernel_timing(F110Sim* sim, double* ms3, int64_t* steps) {
 
 int64_t f110_max_lookups(const F110Sim* sim) { return sim ? (int64_t)sim->max_lookups : 0; }
 int64_t f110_redone_rays(const F110Sim* sim) { return sim ? (int64_t)sim->redone_rays : 0; }
-int f110_get_lidar_variant(const F110Sim* sim, int32_t out[5]) {
+int f110_get_lidar_variant(const F110Sim* sim, int32_t out[4]) {
     if (!sim || !out) return fail(F110_ERR_INVALID, "null argument");
     if (!sim->lidar_ran) return fail(F110_ERR_INVALID, "no step has run on this handle yet");
     memcpy(out, sim->lidar_variant, sizeof(sim->lidar_variant));

@@ -533,10 +533,6 @@ constexpr unsigned LIDAR_CHUNK = LIDAR_CHUNK_OVERRIDE;   // queue positions a wa
 // and the step count (all three are indexed from the unit alone); the slot's cell base is arithmetic from it (the blocks
 // lie at a fixed stride), its direction table one level later, as the table of a single map is; the exact path reads the
 // slot's MapView from global memory.  Everything else -- queue, lists, home segments -- is the single-map kernel's.
-#ifndef F110_MAPS_OFF32
-#define F110_MAPS_OFF32 0      // 1: the slot's base as a 32-bit cell offset added to every lookup's index (no faster: profiles/r04_multimap_off32.json)
-#endif
-
 template <int FB, bool COUNT, int MODE>
 __global__ void __launch_bounds__(LIDAR_THREADS, LIDAR_MIN_BLOCKS)
 lidar_kernel(const __grid_constant__ SimConst c, const __grid_constant__ MapView m, const __grid_constant__ SimState st,
@@ -553,154 +549,6 @@ lidar_maps_kernel(const __grid_constant__ SimConst c, const __grid_constant__ Ma
                   const __grid_constant__ StepScratch sc, const __grid_constant__ F110StepIO io, const __grid_constant__ MapSet ms) {
     constexpr bool MAPS = true;
 #include "f110_lidar_body.cuh"
-}
-
-// ---------------------------------------------------------------- K2, experiment: the car's neighbourhood in shared memory
-//
-// north_star item (2): "TMA-staged shared-memory tiles where it fits".  Selected by F110_LIDAR_TILE=1 (single-agent, tuned
-// maps only); NOT the default -- profiles/r02_tile_experiment.md has the measurement that decides it.
-// A CTA takes whole scans (a tile belongs to one car).  Per scan, warp 0 has the copy engine bring the 65 x 66 cells around
-// the car (33.5 KB; +-2.1 m on the default map, 45 % of the lookups after the first, profiles/r02_tile_study.md) into shared
-// memory -- one cp.async.bulk per row completing on an mbarrier, no thread touches the data -- and the CTA's eight warps
-// then march the scan's 34 units, a lookup inside the tile reading shared memory, any other the map as before.  Same
-// arithmetic as lidar_kernel (same march, same exact path for undecided lookups), so the scans are bit-identical.
-// What it gives up: the warp-granular longest-first queue (a CTA is tied to its scan until the scan's longest ray is done).
-#ifndef TILE_T_OVERRIDE
-#define TILE_T_OVERRIDE 32
-#endif
-constexpr int TILE_T = TILE_T_OVERRIDE;      // half-width in cells
-constexpr int TILE_ROWS = 2 * TILE_T + 1;
-constexpr int TILE_COLS = 2 * TILE_T + 2;    // rows of 528 bytes: the bulk copy moves multiples of 16
-constexpr int TILE_THREADS = 256;
-constexpr int TILE_MIN_BLOCKS = 6;
-
-__device__ __forceinline__ unsigned smem_addr(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-
-template <int FB>
-__global__ void __launch_bounds__(TILE_THREADS, TILE_MIN_BLOCKS)
-lidar_tile_kernel(const __grid_constant__ SimConst c, const __grid_constant__ MapView m, const __grid_constant__ SimState st,
-                  const __grid_constant__ StepScratch sc, const __grid_constant__ F110StepIO io) {
-    cudaGridDependencySynchronize();
-    __shared__ __align__(128) double tile[TILE_ROWS * TILE_COLS];
-    __shared__ __align__(8) unsigned long long mbar;
-    constexpr int pitch = (1 << (32 - FB)) + 16, prows = 1 << (32 - FB);
-    constexpr unsigned gm = ((1u << FB) - 1u) & ~3u;
-    const unsigned lane = threadIdx.x & 31u, wid = threadIdx.x >> 5;
-    const double* __restrict__ dt = m.dt;
-    if (threadIdx.x == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_addr(&mbar)) : "memory");
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    unsigned phase = 0;
-    for (unsigned s = blockIdx.x; s < (unsigned)c.NA; s += gridDim.x) {
-        const double4 head = reinterpret_cast<const double4*>(sc.head)[s];   // fixed-point start X, Y; theta index of beam 0; iTTC limit
-        const unsigned hx = __double2uint_rz(head.x), hy = __double2uint_rz(head.y);
-        int c0 = (int)(hx >> FB) - TILE_T, r0 = (int)(hy >> FB) - TILE_T;
-        c0 = c0 < 0 ? 0 : (c0 > pitch - TILE_COLS ? pitch - TILE_COLS : c0);
-        c0 &= ~1;                                                            // 16-byte aligned row starts
-        r0 = r0 < 0 ? 0 : (r0 > prows - TILE_ROWS ? prows - TILE_ROWS : r0);
-        if (wid == 0) {
-            if (lane == 0)
-                asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_addr(&mbar)), "r"(TILE_ROWS * TILE_COLS * 8) : "memory");
-            __syncwarp();
-            for (int r = (int)lane; r < TILE_ROWS; r += 32) {
-                const double* src = dt + ((size_t)(r0 + r) * pitch + c0);
-                asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                             ::"r"(smem_addr(tile + r * TILE_COLS)), "l"(src), "r"(TILE_COLS * 8), "r"(smem_addr(&mbar)) : "memory");
-            }
-        }
-        {
-            unsigned done = 0, spins = 0;
-            while (!done) {
-                asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
-                             : "=r"(done) : "r"(smem_addr(&mbar)), "r"(phase) : "memory");
-                if (++spins > (1u << 22)) __trap();      // a copy that never lands must not hang the device
-            }
-            phase ^= 1u;
-        }
-        const unsigned env = s;      // single-agent only
-        const bool active = !(io.active_mask && !io.active_mask[env]);
-        const unsigned stepc = st.step_count[env];
-        for (unsigned k = wid; k < c.ups; k += TILE_THREADS / 32) {
-            const unsigned i = k * 32u + lane;
-            const bool live = i < (unsigned)c.B && active;
-            const unsigned ic = i < (unsigned)c.B ? i : (unsigned)c.B - 1u;
-            // beam direction: as in lidar_kernel (laser_models.py:174-184)
-            const double td = (double)c.theta_dis;
-            double t = head.z + (double)ic * c.theta_inc;
-            if (t >= td) t -= td;
-            if (fabs(t - rint(t)) < 1e-9 || t >= td) {
-                t = head.z;
-                for (unsigned q = 0; q < ic; ++q) {
-                    t += c.theta_inc;
-                    while (t >= td) t -= td;
-                }
-            }
-            int ti = (int)t;
-            ti = (unsigned)ti < (unsigned)c.theta_dis ? ti : c.theta_dis - 1;
-            const double2 dir = __ldg(c.dir_fx + ti);
-            const double ttc_lim = head.w;
-
-            double X = head.x, Y = head.y, total_d = 0.0, d = 0.0;
-            bool decided = true;
-            if (live) {
-                unsigned ux = hx, uy = hy, tx, ty;
-                auto cell = [&](unsigned ax, unsigned ay) -> double {
-                    const int cx = (int)(ax >> FB), cy = (int)(ay >> FB);
-                    const unsigned tc = (unsigned)(cx - c0), tr = (unsigned)(cy - r0);
-                    if (tr < (unsigned)TILE_ROWS && tc < (unsigned)TILE_COLS) return tile[tr * TILE_COLS + tc];
-                    return __ldg(dt + (cy * pitch + cx));
-                };
-                asm("lop3.b32 %0, %1, %2, 0, 0x0c;" : "=r"(tx) : "r"(ux), "r"(gm));
-                asm("lop3.b32 %0, %1, %2, 0, 0x0c;" : "=r"(ty) : "r"(uy), "r"(gm));
-                decided = tx != 0u && ty != 0u;
-                if (decided) {
-                    double da = cell(ux, uy), db = 0.0;
-                    bool second = false;
-#define F110_TILE_STEP(D_CUR, D_NEXT)                                                              \
-                    X += D_CUR * dir.x;                                                            \
-                    Y += D_CUR * dir.y;                                                            \
-                    ux = __double2uint_rz(X);                                                      \
-                    uy = __double2uint_rz(Y);                                                      \
-                    D_NEXT = cell(ux, uy);                                                         \
-                    total_d += D_CUR;                                                              \
-                    asm("lop3.b32 %0, %1, %2, 0, 0x0c;" : "=r"(tx) : "r"(ux), "r"(gm));            \
-                    asm("lop3.b32 %0, %1, %2, 0, 0x0c;" : "=r"(ty) : "r"(uy), "r"(gm));
-                    for (;;) {
-                        F110_TILE_STEP(da, db)
-                        if (!(da > 0.0 && total_d <= 30.0 && tx != 0u && ty != 0u)) break;
-                        F110_TILE_STEP(db, da)
-                        if (!(db > 0.0 && total_d <= 30.0 && tx != 0u && ty != 0u)) { second = true; break; }
-                    }
-#undef F110_TILE_STEP
-                    d = second ? db : da;
-                    decided = !(d > 0.0 && total_d <= 30.0);
-                }
-            }
-            if (live && (!decided || d < 0.0)) total_d = trace_ray_exact(m, c, sc, s, ti).x;
-            if (total_d > c.max_range) total_d = c.max_range;
-            if (live) {
-                const unsigned r = s * (unsigned)c.B + i, rid = s * (unsigned)(c.B + 8) + i;   // as in lidar_kernel
-                double range = total_d;
-                if (io.noise) {
-                    range += io.noise[r];
-                } else if (c.noise_std > 0.0) {
-                    const uint2 bits = philox2x32_10(make_uint2(rid, stepc), c.philox_key);
-                    range += c.noise_std * (double)gaussian_from_bits(bits.x, bits.y);
-                }
-                if (io.scans_f64) __stcs(io.scans_f64 + r, range);
-                if (io.scans_f32) __stcs(io.scans_f32 + r, (float)range);
-                if (io.obs) __stcs(io.obs + (size_t)s * (c.B + 8) + i, obs_lidar<true>(range, c.lidar_max, c.obs_rcp));
-                if (!(range > ttc_lim)) {
-                    const double2 bt = __ldg(c.beam_tt + i);
-                    const double ttc = (range - bt.y) / (st.x[3][s] * bt.x);
-                    if ((ttc < c.ttc_thresh) && (ttc >= 0.0)) sc.ttc_hit[s] = 1;
-                }
-            }
-        }
-        __syncthreads();      // every lookup of this scan is done before the next tile lands on the buffer
-    }
 }
 
 // ---------------------------------------------------------------- K3: post
@@ -1364,29 +1212,15 @@ cudaError_t probe_sm_ids(unsigned char* seen) {
     return e;
 }
 
-typedef void (*LidarTileKernel)(SimConst, MapView, SimState, StepScratch, F110StepIO);
-
 cudaError_t launch_lidar(const SimConst& c, const MapView& m, const SimState& st, const StepScratch& sc, const F110StepIO& io,
-                         const MapSet* ms, bool count_lookups, int resident_blocks, bool tile_experiment, int32_t* variant,
-                         cudaStream_t s) {
+                         const MapSet* ms, bool count_lookups, int resident_blocks, int32_t* variant, cudaStream_t s) {
     // TUNED variant: compile-time fraction bits, d > 0 for d > eps, max_range 30, the observation's division by 30 through its
     // reciprocal.  For a map set m carries the set's common fraction bits and the smallest positive cell over all its maps.
     const bool tuned = m.guard == 2u && c.obs_fast_div && c.max_range == 30.0 && c.eps > 0.0 && m.min_positive > c.eps &&
                        m.fx_bits >= 19u && m.fx_bits <= 22u;
     const bool lean = !io.noise && !io.scans_f64 && !io.active_mask;
     const int mode = c.A != 1 ? (lean ? 3 : 0) : (lean && io.obs && !io.scans_f32) ? 2 : 1;
-    const bool tile = tile_experiment && tuned && c.A == 1 && !count_lookups && !ms;   // the tile experiment is single-map only
-    variant[0] = (int32_t)m.fx_bits; variant[1] = tuned ? (int32_t)m.fx_bits : 0; variant[2] = mode;
-    variant[3] = ms ? 1 : 0; variant[4] = tile ? 1 : 0;
-    if (tile) {
-        LidarTileKernel k = m.fx_bits == 19u ? lidar_tile_kernel<19> : m.fx_bits == 20u ? lidar_tile_kernel<20> :
-                            m.fx_bits == 21u ? lidar_tile_kernel<21> : lidar_tile_kernel<22>;
-        int dev = 0, sms = 148;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        const unsigned wave = (unsigned)(sms * TILE_MIN_BLOCKS);
-        return launch_pdl(k, dim3((unsigned)c.NA < wave ? (unsigned)c.NA : wave), dim3(TILE_THREADS), 0, s, c, m, st, sc, io);
-    }
+    variant[0] = (int32_t)m.fx_bits; variant[1] = tuned ? (int32_t)m.fx_bits : 0; variant[2] = mode; variant[3] = ms ? 1 : 0;
     // one wave of persistent warps, or fewer when there are not that many units
     const unsigned want = (sc.num_units + LIDAR_THREADS / 32 - 1) / (LIDAR_THREADS / 32);
     const unsigned blocks = want < (unsigned)resident_blocks ? want : (unsigned)resident_blocks;

@@ -134,10 +134,9 @@ cudaError_t launch_dynamics(const SimConst& c, const MapView& m, const SimState&
 int lidar_resident_blocks(bool single_agent);
 // seen[k] = 1 for every SM id k < F110_SMID_TABLE a wave of the device's CTAs ran on (host array); synchronises
 cudaError_t probe_sm_ids(unsigned char* seen);
-// variant[5] (host): what the launch selected, as f110_get_lidar_variant reports it
+// variant[4] (host): what the launch selected, as f110_get_lidar_variant reports it
 cudaError_t launch_lidar(const SimConst& c, const MapView& m, const SimState& st, const StepScratch& sc, const F110StepIO& io,
-                         const MapSet* ms, bool count_lookups, int resident_blocks, bool tile_experiment, int32_t* variant,
-                         cudaStream_t s);
+                         const MapSet* ms, bool count_lookups, int resident_blocks, int32_t* variant, cudaStream_t s);
 // env_map[e] = slots[e] for every env e with (mask == nullptr || mask[e]) and 0 <= slots[e] < count (all DEVICE pointers)
 cudaError_t launch_set_env_maps(int32_t* env_map, const int32_t* slots, const uint8_t* mask, int N, int count, cudaStream_t s);
 // smallest positive value of a dense device map (set_map time); synchronises the stream

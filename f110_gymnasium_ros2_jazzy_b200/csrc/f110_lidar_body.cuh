@@ -157,8 +157,7 @@
                 const double eps = c.eps;
                 const double max_range = TUNED ? 30.0 : c.max_range;   // an immediate: 30.0 has no low mantissa word
                 const size_t stride = TUNED ? (size_t)(1u << (32 - FB)) * (size_t)((1u << (32 - FB)) + 16u) : ms.stride;
-                const double* __restrict__ dt = (MAPS && !F110_MAPS_OFF32) ? m.dt + (size_t)slot * stride : m.dt;
-                const int off = (MAPS && F110_MAPS_OFF32) ? slot * (int)stride : 0;   // < 2^31: f110_set_maps bounds the set
+                const double* __restrict__ dt = MAPS ? m.dt + (size_t)slot * stride : m.dt;
                 // The loop is software-pipelined by one lookup: the cell of the NEXT position is loaded before it is known
                 // whether the ray goes on (any 32-bit fixed-point coordinate addresses a cell of the padded array, so the
                 // load is always safe).  The dependent chain of a lookup is then load -> multiply-add -> convert -> index ->
@@ -178,7 +177,7 @@
                         // lookup per trip, ptxas rotates (d, d_next) through four register moves -- 4 of the loop's 23
                         // instructions.  One exit test per lookup (ray ended OR lookup undecided; told apart after the
                         // loop, where `still going` means undecided), one counter update per trip.
-                        double da = __ldg(dt + (off + (int)(uy >> fb) * pitch + (int)(ux >> fb))), db = 0.0;
+                        double da = __ldg(dt + ((int)(uy >> fb) * pitch + (int)(ux >> fb))), db = 0.0;
                         unsigned trips = 0;
                         bool second = false;
 #define F110_MARCH_STEP(D_CUR, D_NEXT)                                                                         \
@@ -186,7 +185,7 @@
                             Y += D_CUR * dir.y;                                                                \
                             ux = __double2uint_rz(X);                                                          \
                             uy = __double2uint_rz(Y);                                                          \
-                            D_NEXT = __ldg(dt + (off + (int)(uy >> fb) * pitch + (int)(ux >> fb)));            \
+                            D_NEXT = __ldg(dt + ((int)(uy >> fb) * pitch + (int)(ux >> fb)));                  \
                             total_d += D_CUR;                                                                  \
                             asm("lop3.b32 %0, %1, %2, 0, 0x0c;" : "=r"(tx) : "r"(ux), "r"(gm));                \
                             asm("lop3.b32 %0, %1, %2, 0, 0x0c;" : "=r"(ty) : "r"(uy), "r"(gm));

@@ -135,8 +135,6 @@ int f110_abi_version(void);
 /* params: F110_NUM_PARAMS doubles applied to every agent (Simulator.__init__, base_classes.py:504-510).
  * Environment switches read here (development / test aids, none changes a result):
  *   F110_DEBUG_SYNC=1   synchronise after every kernel of a step and name the one that faulted
- *   F110_LIDAR_TILE=1   single-agent handles run the shared-memory tile experiment of the lidar kernel (DESIGN.md section 3);
- *                       ignored while a map set of two or more maps is installed (the experiment is single-map only)
  *   F110_LIDAR_HOMES=n  the lidar kernel's units are cut into n home segments with a queue each, in natural order, instead
  *                       of one per SM for launches above 48 units per resident warp and one below (n is clamped to
  *                       [1, units]; changes the order units run in, never a result)
@@ -248,10 +246,9 @@ int64_t f110_max_lookups(const F110Sim* sim);
 int64_t f110_redone_rays(const F110Sim* sim);
 /* The lidar kernel variant the last step selected (host-side record, no synchronisation): out[0] the fraction bits of
  * the map (of the set's common format), out[1] the template fraction bits (19..22 for a tuned variant, 0 for the generic
- * one), out[2] the mode (0 opponents, 1 single agent, 2 single agent lean, 3 opponents lean; for the tile kernel the
- * single-agent mode the launch had), out[3] 1 when a map set's kernel ran, out[4] 1 when the tile kernel ran.
- * F110_ERR_INVALID before the first step. */
-int f110_get_lidar_variant(const F110Sim* sim, int32_t out[5]);
+ * one), out[2] the mode (0 opponents, 1 single agent, 2 single agent lean, 3 opponents lean), out[3] 1 when a map
+ * set's kernel ran.  F110_ERR_INVALID before the first step. */
+int f110_get_lidar_variant(const F110Sim* sim, int32_t out[4]);
 /* Development aid (requires F110_FLAG_COUNT_LOOKUPS): per work unit of the last lidar launch, 4 words (start ns, end ns,
  * both the low half of %globaltimer; longest ray in lookups | lanes redone exactly << 24; sm << 24 | queue position).  out == NULL returns the number
  * of units (0 when no timeline is kept); otherwise copies [units][4] words and returns the count, or a negative error. */

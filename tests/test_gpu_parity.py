@@ -194,52 +194,6 @@ def test_large_map_scans_golden_and_oracle(name):
         assert d_ref.max() == 0.0
 
 
-def test_tile_experiment_is_bit_identical_to_the_default_kernel():
-    """F110_LIDAR_TILE=1 (lidar_tile_kernel: the car's neighbourhood staged in shared memory by cp.async.bulk, north_star item 2,
-    an experiment -- see profiles/r02_tile_experiment.md) computes the same scans, observations and flags as lidar_kernel:
-    reference scans on Shanghai (tile everywhere inside the map) and a 200-step batched rollout with on-device noise."""
-    _torch()
-    import torch
-    from f110_gymnasium_ros2_jazzy_b200 import ALL_OUTPUTS, BatchSim, workloads
-    g = H.load('scans')
-    poses, ref = g['Shanghai_map__poses'], g['Shanghai_map__scans']
-    dt, res, origin = H.golden_map('Shanghai_map')
-    start = workloads.start_poses(512)
-    rng = np.random.default_rng(7)
-    acts = rng.uniform([-0.4189, 0.0], [0.4189, 12.0], size=(200, 512, 1, 2)).astype(np.float32)
-    runs = {}
-    for mode in ('0', '1'):
-        os.environ['F110_LIDAR_TILE'] = mode
-        try:
-            sim = BatchSim(len(poses), 1, outputs=ALL_OUTPUTS, noise_std=0.0)
-            roll = BatchSim(512, 1, outputs=ALL_OUTPUTS, noise_std=0.01, seed=3)
-        finally:
-            os.environ.pop('F110_LIDAR_TILE')
-        tab_s, tab_c = H.tables()[:2]
-        sim.set_tables(tab_s, tab_c)
-        sim.set_map_arrays(dt, res, origin)
-        sim.sim_reset(poses[:, None, :])
-        scans = sim.step(None, np.zeros((len(poses), 1, 1080)))['scans_f64'].cpu().numpy()[:, 0]
-        sim.close()
-        roll.set_tables(tab_s, tab_c)
-        roll.set_map_arrays(dt, res, origin)
-        out = roll.reset(start)
-        mask = None
-        trace = []
-        for t in range(200):
-            out = roll.step(acts[t], reset_mask=mask, reset_poses=start) if mask is not None else roll.step(acts[t])
-            torch.cuda.synchronize()
-            mask = out['terminated'].clone()
-            trace.append((out['obs'].cpu().numpy().copy(), out['terminated'].cpu().numpy().copy(), out['state'].cpu().numpy().copy()))
-        roll.close()
-        runs[mode] = (scans, trace)
-    assert np.array_equal(runs['1'][0], ref)                     # the reference's own scans
-    assert np.array_equal(runs['0'][0], runs['1'][0])
-    for (o0, t0, s0), (o1, t1, s1) in zip(runs['0'][1], runs['1'][1]):
-        assert np.array_equal(t0, t1) and np.array_equal(s0, s1) and np.array_equal(o0, o1)
-    assert sum(int(t.sum()) for _, t, _ in runs['1'][1]) > 0     # episodes ended and restarted on the way
-
-
 def test_lean_lidar_variants_equal_the_general_one():
     """The lidar kernel has variants without the tests and address arithmetic for outputs that were not asked for (single
     agent: float32 observation only; opponents: no fp64 scan; both: device noise, no env mask).  Same seed, same actions:

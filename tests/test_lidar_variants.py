@@ -1,13 +1,13 @@
 """Every compiled lidar kernel variant against the oracle, at every fixed-point width, and the device EDT at its limits.
 
-launch_lidar picks one of 84 instantiations: lidar_kernel and lidar_maps_kernel <FB, COUNT, MODE> with FB = 19..22 (the
-tuned variants) or 0 (generic), and lidar_tile_kernel<19..22>.  The runs below use thin synthetic maps at both ends of every
-width from 24 down to 17 fraction bits (tests/helpers.py SYNTH_MAPS), map sets at every common width, and handles that
-force the generic variant at tuned widths.  Each run is one reset step, noise-free, and must equal the oracle bit for bit:
+launch_lidar picks one of 80 instantiations: lidar_kernel and lidar_maps_kernel <FB, COUNT, MODE> with FB = 19..22 (the
+tuned variants) or 0 (generic).  The runs below use thin synthetic maps at both ends of every width from 24 down to 17
+fraction bits (tests/helpers.py SYNTH_MAPS), map sets at every common width, and handles that force the generic variant at
+tuned widths.  Each run is one reset step, noise-free, and must equal the oracle bit for bit:
 scans_f64, scans_f32, the observation's lidar channel, terminated and, with lookup counting, the lookup count.  The one
 exception are the beams an opponent lowers (A = 2): they end on the post kernel's ray / edge intersection, not on the lidar
 kernel's march, and are held to 4 ulp.  Every run also checks which variant ran (f110_get_lidar_variant), and the union of
-the variants must be all 84.
+the variants must be all 80.
 """
 import math
 import os
@@ -61,7 +61,7 @@ def _oracle(name, A, eps=1e-4, max_range=30.0):
     return _ORACLE[key]
 
 
-def _run(maps, mode, count, narrow=False, eps=1e-4, max_range=30.0, tile=False, image=False):
+def _run(maps, mode, count, narrow=False, eps=1e-4, max_range=30.0, image=False):
     """One reset step of a fresh handle holding `maps` (one name, or a set) -> (variant, list of mismatches)."""
     import torch
     from f110_gymnasium_ros2_jazzy_b200 import ALL_OUTPUTS, BatchSim
@@ -70,13 +70,8 @@ def _run(maps, mode, count, narrow=False, eps=1e-4, max_range=30.0, tile=False, 
     refs = [_oracle(n, A, eps, max_range) for n in names]
     poses = np.concatenate([_poses(n, A) for n in names])
     slots = np.concatenate([np.full(len(r['terminated']), k, np.int32) for k, r in enumerate(refs)])
-    if tile:
-        os.environ['F110_LIDAR_TILE'] = '1'
-    try:
-        sim = BatchSim(len(poses), A, outputs=outputs or ALL_OUTPUTS, noise_std=0.0, count_lookups=count,
-                       narrow_fraction=narrow, eps=eps, max_range=max_range, device=0)
-    finally:
-        os.environ.pop('F110_LIDAR_TILE', None)
+    sim = BatchSim(len(poses), A, outputs=outputs or ALL_OUTPUTS, noise_std=0.0, count_lookups=count,
+                   narrow_fraction=narrow, eps=eps, max_range=max_range, device=0)
     bad = []
     try:
         if len(names) > 1:
@@ -129,23 +124,19 @@ def _run(maps, mode, count, narrow=False, eps=1e-4, max_range=30.0, tile=False, 
     return variant, bad
 
 
-def _expected(maps, mode, count, narrow=False, eps=1e-4, max_range=30.0, tile=False):
+def _expected(maps, mode, count, narrow=False, eps=1e-4, max_range=30.0):
     fb = H.fraction_bits(max(max(H.synthetic_map(n)[0].shape) for n in maps))
     min_positive = min(H.synthetic_map(n)[2] for n in maps)       # one cell from an obstacle
     tuned = not narrow and max_range == 30.0 and 0 < eps < min_positive and 19 <= fb <= 22
-    single = MODES[mode][0] == 1
-    return dict(fraction_bits=fb, template_fb=fb if tuned else 0, mode=mode, maps=int(len(maps) > 1),
-                tile=int(tile and tuned and single and not count and len(maps) == 1))
+    return dict(fraction_bits=fb, template_fb=fb if tuned else 0, mode=mode, maps=int(len(maps) > 1))
 
 
 def _key(v, count):
-    if v['tile']:
-        return ('lidar_tile_kernel', v['template_fb'], None, None)
     return ('lidar_maps_kernel' if v['maps'] else 'lidar_kernel', v['template_fb'], count, v['mode'])
 
 
-ALL_VARIANTS = ({(k, fb, c, m) for k in ('lidar_kernel', 'lidar_maps_kernel') for fb in (0, 19, 20, 21, 22)
-                 for c in (False, True) for m in range(4)} | {('lidar_tile_kernel', fb, None, None) for fb in (19, 20, 21, 22)})
+ALL_VARIANTS = {(k, fb, c, m) for k in ('lidar_kernel', 'lidar_maps_kernel') for fb in (0, 19, 20, 21, 22)
+                for c in (False, True) for m in range(4)}
 
 
 def _plan():
@@ -154,8 +145,6 @@ def _plan():
         for count in (False, True):
             runs += [((n,), mode, count, {}) for n in sorted(H.SYNTH_MAPS)]
             runs += [(SETS[s], mode, count, {}) for s in sorted(SETS)]
-    for n in ('w19_4095', 'w20_4094', 'w21_1500', 'w22_511', 'w22_1022', 'w19_8190'):
-        runs += [((n,), 1, False, dict(tile=True)), ((n,), 2, False, dict(tile=True))]
     for kw in (dict(narrow=True), dict(max_range=25.0), dict(eps=0.05)):       # eps = the smallest positive cell of these
         runs += [(('w21_1500',), 1, True, kw), (('w20_4094',), 0, False, kw), (SETS['set20'], 3, True, kw)]
     runs.append((('w17_16383',), 1, True, dict(image=True)))     # a width-17 map built by the device EDT
@@ -183,8 +172,8 @@ def test_every_variant_against_the_oracle():
         seen.setdefault(_key(variant, count), label)
     missing = ALL_VARIANTS - set(seen)
     print('\n%-18s %3s %5s %4s  first run' % ('kernel', 'FB', 'COUNT', 'MODE'))
-    for k in sorted(seen, key=lambda k: (k[0], k[1], str(k[2]), str(k[3]))):
-        print('%-18s %3d %5s %4s  %s' % (k[0], k[1], '-' if k[2] is None else int(k[2]), '-' if k[3] is None else k[3], seen[k]))
+    for k in sorted(seen):
+        print('%-18s %3d %5d %4d  %s' % (*k, seen[k]))
     print('%d of %d variants ran' % (len(set(seen) & ALL_VARIANTS), len(ALL_VARIANTS)))
     for label, msgs in failures:
         print('FAILED', label, msgs)
