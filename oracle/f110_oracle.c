@@ -656,6 +656,17 @@ typedef struct {
     int32_t* toggles; double* lap_times; double* lap_counts; double* time;
 } StepArgs;
 
+/* RaceCar.reset base_classes.py:183-204 for every car (Simulator.reset :627-643) */
+static void cars_reset(F110Oracle* o, Env* v, const double* poses /*[A][3]*/) {
+    for (int a = 0; a < o->A; ++a) {
+        Car* c = &v->cars[a];
+        memset(c->state, 0, sizeof(c->state));
+        c->state[0] = poses[3 * a]; c->state[1] = poses[3 * a + 1]; c->state[4] = poses[3 * a + 2];
+        c->steer_cnt = 0; c->steer_buf[0] = c->steer_buf[1] = 0.;
+        c->in_collision = 0;
+    }
+}
+
 /* RaceCar.reset base_classes.py:183-204 + F110Env.reset bookkeeping f110_env.py:438-455 */
 static void env_reset(F110Oracle* o, Env* v, const double* poses /*[A][3]*/) {
     int A = o->A;
@@ -667,12 +678,8 @@ static void env_reset(F110Oracle* o, Env* v, const double* poses /*[A][3]*/) {
         v->start_xs[a] = poses[3 * a];
         v->start_ys[a] = poses[3 * a + 1];
         v->start_thetas[a] = poses[3 * a + 2];
-        Car* c = &v->cars[a];
-        memset(c->state, 0, sizeof(c->state));
-        c->state[0] = poses[3 * a]; c->state[1] = poses[3 * a + 1]; c->state[4] = poses[3 * a + 2];
-        c->steer_cnt = 0; c->steer_buf[0] = c->steer_buf[1] = 0.;
-        c->in_collision = 0;
     }
+    cars_reset(o, v, poses);
     double th = -v->start_thetas[o->ego_idx];
     v->start_rot[0] = cos(th); v->start_rot[1] = -sin(th);
     v->start_rot[2] = sin(th); v->start_rot[3] = cos(th);
@@ -851,10 +858,11 @@ int f110o_step(F110Oracle* o, const void* actions, int actions_f64, const double
     return 0;
 }
 
-/* Simulator.reset only (base_classes.py:627-643): no zero-action step; -1 = the ValueError case */
+/* Simulator.reset only (base_classes.py:627-643): the cars move, no zero-action step, and F110Env's bookkeeping (start
+ * poses, toggles, time) stays as it was; -1 = the ValueError case */
 int f110o_sim_reset(F110Oracle* o, const double* poses /*[N][A][3]*/, int num_poses_per_env) {
     if (num_poses_per_env != o->A) return -1;
-    for (int e = 0; e < o->N; ++e) env_reset(o, &o->envs[e], poses + (size_t)e * o->A * 3);
+    for (int e = 0; e < o->N; ++e) cars_reset(o, &o->envs[e], poses + (size_t)e * o->A * 3);
     return 0;
 }
 
