@@ -2,6 +2,7 @@
 // every thread performs `chain` DEPENDENT 8-byte loads at pseudo-random cells of the handle's distance-transform
 // map (the next address depends on the value just loaded), with the lidar kernel's launch shape and no other work.
 // It answers "how fast can this chip chase `chain` fp64 cells per thread through a map of this size".
+// Also f110_trig_probe: the dynamics kernel's sin / cos / tan, for the tests that hold that kernel to a model bit for bit.
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -21,7 +22,28 @@ __global__ void __launch_bounds__(128) gather_probe_kernel(const double* __restr
     }
     if (acc == -1.0) sink[0] = acc;   // never true: keeps the chain alive
 }
+
+// The trig calls of the dynamics kernel, compiled with the library's flags: sincos as for the heading terms, tan and cos as
+// for the steering angle of the kinematic branch.
+__global__ void __launch_bounds__(128) trig_probe_kernel(const double* __restrict__ x, int64_t n, double* __restrict__ out) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const double v = x[i];
+    double s, c;
+    sincos(v, &s, &c);
+    out[i] = s;
+    out[n + i] = c;
+    out[2 * n + i] = tan(v);
+    out[3 * n + i] = cos(v);
+}
 }  // namespace
+
+extern "C" int f110_trig_probe(const double* x_dev, int64_t n, double* out_dev, void* stream) {
+    if (!x_dev || !out_dev || n < 0) return F110_ERR_INVALID;
+    if (n == 0) return F110_OK;
+    trig_probe_kernel<<<(unsigned)((n + 127) / 128), 128, 0, (cudaStream_t)stream>>>(x_dev, n, out_dev);
+    return cudaGetLastError() == cudaSuccess ? F110_OK : F110_ERR_CUDA;
+}
 
 extern "C" int f110_gather_probe(const double* map_dev, int64_t num_cells, int64_t window_cells, int32_t chain,
                                  int64_t num_threads, int32_t repeats, double* sink_dev, float* ms_out, void* stream) {

@@ -301,6 +301,13 @@ int f110_reward_compute(F110Reward* r, const float* obs, const uint8_t* reset_ma
 int f110_gather_probe(const double* map_dev, int64_t num_cells, int64_t window_cells, int32_t chain,
                       int64_t num_threads, int32_t repeats, double* sink_dev, float* ms_out, void* stream);
 
+/* ---- development aid: the dynamics kernel's trig, compiled with the library's flags ----
+ * For each DEVICE x_dev[i], i < n, writes into the DEVICE array out_dev [4][n]: out[0][i], out[1][i] = sin, cos from one
+ * sincos(x) call (the heading terms), out[2][i] = tan(x), out[3][i] = cos(x) (the steering angle of the kinematic
+ * branch).  A model of the dynamics kernel that takes its trig from here reproduces the kernel bit for bit.  Enqueues on
+ * `stream`, does not synchronise. */
+int f110_trig_probe(const double* x_dev, int64_t n, double* out_dev, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

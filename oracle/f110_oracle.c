@@ -626,6 +626,28 @@ static void update_pose(F110Oracle* o, Car* car, double raw_steer, double vel) {
     x[6] = np_clip(x[6], -SLIP_CAP, SLIP_CAP);
 }
 
+/* RaceCar.update_pose for n cars sharing one parameter set, one step each (test entry point): state [n][7],
+ * steer_buf [n][2] (newest first) and steer_cnt [n] are updated in place; raw_steer / speed [n] are the action. */
+void f110o_update_pose(const double* params, double timestep, int integrator, int n, double* state, double* steer_buf,
+                       int* steer_cnt, const double* raw_steer, const double* speed) {
+    F110Oracle o;
+    memset(&o, 0, sizeof(o));
+    o.timestep = timestep;
+    o.integrator = integrator;
+    for (int i = 0; i < n; ++i) {
+        Car car;
+        memset(&car, 0, sizeof(car));
+        memcpy(car.params, params, sizeof(double) * NPARAM);
+        memcpy(car.state, state + 7 * i, sizeof(double) * 7);
+        car.steer_buf[0] = steer_buf[2 * i]; car.steer_buf[1] = steer_buf[2 * i + 1];
+        car.steer_cnt = steer_cnt[i];
+        update_pose(&o, &car, raw_steer[i], speed[i]);
+        memcpy(state + 7 * i, car.state, sizeof(double) * 7);
+        steer_buf[2 * i] = car.steer_buf[0]; steer_buf[2 * i + 1] = car.steer_buf[1];
+        steer_cnt[i] = car.steer_cnt;
+    }
+}
+
 /* baseline-only Gaussian generator (xoshiro256++ + Marsaglia polar). NOT numpy's stream: parity
  * runs inject the numpy noise through the `noise` argument instead. */
 static inline uint64_t rotl(uint64_t x, int k) { return (x << k) | (x >> (64 - k)); }

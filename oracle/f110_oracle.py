@@ -61,6 +61,8 @@ def lib():
         L.f110o_vehicle_dynamics_st.argtypes = [vp] * 4
         L.f110o_vehicle_dynamics_ks.argtypes = [vp] * 4
         L.f110o_pid.argtypes = [C.c_double] * 8 + [dp, dp]
+        L.f110o_update_pose.argtypes = [vp, C.c_double, C.c_int, C.c_int, vp, vp, vp, vp, vp]
+        L.f110o_update_pose.restype = None
         L.f110o_get_vertices.argtypes = [vp, C.c_double, C.c_double, vp]
         L.f110o_collision.argtypes = [vp, vp]
         L.f110o_collision.restype = C.c_int
@@ -260,6 +262,21 @@ class Oracle(object):
         a, s = C.c_double(), C.c_double()
         self.L.f110o_pid(speed, steer, current_speed, current_steer, max_sv, max_a, max_v, min_v, C.byref(a), C.byref(s))
         return a.value, s.value
+
+    @staticmethod
+    def update_pose(state, steer_buf, steer_cnt, raw_steer, speed, params, timestep=0.01, integrator=1):
+        """RaceCar.update_pose (base_classes.py:256-417) of n cars with one parameter set, one step each: state [n, 7],
+        steer_buf [n, 2] (newest first), steer_cnt [n], raw_steer / speed [n] (float32 actions are widened as the env
+        does) -> new (state, steer_buf, steer_cnt)."""
+        x = np.array(state, np.float64).reshape(-1, 7)
+        n = x.shape[0]
+        b = np.array(steer_buf, np.float64).reshape(n, 2)
+        c = np.array(steer_cnt, np.int32).reshape(n)
+        rs = np.ascontiguousarray(np.asarray(raw_steer).astype(np.float64).reshape(n))
+        sp = np.ascontiguousarray(np.asarray(speed).astype(np.float64).reshape(n))
+        lib().f110o_update_pose(_p(params_vector(params)), float(timestep), int(integrator), n, _p(x), _p(b), _p(c),
+                                _p(rs), _p(sp))
+        return x, b, c
 
     def get_vertices(self, pose, length, width):
         v = np.empty((4, 2)); pose = np.ascontiguousarray(pose, np.float64)
