@@ -27,7 +27,7 @@ EXPORTS = ["f110_last_error", "f110_abi_version", "f110_create", "f110_destroy",
            "f110_map_count", "f110_get_map_slot", "f110_set_env_maps", "f110_set_env_maps_host", "f110_get_env_maps", "f110_set_tables",
            "f110_set_beam_tables", "f110_set_params", "f110_sim_reset", "f110_sim_reset_host", "f110_step", "f110_step_host", "f110_step_host_async", "f110_host_sync", "f110_step_host_multi",
            "f110_state_nbytes", "f110_get_state", "f110_set_state", "f110_get_stats", "f110_get_lookup_count",
-           "f110_kernel_launches", "f110_max_lookups", "f110_redone_rays", "f110_get_lidar_variant", "f110_map_generation", "f110_debug_unit_timeline", "f110_set_kernel_timing", "f110_get_kernel_timing", "f110_gap_follow", "f110_gather_probe", "f110_trig_probe", "f110_edt_kernel_ms", "f110_reward_create", "f110_reward_destroy",
+           "f110_kernel_launches", "f110_max_lookups", "f110_redone_rays", "f110_get_lidar_variant", "f110_map_generation", "f110_debug_unit_timeline", "f110_set_kernel_timing", "f110_get_kernel_timing", "f110_gap_follow", "f110_gather_probe", "f110_trig_probe", "f110_hypot_probe", "f110_edt_kernel_ms", "f110_reward_create", "f110_reward_destroy",
            "f110_reward_compute"]
 
 
@@ -115,6 +115,7 @@ def load():
     L.f110_edt_kernel_ms.restype = C.c_float
     L.f110_gather_probe.argtypes = [vp, C.c_int64, C.c_int64, C.c_int32, C.c_int64, C.c_int32, vp, C.POINTER(C.c_float), vp]
     L.f110_trig_probe.argtypes = [vp, C.c_int64, vp, vp]
+    L.f110_hypot_probe.argtypes = [vp, vp, C.c_int64, vp, vp]
     L.f110_reward_create.argtypes = [C.POINTER(F110RewardConfig), vp, vp, vp, C.POINTER(vp)]
     L.f110_reward_destroy.argtypes = [vp]
     L.f110_reward_destroy.restype = None

@@ -73,8 +73,9 @@ __device__ __forceinline__ float lds_f32(unsigned addr) {
     return v;
 }
 
-// preprocess_lidar :3-12 for beam i: mean of the clipped ranges over [i - w/2, i + w/2] cut at the ends.  numpy sums fewer
-// than 8 float32 elements sequentially.  `clipped` is the array's 32-bit shared-memory address (formed once: indexed as a
+// preprocess_lidar :3-12 for beam i: mean of the clipped ranges over [i - w/2, i + w/2] cut at the ends, summed in numpy's
+// order: fewer than 8 float32 elements in sequence, 8 to 15 as ((r0+r1)+(r2+r3))+((r4+r5)+(r6+r7)) over the first eight and
+// the rest in sequence (np.add.reduce's pairwise sum; a window holds at most 15 beams).  `clipped` is the array's 32-bit shared-memory address (formed once: indexed as a
 // C array, every access re-derived the shared window's base); W > 0 = the window size as a compile-time constant, whose
 // interior beams divide by a constant.
 template <int W>
@@ -88,8 +89,23 @@ __device__ __forceinline__ float window_mean(unsigned clipped, int i, int n, int
     }
     const int s = max(0, i - half), e = min(n - 1, i + half);
     float acc = 0.f;
-    for (int k = s; k <= e; ++k) acc += lds_f32(clipped + 4u * (unsigned)k);
+    int k = s;
+    if (W == 0 && e - s + 1 >= 8) {                             // W = 5 windows never reach 8 beams
+        float r[8];
+#pragma unroll
+        for (int j = 0; j < 8; ++j) r[j] = lds_f32(clipped + 4u * (unsigned)(s + j));
+        acc = ((r[0] + r[1]) + (r[2] + r[3])) + ((r[4] + r[5]) + (r[6] + r[7]));
+        k = s + 8;
+    }
+    for (; k <= e; ++k) acc += lds_f32(clipped + 4u * (unsigned)k);
     return __fdiv_rn(acc, (float)(e - s + 1));
+}
+
+// np.argmin's order: (v, i) comes before (bv, bi) if v is the first NaN, or neither is NaN and v is smaller, or ties earlier
+__device__ __forceinline__ bool argmin_before(float v, int i, float bv, int bi) {
+    const bool vn = v != v, bn = bv != bv;
+    if (vn != bn) return vn;
+    return (vn || v == bv) ? i < bi : v < bv;
 }
 
 // One WARP per scan, beam i = 32 k + lane in round k: every access coalesced, no barrier (round 1: a CTA per scan with five
@@ -128,20 +144,20 @@ __global__ void __launch_bounds__(GF_WARPS * 32) gap_follow_kernel(const float* 
         }
     }
     __syncwarp();
-    // create_bubble :14-19: np.argmin = first minimum over the whole scan
+    // create_bubble :14-19: np.argmin = the first NaN if any, else the first minimum over the whole scan
     const unsigned clipped_addr = (unsigned)__cvta_generic_to_shared(clipped);
     float best_v = INFINITY;
     int best_i = 0x7fffffff;
     for (int i = lane; i < n; i += 32) {
         const float m = window_mean<W>(clipped_addr, i, n, window_size);
         proc[i] = m;
-        if (m < best_v) { best_v = m; best_i = i; }              // i increases: the first minimum of this lane
+        if (argmin_before(m, i, best_v, best_i)) { best_v = m; best_i = i; }    // the lane's first NaN / minimum
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
         const float v2 = __shfl_down_sync(0xffffffffu, best_v, o);
         const int i2 = __shfl_down_sync(0xffffffffu, best_i, o);
-        if (v2 < best_v || (v2 == best_v && i2 < best_i)) { best_v = v2; best_i = i2; }
+        if (argmin_before(v2, i2, best_v, best_i)) { best_v = v2; best_i = i2; }
     }
     int closest = __shfl_sync(0xffffffffu, best_i, 0);
     closest = closest == 0x7fffffff ? 0 : closest;
@@ -199,9 +215,12 @@ __global__ void __launch_bounds__(GF_WARPS * 32) gap_follow_kernel(const float* 
 extern "C" int f110_gap_follow(const float* scans, int64_t num_scans, int64_t scan_stride, int32_t num_beams,
                                float* actions, int64_t action_stride, double angle_min, double angle_increment,
                                float max_distance, int32_t window_size, int32_t bubble_radius, float threshold, void* stream) {
-    if (!scans || !actions || num_scans < 0 || num_beams < 1 || num_beams > 8192 || window_size < 1 || window_size > 15)
-        return f110_set_error(F110_ERR_INVALID, "f110_gap_follow: need non-null buffers, 1 <= num_beams <= 8192, 1 <= window_size <= 15");
+    if (!scans || !actions || num_scans < 0 || num_beams < 1 || num_beams > 8192 || window_size < 1 || window_size > 15 ||
+        bubble_radius < 0)
+        return f110_set_error(F110_ERR_INVALID, "f110_gap_follow: need non-null buffers, 1 <= num_beams <= 8192, 1 <= window_size <= 15, "
+                                                "bubble_radius >= 0");
     if (num_scans == 0) return F110_OK;
+    if (bubble_radius > num_beams) bubble_radius = num_beams;      // the same bubble (the whole scan), and closest + radius cannot overflow
     const size_t per_warp = sizeof(float) * (2 * (size_t)num_beams + (size_t)(num_beams + 31) / 32);
     int warps = (int)((48 * 1024) / per_warp);          // stay within the 48 KB that need no opt-in where a scan allows it
     warps = warps > GF_WARPS ? GF_WARPS : (warps < 1 ? 1 : warps);
@@ -270,8 +289,10 @@ constexpr int MID_BLOCK = 64;   // midpoints per pruning block
 struct Cand { double d2; int idx; };
 __device__ __forceinline__ bool cand_less(const Cand& a, const Cand& b) { return a.d2 < b.d2 || (a.d2 == b.d2 && a.idx < b.idx); }
 
-// sorted insertion into a register-resident top-5, ordered by (distance, index)
+// sorted insertion into a register-resident top-5, ordered by (distance, index).  A midpoint at an infinite (or NaN)
+// distance is no neighbour, as in cKDTree.query and the oracle: a car that far off falls back to the nearest node.
 __device__ __forceinline__ void topk_insert(Cand (&best)[KNN], double d2, int idx) {
+    if (!(d2 < INFINITY)) return;
     Cand c;
     c.d2 = d2; c.idx = idx;
     if (!cand_less(c, best[KNN - 1])) return;
@@ -874,7 +895,7 @@ extern "C" int f110_reward_create(const F110RewardConfig* cfg, const double* xy,
     if (!cfg || !xy || !out || cfg->num_envs < 1 || cfg->num_points < 2 || cfg->num_beams < 1 || cfg->num_beams > 8192)
         return f110_set_error(F110_ERR_INVALID, "f110_reward_create: need num_envs >= 1, num_points >= 2, 1 <= num_beams <= 8192");
     if ((cfg->num_points - 1 + MID_BLOCK - 1) / MID_BLOCK > 256)
-        return f110_set_error(F110_ERR_INVALID, "f110_reward_create: at most 16384 centerline points");
+        return f110_set_error(F110_ERR_INVALID, "f110_reward_create: at most 16385 centerline points");
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
         cudaGetLastError();

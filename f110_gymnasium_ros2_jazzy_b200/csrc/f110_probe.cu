@@ -2,11 +2,14 @@
 // every thread performs `chain` DEPENDENT 8-byte loads at pseudo-random cells of the handle's distance-transform
 // map (the next address depends on the value just loaded), with the lidar kernel's launch shape and no other work.
 // It answers "how fast can this chip chase `chain` fp64 cells per thread through a map of this size".
-// Also f110_trig_probe: the dynamics kernel's sin / cos / tan, for the tests that hold that kernel to a model bit for bit.
+// Also f110_trig_probe: the dynamics kernel's sin / cos / tan, and f110_hypot_probe: the shaped reward's hypot, for the tests
+// that hold those kernels to a model bit for bit.
 #include <cuda_runtime.h>
 #include <stdint.h>
 
 #include "f110_b200.h"
+
+int f110_set_error(int code, const char* msg);   // f110_capi.cu
 
 namespace {
 __global__ void __launch_bounds__(128) gather_probe_kernel(const double* __restrict__ map, unsigned mask, unsigned offset,
@@ -36,13 +39,28 @@ __global__ void __launch_bounds__(128) trig_probe_kernel(const double* __restric
     out[2 * n + i] = tan(v);
     out[3 * n + i] = cos(v);
 }
+
+// The reward kernels' one inexact call besides sincos: hypot(ex - ox, ey - oy) of the opponent bubble.
+__global__ void __launch_bounds__(128) hypot_probe_kernel(const double* __restrict__ a, const double* __restrict__ b, int64_t n,
+                                                          double* __restrict__ out) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    out[i] = hypot(a[i], b[i]);
+}
 }  // namespace
 
+extern "C" int f110_hypot_probe(const double* a_dev, const double* b_dev, int64_t n, double* out_dev, void* stream) {
+    if (!a_dev || !b_dev || !out_dev || n < 0) return f110_set_error(F110_ERR_INVALID, "f110_hypot_probe: need non-null buffers and n >= 0");
+    if (n == 0) return F110_OK;
+    hypot_probe_kernel<<<(unsigned)((n + 127) / 128), 128, 0, (cudaStream_t)stream>>>(a_dev, b_dev, n, out_dev);
+    return cudaGetLastError() == cudaSuccess ? F110_OK : f110_set_error(F110_ERR_CUDA, "f110_hypot_probe: kernel launch failed");
+}
+
 extern "C" int f110_trig_probe(const double* x_dev, int64_t n, double* out_dev, void* stream) {
-    if (!x_dev || !out_dev || n < 0) return F110_ERR_INVALID;
+    if (!x_dev || !out_dev || n < 0) return f110_set_error(F110_ERR_INVALID, "f110_trig_probe: need non-null buffers and n >= 0");
     if (n == 0) return F110_OK;
     trig_probe_kernel<<<(unsigned)((n + 127) / 128), 128, 0, (cudaStream_t)stream>>>(x_dev, n, out_dev);
-    return cudaGetLastError() == cudaSuccess ? F110_OK : F110_ERR_CUDA;
+    return cudaGetLastError() == cudaSuccess ? F110_OK : f110_set_error(F110_ERR_CUDA, "f110_trig_probe: kernel launch failed");
 }
 
 extern "C" int f110_gather_probe(const double* map_dev, int64_t num_cells, int64_t window_cells, int32_t chain,

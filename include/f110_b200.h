@@ -287,7 +287,7 @@ typedef struct F110RewardConfig {
            near_wall_dist, w_wall, wall_quantile, opp_safe_dist, w_opp, ego_crash_penalty, opp_crash_bonus;
 } F110RewardConfig;
 typedef struct F110Reward F110Reward;
-/* xy: HOST [num_points][2] centerline; wR / wL: HOST [num_points] half-widths or NULL (CSV columns w_tr_right_m / _left_m). */
+/* xy: HOST [num_points][2] centerline, 2 <= num_points <= 16385; wR / wL: HOST [num_points] half-widths or NULL (CSV columns w_tr_right_m / _left_m). */
 int f110_reward_create(const F110RewardConfig* cfg, const double* xy, const double* wR, const double* wL, F110Reward** out);
 void f110_reward_destroy(F110Reward* r);
 /* obs: DEVICE float [num_envs][num_beams + 8] (F110StepIO.obs); reset_mask: DEVICE [num_envs] or NULL, non-zero =
@@ -307,6 +307,10 @@ int f110_gather_probe(const double* map_dev, int64_t num_cells, int64_t window_c
  * branch).  A model of the dynamics kernel that takes its trig from here reproduces the kernel bit for bit.  Enqueues on
  * `stream`, does not synchronise. */
 int f110_trig_probe(const double* x_dev, int64_t n, double* out_dev, void* stream);
+/* The shaped reward's hypot, compiled with the library's flags: out_dev[i] = hypot(a_dev[i], b_dev[i]) for i < n, all
+ * DEVICE arrays.  With f110_trig_probe's sincos it is all a model of the reward kernels needs beyond IEEE arithmetic to
+ * reproduce them bit for bit.  Enqueues on `stream`, does not synchronise. */
+int f110_hypot_probe(const double* a_dev, const double* b_dev, int64_t n, double* out_dev, void* stream);
 
 #ifdef __cplusplus
 }

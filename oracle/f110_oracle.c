@@ -893,28 +893,50 @@ long f110o_last_lookups(F110Oracle* o) { return o->lookups; }
 /* ------------------------------------------------------------------ rl_training/utils/gap_follow.py
  * (SURVEY 8f row 1: the rule-based opponent of train_ddpg.py:168).  Paths relative to /root/reference/.
  * preprocess_lidar :3-12, create_bubble :14-19, find_max_gap :21-38, find_best_point :40-41,
- * gap_follow_action :43-58.  scan is float32 (info["scans"][1]); numpy's mean of a float32 slice
- * shorter than 8 accumulates sequentially in float32 and divides by the count in float32. */
+ * gap_follow_action :43-58.  scan is float32 (info["scans"][1]); numpy's mean of a float32 slice sums it in
+ * float32 in numpy's pairwise order (np_sum_f32) and divides by the count in float32. */
+
+/* np.add.reduce of a contiguous float32 slice of n <= 128 elements: fewer than 8 in sequence from 0; otherwise eight
+ * partial sums over stride-8 columns, joined as ((r0+r1)+(r2+r3))+((r4+r5)+(r6+r7)), then the remainder in sequence */
+static float np_sum_f32(const float* a, int n) {
+    if (n < 8) {
+        float res = 0.f;
+        for (int i = 0; i < n; ++i) res += a[i];
+        return res;
+    }
+    float r[8];
+    for (int j = 0; j < 8; ++j) r[j] = a[j];
+    int i = 8;
+    for (; i < n - (n % 8); i += 8)
+        for (int j = 0; j < 8; ++j) r[j] += a[i + j];
+    float res = ((r[0] + r[1]) + (r[2] + r[3])) + ((r[4] + r[5]) + (r[6] + r[7]));
+    for (; i < n; ++i) res += a[i];
+    return res;
+}
+
 void f110o_gap_follow(const float* scan, int n, double angle_min, double angle_increment,
                       float max_distance, int window_size, int bubble_radius, float threshold,
                       double* steer_out, double* speed_out, int* best_out, float* proc_out /* [n] or NULL */) {
+    float* clipped = (float*)malloc(sizeof(float) * n);
     float* proc = (float*)malloc(sizeof(float) * n);
+    for (int i = 0; i < n; ++i) {                 /* np.clip: NaN stays NaN */
+        float v = scan[i];
+        if (v < 0.f) v = 0.f;
+        if (v > max_distance) v = max_distance;
+        clipped[i] = v;
+    }
     int half = window_size / 2;
     for (int i = 0; i < n; ++i) {
         int s = i - half < 0 ? 0 : i - half;
         int e = i + half > n - 1 ? n - 1 : i + half;
-        float acc = 0.f;
-        for (int k = s; k <= e; ++k) {
-            float v = scan[k];
-            if (v < 0.f) v = 0.f;
-            if (v > max_distance) v = max_distance;
-            acc += v;
-        }
-        proc[i] = acc / (float)(e - s + 1);
+        proc[i] = np_sum_f32(clipped + s, e - s + 1) / (float)(e - s + 1);
     }
     if (proc_out) memcpy(proc_out, proc, sizeof(float) * n);
+    /* np.argmin: the first NaN if there is one, otherwise the first minimum */
     int closest = 0;
-    for (int i = 1; i < n; ++i) if (proc[i] < proc[closest]) closest = i;
+    for (int i = 1; i < n && proc[closest] == proc[closest]; ++i)
+        if (proc[i] != proc[i] || proc[i] < proc[closest]) closest = i;
+    if (bubble_radius > n) bubble_radius = n;     /* python slices cannot overflow: the same bubble */
     {
         int s = closest - bubble_radius < 0 ? 0 : closest - bubble_radius;
         int e = closest + bubble_radius > n - 1 ? n - 1 : closest + bubble_radius;
@@ -938,7 +960,7 @@ void f110o_gap_follow(const float* scan, int n, double angle_min, double angle_i
     else if (fabs(steering) < d20) speed = 2;
     else speed = 1.5;
     *steer_out = steering; *speed_out = speed; *best_out = best;
-    free(proc);
+    free(proc); free(clipped);
 }
 
 /* ------------------------------------------------------------------ shaped reward (SURVEY 8f row 2)
@@ -1006,7 +1028,8 @@ void f110o_reward_destroy(F110RewardOracle* o) {
 
 /* project_xy, track_progress.py:58-95: the 5 nearest segment midpoints (cKDTree.query, ascending distance), best
  * orthogonal projection among them (first strictly smaller distance wins) */
-static void project_xy(const F110RewardOracle* o, double x, double y, double* s_out, double* t_out) {
+static void project_xy(const F110RewardOracle* o, double x, double y, double* s_out, double* t_out,
+                       double* knn_out /*[5] or NULL*/, double* fallback_out /* or NULL */) {
     int K = o->n - 1 < 5 ? o->n - 1 : 5;
     int idx[5]; double dd[5];
     for (int k = 0; k < K; ++k) { idx[k] = -1; dd[k] = INFINITY; }
@@ -1019,6 +1042,7 @@ static void project_xy(const F110RewardOracle* o, double x, double y, double* s_
             dd[k] = d2; idx[k] = i;
         }
     }
+    if (knn_out) for (int k = 0; k < 5; ++k) knn_out[k] = k < K ? (double)idx[k] : -1.0;
     int have = 0; double best_d = 0, best_s = 0, best_t = 0;
     for (int k = 0; k < K; ++k) {
         int i = idx[k];
@@ -1043,8 +1067,11 @@ static void project_xy(const F110RewardOracle* o, double x, double y, double* s_
             double d = sqrt(dx * dx + dy * dy);
             if (d < bd) { bd = d; j = i; }
         }
-        *s_out = o->s[j]; *t_out = 0.0; return;
+        *s_out = o->s[j]; *t_out = 0.0;
+        if (fallback_out) *fallback_out = 1.0;
+        return;
     }
+    if (fallback_out) *fallback_out = 0.0;
     *s_out = best_s; *t_out = best_t;
 }
 
@@ -1091,19 +1118,32 @@ static float quantile_f32(float* v, int n, double q) {
 
 static double wrap_pi(double a) { return py_mod(a + PI, 2 * PI) - PI; }
 
-static double reward_one(const F110RewardOracle* o, RewardState* r, const float* obs) {
+/* Per-env breakdown of one reward call, F110O_REWARD_TERMS doubles (f110_oracle.py REWARD_TERM_NAMES):
+ *  0-4 the ego's 5 nearest midpoints (distance, then index; -1 where the centerline has fewer), 5-9 the opponent's,
+ *  10, 11 1 where the ego's / opponent's projection fell back to the nearest node, 12-15 e_s, e_t, o_s, o_t,
+ *  16 the lateral segment index, 17-19 de, dop (after the flip) and flip, 20 the wall quantile dmin (NaN when not taken),
+ *  21-27 r_prog, r_alive, r_lead, r_lat, r_wall, r_opp, r_flank, 28 the early return (0 none, 1 ego crash, 2 opponent
+ *  crash bonus), 29 steps, 30 oth (wrapped to [-pi, pi)), 31 w_eff.  Fields a call does not reach are NaN. */
+#define F110O_REWARD_TERMS 32
+
+static double reward_one(const F110RewardOracle* o, RewardState* r, const float* obs, double* t) {
+    double tt[F110O_REWARD_TERMS];
+    if (!t) t = tt;
+    for (int k = 0; k < F110O_REWARD_TERMS; ++k) t[k] = NAN;
     int B = o->B;
     double ex = (double)obs[B + 0], ey = (double)obs[B + 1];
     int ego_col = obs[B + 3] != 0.0f;
     double ox = (double)obs[B + 4], oy = (double)obs[B + 5], oth = wrap_pi((double)obs[B + 6]);
     int opp_col = obs[B + 7] != 0.0f;
     r->steps += 1;                                                              /* :299 */
-    if (ego_col) return -o->ego_crash_penalty;                                  /* :302-303 */
-    if (opp_col && o->opp_crash_bonus > 0.0) return +o->opp_crash_bonus;        /* :304-305 */
+    t[29] = r->steps; t[30] = oth; t[28] = 0.0;
+    if (ego_col) { t[28] = 1.0; return -o->ego_crash_penalty; }                 /* :302-303 */
+    if (opp_col && o->opp_crash_bonus > 0.0) { t[28] = 2.0; return +o->opp_crash_bonus; }   /* :304-305 */
     /* _Prog.update :129-167 */
     double e_s, e_t, o_s, o_t;
-    project_xy(o, ex, ey, &e_s, &e_t);
-    project_xy(o, ox, oy, &o_s, &o_t);
+    project_xy(o, ex, ey, &e_s, &e_t, t + 0, t + 10);
+    project_xy(o, ox, oy, &o_s, &o_t, t + 5, t + 11);
+    t[12] = e_s; t[13] = e_t; t[14] = o_s; t[15] = o_t;
     if (!r->has_s_prev[0]) { r->has_s_prev[0] = 1; r->s_prev[0] = e_s; }
     if (!r->has_s_prev[1]) { r->has_s_prev[1] = 1; r->s_prev[1] = o_s; }
     double de = signed_step(o, r, 0, ex, ey, e_s, r->s_prev[0]);
@@ -1114,6 +1154,7 @@ static double reward_one(const F110RewardOracle* o, RewardState* r, const float*
         if (r->buf_n == 20 && r->buf_sum / 20 < 0.0) r->flip = -1.0;
     }
     de *= r->flip; dop *= r->flip;
+    t[17] = de; t[18] = dop; t[19] = r->flip;
     r->cum[0] += de; r->cum[1] += dop;
     r->ema_abs = 0.8 * r->ema_abs + (1.0 - 0.8) * fabs(de);
     r->t_last[0] = e_t; r->t_last[1] = o_t;
@@ -1129,10 +1170,12 @@ static double reward_one(const F110RewardOracle* o, RewardState* r, const float*
     }
     /* lateral :323-333 */
     int idx = seg_index_at_s(o, e_s);
+    t[16] = idx;
     double wR = o->default_half_width, wL = o->default_half_width;
     if (o->has_widths) { wR = o->wR[idx]; wL = o->wL[idx]; }
     double w_eff = e_t >= 0.0 ? wL : wR;
     if (w_eff < 0.2) w_eff = 0.2;
+    t[31] = w_eff;
     double lat_norm = fabs(e_t) / w_eff;
     double lat_term = lat_norm * lat_norm < o->lat_cap ? lat_norm * lat_norm : o->lat_cap;
     double r_lat = -o->w_lat * lat_term;
@@ -1148,6 +1191,7 @@ static double reward_one(const F110RewardOracle* o, RewardState* r, const float*
             tmp[i] = v;
         }
         double dmin = (double)quantile_f32(tmp, B, o->wall_q);
+        t[20] = dmin;
         if (dmin < o->near_wall_dist) {
             double x = (o->near_wall_dist - dmin) / (o->near_wall_dist > 1e-6 ? o->near_wall_dist : 1e-6);
             r_wall = -o->w_wall * (x * x);
@@ -1174,12 +1218,34 @@ static double reward_one(const F110RewardOracle* o, RewardState* r, const float*
             r_flank = 0.1 * (x_rel / 1.8) * (yb / 0.8);
         }
     }
+    t[21] = r_prog; t[22] = r_alive; t[23] = r_lead; t[24] = r_lat; t[25] = r_wall; t[26] = r_opp; t[27] = r_flank;
     return r_prog + r_alive + r_lead + r_lat + r_wall + r_opp + r_flank;
 }
 
-void f110o_reward_compute(F110RewardOracle* o, const float* obs /*[N][B+8]*/, const uint8_t* reset_mask, double* out) {
+void f110o_reward_compute_terms(F110RewardOracle* o, const float* obs /*[N][B+8]*/, const uint8_t* reset_mask, double* out,
+                                double* terms /*[N][F110O_REWARD_TERMS] or NULL*/) {
     for (int e = 0; e < o->N; ++e) {
         if (reset_mask && reset_mask[e]) reward_state_reset(&o->st[e]);
-        out[e] = reward_one(o, &o->st[e], obs + (size_t)e * (o->B + 8));
+        out[e] = reward_one(o, &o->st[e], obs + (size_t)e * (o->B + 8), terms ? terms + (size_t)e * F110O_REWARD_TERMS : NULL);
     }
+}
+
+void f110o_reward_compute(F110RewardOracle* o, const float* obs /*[N][B+8]*/, const uint8_t* reset_mask, double* out) {
+    f110o_reward_compute_terms(o, obs, reset_mask, out, NULL);
+}
+
+/* the oracle's own float32 quantile and lateral segment lookup, for the tests that pin them to numpy */
+float f110o_quantile_f32(const float* v, int n, double q) {
+    float* tmp = (float*)malloc(sizeof(float) * (n > 0 ? n : 1));
+    memcpy(tmp, v, sizeof(float) * n);
+    float r = quantile_f32(tmp, n, q);
+    free(tmp);
+    return r;
+}
+
+int f110o_reward_seg_index(const F110RewardOracle* o, double s) { return seg_index_at_s(o, s); }
+
+void f110o_reward_knn(const F110RewardOracle* o, double x, double y, double* knn /*[5]*/, double* st /*[2]*/) {
+    double fb;
+    project_xy(o, x, y, st, st + 1, knn, &fb);
 }

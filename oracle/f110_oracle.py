@@ -71,6 +71,12 @@ def lib():
         L.f110o_reward_create.argtypes = [C.c_int, C.c_int, vp, vp, vp, C.c_int, C.c_int, vp, C.c_int, C.c_int]
         L.f110o_reward_destroy.argtypes = [vp]
         L.f110o_reward_compute.argtypes = [vp, vp, vp, vp]
+        L.f110o_reward_compute_terms.argtypes = [vp, vp, vp, vp, vp]
+        L.f110o_quantile_f32.argtypes = [vp, C.c_int, C.c_double]
+        L.f110o_quantile_f32.restype = C.c_float
+        L.f110o_reward_seg_index.argtypes = [vp, C.c_double]
+        L.f110o_reward_seg_index.restype = C.c_int
+        L.f110o_reward_knn.argtypes = [vp, C.c_double, C.c_double, vp, vp]
         L.f110o_gap_follow.argtypes = [vp, C.c_int, C.c_double, C.c_double, C.c_float, C.c_int, C.c_int, C.c_float,
                                        dp, dp, C.POINTER(C.c_int), vp]
         _LIB = L
@@ -295,14 +301,16 @@ class Oracle(object):
         return c, i
 
 
-def gap_follow_action(scan, angle_min=-np.pi / 2, angle_increment=np.pi / 1080, want_proc=False):
-    """rl_training/utils/gap_follow.py:43-58 restated (oracle): float32 scan -> (steer, speed) as float64."""
+def gap_follow_action(scan, angle_min=-np.pi / 2, angle_increment=np.pi / 1080, max_distance=3.0, window_size=5,
+                      bubble_radius=30, threshold=0.5, want_proc=False):
+    """rl_training/utils/gap_follow.py:43-58 restated (oracle): float32 scan -> (steer, speed) as float64.  The keyword
+    arguments are the reference's parameters with its defaults; want_proc also returns the window means."""
     L = lib()
     scan = np.ascontiguousarray(scan, np.float32)
     st, sp, best = C.c_double(), C.c_double(), C.c_int()
     proc = np.empty(scan.shape[0], np.float32) if want_proc else None
-    L.f110o_gap_follow(_p(scan), scan.shape[0], angle_min, angle_increment, 3.0, 5, 30, 0.5, C.byref(st), C.byref(sp),
-                       C.byref(best), _p(proc))
+    L.f110o_gap_follow(_p(scan), scan.shape[0], float(angle_min), float(angle_increment), float(max_distance), int(window_size),
+                       int(bubble_radius), float(threshold), C.byref(st), C.byref(sp), C.byref(best), _p(proc))
     out = np.array([st.value, sp.value])
     return (out, proc) if want_proc else out
 
@@ -317,15 +325,31 @@ REWARD_DEFAULTS = dict(dt=0.01, w_prog=1.2, forward_sign=+1.0, alive_bonus=0.02,
                        grace_steps_wall=25, grace_steps_opp=25)
 
 
+# the columns of RewardOracle.terms (f110o_reward_compute_terms in f110_oracle.c)
+REWARD_TERM_NAMES = (['knn_ego%d' % k for k in range(5)] + ['knn_opp%d' % k for k in range(5)] +
+                     ['fallback_ego', 'fallback_opp', 'e_s', 'e_t', 'o_s', 'o_t', 'seg', 'de', 'dop', 'flip', 'dmin',
+                      'r_prog', 'r_alive', 'r_lead', 'r_lat', 'r_wall', 'r_opp', 'r_flank', 'early', 'steps', 'oth', 'w_eff'])
+REWARD_TERM = {k: i for i, k in enumerate(REWARD_TERM_NAMES)}
+
+
+def quantile_f32(values, q):
+    """The oracle's np.quantile(float32 array, q) (method 'linear')."""
+    v = np.ascontiguousarray(values, np.float32)
+    return np.float32(lib().f110o_quantile_f32(_p(v), len(v), float(q)))
+
+
 class RewardOracle(object):
     """CenterlineSafetyProgressReward (rewards.py:185-355) over a CenterlineProgress (track_progress.py), one
-    independent instance per env.  centerline: [n, 4] rows x_m, y_m, w_tr_right_m, w_tr_left_m."""
+    independent instance per env.  centerline: [n, 4] rows x_m, y_m, w_tr_right_m, w_tr_left_m, or [n, 2] without the
+    widths (the reward then uses default_half_width on both sides)."""
 
     def __init__(self, num_envs, centerline, num_beams=1080, closed=True, **kw):
         self.L = lib()
         p = dict(REWARD_DEFAULTS); p.update(kw)
         cl = np.ascontiguousarray(centerline, np.float64)
-        xy = np.ascontiguousarray(cl[:, :2]); wR = np.ascontiguousarray(cl[:, 2]); wL = np.ascontiguousarray(cl[:, 3])
+        xy = np.ascontiguousarray(cl[:, :2])
+        wR = np.ascontiguousarray(cl[:, 2]) if cl.shape[1] >= 4 else None
+        wL = np.ascontiguousarray(cl[:, 3]) if cl.shape[1] >= 4 else None
         pv = np.array([float(p[k]) for k in REWARD_PARAM_KEYS])
         self.N, self.B = num_envs, num_beams
         self.h = self.L.f110o_reward_create(num_envs, num_beams, _p(xy), _p(wR), _p(wL), len(xy), int(closed), _p(pv),
@@ -336,8 +360,24 @@ class RewardOracle(object):
             self.L.f110o_reward_destroy(self.h); self.h = None
 
     def __call__(self, obs, reset_mask=None):
+        return self.compute_terms(obs, reset_mask)[0]
+
+    def compute_terms(self, obs, reset_mask=None):
+        """One reward call -> (total [N], terms [N, len(REWARD_TERM_NAMES)]): the per-env breakdown of what the call
+        did (neighbours, projections, branch taken, each summand); NaN where the call did not get that far."""
         obs = np.ascontiguousarray(obs, np.float32).reshape(self.N, self.B + 8)
         out = np.empty(self.N)
+        terms = np.empty((self.N, len(REWARD_TERM_NAMES)))
         rm = None if reset_mask is None else np.ascontiguousarray(reset_mask, np.uint8)
-        self.L.f110o_reward_compute(self.h, _p(obs), _p(rm), _p(out))
-        return out
+        self.L.f110o_reward_compute_terms(self.h, _p(obs), _p(rm), _p(out), _p(terms))
+        return out, terms
+
+    def seg_index(self, s):
+        """The lateral term's segment lookup: np.searchsorted(s_knots, s, 'right') - 1 clamped to [0, n - 2]."""
+        return self.L.f110o_reward_seg_index(self.h, float(s))
+
+    def knn(self, x, y):
+        """The 5 nearest segment midpoints of (x, y) in the oracle's order (distance, then index), and (s, t)."""
+        k, st = np.empty(5), np.empty(2)
+        self.L.f110o_reward_knn(self.h, float(x), float(y), _p(k), _p(st))
+        return k.astype(np.int64), st

@@ -845,7 +845,7 @@ def test_gap_follow_kernel_bit_exact():
 
 def test_consumers_survive_non_finite_inputs():
     """The observation of a poisoned car (NaN pose, NaN/inf beams) goes through the gap-follow and reward kernels without
-    a fault, and the rows next to it come out exactly as they do without it."""
+    a fault, the rows next to it come out exactly as they do without it, and the poisoned rows equal the oracle's."""
     torch = _torch()
     from f110_gymnasium_ros2_jazzy_b200 import ShapedReward, gap_follow_actions
     from tests.test_oracle_golden import REWARD_KW
@@ -865,20 +865,29 @@ def test_consumers_survive_non_finite_inputs():
         out.append(act.cpu().numpy())
     keep = np.ones(64, bool); keep[[5, 9, 11]] = False
     assert np.array_equal(out[0][keep], out[1][keep])
+    from oracle.f110_oracle import RewardOracle, gap_follow_action
+    for k in (5, 9, 11):
+        assert np.array_equal(out[1][k, 1], gap_follow_action(bad[k]).astype(np.float32)), k
 
     obs = r['obs'][:8].copy()
     badobs = obs.copy()
     badobs[2, 1080:1083] = np.nan          # pose
     badobs[3, :1080] = np.nan              # lidar
     badobs[4, 1080] = np.inf
+    from tests.test_consumer_kernels import DeviceMath, expected_reward
+    dm = DeviceMath()
     res = []
     for arr in (obs, badobs):
         rw = ShapedReward(8, r['centerline'], **REWARD_KW)
+        orc = RewardOracle(8, r['centerline'], **REWARD_KW)
         mask = torch.ones(8, dtype=torch.uint8, device='cuda')
         for _ in range(3):
             got = rw(torch.from_numpy(arr).cuda(), mask)
+            tot, terms = orc.compute_terms(arr, mask.cpu().numpy())
             mask = torch.zeros(8, dtype=torch.uint8, device='cuda')
-        torch.cuda.synchronize()
+            torch.cuda.synchronize()
+            want, _ = expected_reward(dm, arr, tot, terms, 1080, REWARD_KW)
+            assert np.array_equal(got.cpu().numpy(), want, equal_nan=True)
         res.append(got.cpu().numpy())
         rw.close()
     keep = np.ones(8, bool); keep[[2, 3, 4]] = False
@@ -1079,14 +1088,17 @@ def test_c4_full_size_sharded_properties():
 
 @pytest.mark.parametrize('form', ['warp', 'cta'])
 def test_shaped_reward_kernel_matches_reference_and_oracle(form, monkeypatch):
-    """f110_reward_compute: (a) the recorded reference episodes, each replayed in its own env slot of one batch, (b) the
-    oracle on a seeded batch of independent envs.  Tolerance 1e-9 (fp64, device libm); crash returns are exact.  Both
-    forms of the kernel: a warp per env (the default) and a CTA per env (scans too long for a warp's shared memory; forced)."""
+    """f110_reward_compute: (a) the recorded reference episodes, each replayed in its own env slot of one batch, within
+    1e-9 of the reference (numpy, BLAS and glibc there), (b) the oracle on the same batch of independent envs, exactly,
+    once its opponent and flank terms are recomputed with the device's hypot and sincos.  Both forms of the kernel: a warp
+    per env (the default) and a CTA per env (scans too long for a warp's shared memory; forced)."""
     monkeypatch.setenv('F110_REWARD_CTA', '1' if form == 'cta' else '0')
     torch = _torch()
     from f110_gymnasium_ros2_jazzy_b200 import ShapedReward
     from oracle.f110_oracle import RewardOracle
+    from tests.test_consumer_kernels import DeviceMath, expected_reward
     from tests.test_oracle_golden import REWARD_ALT_KW, REWARD_KW
+    dm = DeviceMath()
     g = H.reward_recording()
     obs, starts = g['obs'], g['episode_start']
     T = len(obs)
@@ -1095,16 +1107,14 @@ def test_shaped_reward_kernel_matches_reference_and_oracle(form, monkeypatch):
         N = 4
         rw = ShapedReward(N, g['centerline'], **kw)
         orc = RewardOracle(N, g['centerline'], **kw)
-        worst = 0.0
         for t in range(T):
             batch = np.stack([obs[(t + 37 * k) % T] for k in range(N)])
             mask = np.array([starts[(t + 37 * k) % T] or t == 0 for k in range(N)], np.uint8)
             got = rw(torch.from_numpy(batch).cuda(), torch.from_numpy(mask).cuda()).cpu().numpy()
-            ref = orc(batch, mask)
-            worst = max(worst, np.abs(got - ref).max())
+            tot, terms = orc.compute_terms(batch, mask)
+            want, _ = expected_reward(dm, batch, tot, terms, 1080, kw)
+            assert np.array_equal(got, want), (key, t, got, want)
             assert abs(got[0] - g[key][t]) < 1e-9, (key, t, got[0], g[key][t])
-        assert worst < 1e-9
-        print('reward', key, 'worst vs oracle', worst)
         rw.close()
 
 
