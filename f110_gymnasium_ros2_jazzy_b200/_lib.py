@@ -28,7 +28,7 @@ EXPORTS = ["f110_last_error", "f110_abi_version", "f110_create", "f110_destroy",
            "f110_set_beam_tables", "f110_set_params", "f110_sim_reset", "f110_sim_reset_host", "f110_step", "f110_step_host", "f110_step_host_async", "f110_host_sync", "f110_step_host_multi",
            "f110_state_nbytes", "f110_get_state", "f110_set_state", "f110_get_stats", "f110_get_lookup_count",
            "f110_kernel_launches", "f110_max_lookups", "f110_redone_rays", "f110_get_lidar_variant", "f110_map_generation", "f110_debug_unit_timeline", "f110_set_kernel_timing", "f110_get_kernel_timing", "f110_gap_follow", "f110_gather_probe", "f110_trig_probe", "f110_hypot_probe", "f110_edt_kernel_ms", "f110_reward_create", "f110_reward_destroy",
-           "f110_reward_compute"]
+           "f110_reward_compute", "f110_reward_create_set", "f110_reward_count", "f110_reward_compute_slots"]
 
 
 class F110Config(C.Structure):
@@ -61,6 +61,10 @@ class F110RewardConfig(C.Structure):
                [(n, C.c_double) for n in ("dt", "w_prog", "forward_sign", "alive_bonus", "w_rel_lead", "lead_clip", "w_lat",
                                           "lat_cap", "default_half_width", "lidar_max", "near_wall_dist", "w_wall",
                                           "wall_quantile", "opp_safe_dist", "w_opp", "ego_crash_penalty", "opp_crash_bonus")]
+
+
+class F110Centerline(C.Structure):
+    _fields_ = [("xy", C.c_void_p), ("wR", C.c_void_p), ("wL", C.c_void_p), ("num_points", C.c_int32), ("closed", C.c_int32)]
 
 
 _lib = None
@@ -120,6 +124,10 @@ def load():
     L.f110_reward_destroy.argtypes = [vp]
     L.f110_reward_destroy.restype = None
     L.f110_reward_compute.argtypes = [vp, vp, vp, vp, vp, vp]
+    L.f110_reward_create_set.argtypes = [C.POINTER(F110RewardConfig), C.POINTER(F110Centerline), C.c_int32, C.POINTER(vp)]
+    L.f110_reward_count.argtypes = [vp]
+    L.f110_reward_count.restype = C.c_int32
+    L.f110_reward_compute_slots.argtypes = [vp, vp, vp, vp, vp, vp, vp]
     L.f110_max_lookups.argtypes = [vp]
     L.f110_max_lookups.restype = C.c_int64
     L.f110_redone_rays.argtypes = [vp]

@@ -146,7 +146,7 @@ class BatchSim(object):
         """Installs a map set (f110_set_maps): env e then drives on map floor(e * K / N) until set_env_maps says otherwise.
         Each spec is a yaml path (loaded like set_map: scipy's EDT on the host, or the device EDT with edt='device'), a
         (dt float64 [H, W], resolution, origin) tuple, or a (free_mask bool / uint8 [H, W], resolution, origin) tuple (device
-        EDT).  The shaped reward keeps one centerline per handle: it does not follow the slots."""
+        EDT).  ShapedReward(centerlines=[...]) with one centerline per map scores each env on the line of its slot."""
         from .maps import load_map_image
         descs, keep, shapes = (_lib.F110MapDesc * len(specs))(), [], []
         for k, spec in enumerate(specs):
@@ -196,9 +196,13 @@ class BatchSim(object):
         _lib.check(self.lib.f110_set_env_maps_host(self.h, sl.ctypes.data_as(C.c_void_p),
                                                    None if m is None else m.ctypes.data_as(C.c_void_p)))
 
-    def env_maps(self):
-        """Device int32 [N]: each env's map slot (all 0 for a single map), valid in stream order."""
-        out = torch.empty(self.N, dtype=torch.int32, device=self.device)
+    def env_maps(self, out=None):
+        """Device int32 [N]: each env's map slot (all 0 for a single map), valid in stream order.  ``out``: a contiguous
+        device int32 [N] tensor to write instead of a new one (one stream-ordered copy, capturable into a CUDA graph)."""
+        if out is None:
+            out = torch.empty(self.N, dtype=torch.int32, device=self.device)
+        elif not (out.is_cuda and out.dtype == torch.int32 and out.is_contiguous() and out.numel() == self.N):
+            raise ValueError("env_maps(out=...) needs a contiguous CUDA int32 tensor of %d entries" % self.N)
         _lib.check(self.lib.f110_get_env_maps(self.h, _ptr(out), self._stream()))
         return out
 

@@ -7,6 +7,7 @@
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdint.h>
+#include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
 
@@ -263,6 +264,9 @@ struct F110Reward {
     int nblk;
     void* state;                                  // device RewardState[N]
     int device;
+    int count;                                    // centerlines: 1, or a set of K (n, L, nblk and cfg.closed then unused)
+    void* lines;                                  // device RewardLine[count] (sets only)
+    int* prev_slot;                               // device [N]: each env's slot at its previous call, -1 at first (sets only)
 };
 
 namespace {
@@ -280,6 +284,22 @@ struct RewardView {
     const double *xy, *s, *tan, *nrm, *mid, *wR, *wL, *blk;
     int nblk;
     RewardState* st;
+};
+
+// A set of K centerlines: the lines lie back to back in one allocation per array, line k's points from `off` on (xy, s,
+// wR, wL; tan, nrm, mid likewise, one entry short), its bounding circles from block `boff` on.  The set kernels read the
+// env's slot, then the slot's record, and point a RewardView at that line; from there on they are the single-line kernels.
+struct RewardLine {
+    int off, n, nblk, boff;
+    double L;
+    int closed, has_widths;
+};
+
+struct RewardSetView {
+    const RewardLine* lines;
+    const int* slots;                             // [N] the caller's
+    int* prev;                                    // [N] F110Reward::prev_slot
+    int count;
 };
 
 constexpr int RW_THREADS = 128;
@@ -402,234 +422,36 @@ __device__ double signed_step(const RewardView& v, RewardState& r, int who, doub
     return copysign(fabs(ds_geom), fabs(ds_sign) > 1e-6 ? ds_sign : ds_geom);
 }
 
+// v (a view of the whole set) <- the view of one of its lines
+__device__ __forceinline__ void select_line(RewardView& v, const RewardLine& ln) {
+    const size_t o = (size_t)ln.off;
+    v.n = ln.n; v.L = ln.L; v.nblk = ln.nblk; v.p.closed = ln.closed;
+    v.xy += 2 * o; v.s += o; v.tan += 2 * o; v.nrm += 2 * o; v.mid += 2 * o;
+    v.wR = ln.has_widths ? v.wR + o : nullptr;
+    v.wL = ln.has_widths ? v.wL + o : nullptr;
+    v.blk += 3 * (size_t)ln.boff;
+}
+
+__device__ __forceinline__ void write_nan(double* out64, float* out32, int env) {
+    if (out64) out64[env] = __longlong_as_double(0x7ff8000000000000LL);
+    if (out32) out32[env] = __int_as_float(0x7fc00000);
+}
+
 __global__ void __launch_bounds__(RW_THREADS) shaped_reward_kernel(RewardView v, const float* __restrict__ obs,
                                                                    const uint8_t* __restrict__ reset_mask,
                                                                    double* __restrict__ out64, float* __restrict__ out32) {
-    const int env = blockIdx.x, tid = threadIdx.x;
-    const int B = v.p.num_beams;
-    const float* ob = obs + (size_t)env * (B + 8);
-    extern __shared__ unsigned s_bits[];            // [B] lidar as order-preserving unsigned
-    __shared__ Cand s_cand[(RW_THREADS / 32) * KNN];
-    __shared__ double s_lb[256];                    // lower bound of every midpoint block (nblk <= 256)
-    __shared__ double s_tau[RW_THREADS / 32];
-    __shared__ int s_cblk[256];
-    __shared__ int s_ncand;
-    __shared__ int s_knn[2][KNN];
-    __shared__ double s_pose[5];                    // ex, ey, ox, oy, oth
-    __shared__ double s_proj[4];                    // e_s, e_t, o_s, o_t
-    __shared__ int s_flag[3];                       // early-out, steps, do-wall
-    __shared__ unsigned s_hist[256];
-    __shared__ unsigned s_sel[4];                   // prefix, remaining rank, count<=, min>
-    __shared__ float s_q[2];
-    __shared__ int s_seg[2];                        // segment each car was projected on (hint for the arclength lookups)
-    RewardState& r = v.st[env];
+#define F110_REWARD_SET 0
+#include "f110_reward_cta_body.cuh"
+#undef F110_REWARD_SET
+}
 
-    if (tid == 0) {
-        if (reset_mask && reset_mask[env]) {        // reward_fn.reset() (rewards.py:262-264, _Prog.reset :98-106)
-            RewardState z;
-            memset(&z, 0, sizeof(z));
-            z.flip = +1.0;
-            r = z;
-        }
-        // parse_flat_obs :11-39 (the float32 fields are widened by float())
-        s_pose[0] = (double)ob[B + 0]; s_pose[1] = (double)ob[B + 1];
-        s_pose[2] = (double)ob[B + 4]; s_pose[3] = (double)ob[B + 5];
-        double th = (double)ob[B + 6] + 3.141592653589793;
-        double m = fmod(th, 2 * 3.141592653589793);
-        if (m != 0.0) { if (m < 0.0) m += 2 * 3.141592653589793; } else m = 0.0;
-        s_pose[4] = m - 3.141592653589793;
-        const bool ego_col = ob[B + 3] != 0.0f, opp_col = ob[B + 7] != 0.0f;
-        r.steps += 1;                                                   // :299
-        s_flag[1] = r.steps;
-        s_flag[0] = 0;
-        if (ego_col) { s_flag[0] = 1; if (out64) out64[env] = -v.p.ego_crash_penalty; if (out32) out32[env] = (float)-v.p.ego_crash_penalty; }
-        else if (opp_col && v.p.opp_crash_bonus > 0.0) { s_flag[0] = 1; if (out64) out64[env] = v.p.opp_crash_bonus; if (out32) out32[env] = (float)v.p.opp_crash_bonus; }
-        s_flag[2] = r.steps >= v.p.grace_steps_wall;
-    }
-    __syncthreads();
-    if (s_flag[0]) return;
-
-    // ---- 5 nearest midpoints of both cars (cKDTree.query(p, k=5)), exactly, without visiting all of them: the
-    // midpoints are grouped in blocks of 64 consecutive ones with a bounding circle (centre, R).  Any block holds >= 5
-    // points within |p - c| + R of p, so tau = min over blocks of that bound is an upper bound on the 5th-nearest
-    // distance, and only blocks with |p - c| - R <= tau can contain one of the 5.  On a race track that is 1-3 blocks.
-    for (int who = 0; who < 2; ++who) {
-        const double px = s_pose[2 * who], py = s_pose[2 * who + 1];
-        double ub = INFINITY;
-        for (int k = tid; k < v.nblk; k += RW_THREADS) {
-            const double dx = v.blk[3 * k] - px, dy = v.blk[3 * k + 1] - py, R = v.blk[3 * k + 2];
-            const double d = sqrt(dx * dx + dy * dy);
-            s_lb[k] = d - R;
-            const int cnt = min(MID_BLOCK, v.n - 1 - k * MID_BLOCK);
-            if (cnt >= KNN) ub = fmin(ub, d + R);
-        }
-        for (int o = 16; o > 0; o >>= 1) ub = fmin(ub, __shfl_xor_sync(0xffffffffu, ub, o));
-        if ((tid & 31) == 0) s_tau[tid >> 5] = ub;
-        __syncthreads();
-        double tau = fmin(fmin(s_tau[0], s_tau[1]), fmin(s_tau[2], s_tau[3]));
-        tau = tau * (1.0 + 1e-12) + 1e-12;                              // slack for the rounding of the bounds
-        Cand best[KNN];
-#pragma unroll
-        for (int k = 0; k < KNN; ++k) { best[k].d2 = INFINITY; best[k].idx = 0x7fffffff; }
-        // compact the blocks that can hold one of the 5 (all of them if no block has 5 points)
-        if (tid == 0) s_ncand = 0;
-        __syncthreads();
-        for (int k = tid; k < v.nblk; k += RW_THREADS)
-            if (!(tau < INFINITY) || s_lb[k] <= tau) s_cblk[atomicAdd(&s_ncand, 1)] = k;
-        __syncthreads();
-        const int ncand = s_ncand;
-        for (int j0 = 0; j0 < ncand; j0 += RW_THREADS / MID_BLOCK) {
-            const int j = j0 + tid / MID_BLOCK;                         // two blocks per pass
-            if (j < ncand) {
-                const int i = s_cblk[j] * MID_BLOCK + (tid % MID_BLOCK);
-                if (i < v.n - 1) {
-                    const double dx = v.mid[2 * i] - px, dy = v.mid[2 * i + 1] - py;
-                    topk_insert(best, dx * dx + dy * dy, i);
-                }
-            }
-        }
-        block_topk(best, s_cand, s_knn[who]);
-    }
-    if (tid == 0) s_seg[0] = project_on_candidates(v, s_knn[0], KNN, s_pose[0], s_pose[1], s_proj[0], s_proj[1]);
-    if (tid == 32) s_seg[1] = project_on_candidates(v, s_knn[1], KNN, s_pose[2], s_pose[3], s_proj[2], s_proj[3]);
-
-    // ---- np.quantile(rng, wall_q) of the float32 lidar (rewards.py:335-339): radix select of the two order statistics
-    if (s_flag[2]) {
-        const float lm = (float)v.p.lidar_max;
-        for (int i = tid; i < B; i += RW_THREADS) {
-            float x = ob[i];
-            if (x <= 0.0f || !isfinite(x)) x = lm;                      // zeros / NaNs count as far
-            x = x < 0.0f ? 0.0f : (x > lm ? lm : x);
-            s_bits[i] = __float_as_uint(x);                             // x >= 0: unsigned order == float order
-        }
-        const float vi = (float)(B - 1) * (float)v.p.wall_quantile;     // numpy forms the virtual index in float32
-        const int lo = (int)floorf(vi);
-        if (tid == 0) { s_sel[0] = 0u; s_sel[1] = (unsigned)lo; }
-        __syncthreads();
-        for (int shift = 24; shift >= 0; shift -= 8) {
-            for (int b = tid; b < 256; b += RW_THREADS) s_hist[b] = 0u;
-            __syncthreads();
-            const unsigned prefix = s_sel[0];
-            const unsigned himask = shift == 24 ? 0u : (0xFFFFFFFFu << (shift + 8));
-            for (int i = tid; i < B; i += RW_THREADS) {
-                const unsigned u = s_bits[i];
-                if ((u & himask) == prefix) atomicAdd(&s_hist[(u >> shift) & 0xFFu], 1u);
-            }
-            __syncthreads();
-            if (tid < 32) {
-                // which of the 256 bins holds rank s_sel[1]?  lane l owns bins 8l..8l+7: warp scan of the lane sums, then
-                // the owning lane walks its own 8 bins
-                unsigned c[8], sum = 0;
-#pragma unroll
-                for (int j = 0; j < 8; ++j) { c[j] = s_hist[8 * tid + j]; sum += c[j]; }
-                unsigned incl = sum;
-                for (int o = 1; o < 32; o <<= 1) { const unsigned t = __shfl_up_sync(0xffffffffu, incl, o); if (tid >= o) incl += t; }
-                const unsigned rank = s_sel[1];
-                const unsigned excl = incl - sum;
-                const bool mine = rank >= excl && rank < incl;
-                const unsigned owner = __ffs(__ballot_sync(0xffffffffu, mine)) - 1;   // counts sum to >= rank + 1: exists
-                __syncwarp();
-                if (tid == (int)owner) {
-                    unsigned rem = rank - excl, b = 0;
-#pragma unroll
-                    for (int j = 0; j < 7; ++j) if (b == (unsigned)j && rem >= c[j]) { rem -= c[j]; ++b; }
-                    s_sel[0] = prefix | ((8u * tid + b) << shift);
-                    s_sel[1] = rem;
-                }
-            }
-            __syncthreads();
-        }
-        const unsigned vk = s_sel[0];                                   // bits of sorted[lo]
-        if (tid == 0) { s_sel[2] = 0u; s_sel[3] = 0xFFFFFFFFu; }
-        __syncthreads();
-        unsigned cnt = 0, mn = 0xFFFFFFFFu;
-        for (int i = tid; i < B; i += RW_THREADS) {
-            const unsigned u = s_bits[i];
-            if (u <= vk) ++cnt; else mn = u < mn ? u : mn;
-        }
-        atomicAdd(&s_sel[2], cnt);
-        atomicMin(&s_sel[3], mn);
-        __syncthreads();
-        if (tid == 0) {
-            const int hi = lo + 1 < B ? lo + 1 : B - 1;
-            const float a = __uint_as_float(vk);
-            const float b = (hi == lo || s_sel[2] >= (unsigned)(lo + 2)) ? a : __uint_as_float(s_sel[3]);
-            const float g = __fsub_rn(vi, (float)lo);
-            const float d = __fsub_rn(b, a);
-            // _lerp in float32: b - (b-a)*(1-g) for g >= 0.5, else a + (b-a)*g
-            s_q[0] = g >= 0.5f ? __fsub_rn(b, __fmul_rn(d, __fsub_rn(1.0f, g))) : __fadd_rn(a, __fmul_rn(d, g));
-        }
-    }
-    __syncthreads();
-
-    if (tid == 0) {
-        const double ex = s_pose[0], ey = s_pose[1], ox = s_pose[2], oy = s_pose[3], oth = s_pose[4];
-        const double e_s = s_proj[0], e_t = s_proj[1], o_s = s_proj[2], o_t = s_proj[3];
-        // _Prog.update :129-167
-        if (!r.has_s_prev[0]) { r.has_s_prev[0] = 1; r.s_prev[0] = e_s; }
-        if (!r.has_s_prev[1]) { r.has_s_prev[1] = 1; r.s_prev[1] = o_s; }
-        double de = signed_step(v, r, 0, ex, ey, e_s, r.s_prev[0], s_seg[0]);
-        double dop = signed_step(v, r, 1, ox, oy, o_s, r.s_prev[1], s_seg[1]);
-        r.s_prev[0] = e_s; r.s_prev[1] = o_s;
-        if (r.buf_n < 20) {
-            r.buf_sum += de; r.buf_n += 1;
-            if (r.buf_n == 20 && r.buf_sum / 20 < 0.0) r.flip = -1.0;
-        }
-        de *= r.flip; dop *= r.flip;
-        r.cum[0] += de; r.cum[1] += dop;
-        r.ema_abs = 0.8 * r.ema_abs + (1.0 - 0.8) * fabs(de);
-        r.t_last[0] = e_t; r.t_last[1] = o_t;
-        const int steps = s_flag[1];
-        double dego = de;
-        if (steps < 10 && dego < 0.0) dego = 0.0;                        // :311-312
-        const double r_prog = v.p.w_prog * v.p.forward_sign * dego;
-        const double r_alive = v.p.alive_bonus;
-        double r_lead = 0.0;
-        if (v.p.w_rel_lead != 0.0) {
-            double lead = r.cum[0] - r.cum[1];
-            lead = lead < -v.p.lead_clip ? -v.p.lead_clip : (lead > v.p.lead_clip ? v.p.lead_clip : lead);
-            r_lead = v.p.w_rel_lead * (lead / v.p.lead_clip);
-        }
-        const int idx = seg_index_at_s(v, e_s, s_seg[0]);                // lateral :323-333
-        double wR = v.p.default_half_width, wL = v.p.default_half_width;
-        if (v.wR && v.wL) { wR = v.wR[idx]; wL = v.wL[idx]; }
-        double w_eff = e_t >= 0.0 ? wL : wR;
-        w_eff = w_eff < 0.2 ? 0.2 : w_eff;
-        const double lat_norm = fabs(e_t) / w_eff;
-        const double lat_sq = lat_norm * lat_norm;
-        const double r_lat = -v.p.w_lat * (lat_sq < v.p.lat_cap ? lat_sq : v.p.lat_cap);
-        double r_wall = 0.0;                                             // :335-343
-        if (s_flag[2]) {
-            const double dmin = (double)s_q[0];
-            if (dmin < v.p.near_wall_dist) {
-                const double x = (v.p.near_wall_dist - dmin) / (v.p.near_wall_dist > 1e-6 ? v.p.near_wall_dist : 1e-6);
-                r_wall = -v.p.w_wall * (x * x);
-            }
-        }
-        double r_opp = 0.0;                                              // :345-352
-        if (steps >= v.p.grace_steps_opp) {
-            const double rho = hypot(ex - ox, ey - oy);
-            if (rho < v.p.opp_safe_dist) {
-                const double y = (v.p.opp_safe_dist - rho) / (v.p.opp_safe_dist > 1e-6 ? v.p.opp_safe_dist : 1e-6);
-                r_opp = -v.p.w_opp * (y * y);
-            }
-        }
-        double r_flank = 0.0;                                            // :353-358
-        {
-            const double dx = ex - ox, dy = ey - oy;
-            double sn, cs;
-            sincos(-oth, &sn, &cs);
-            const double x_rel = cs * dx - sn * dy, y_rel = sn * dx + cs * dy;
-            if (0.2 <= x_rel && x_rel <= 1.8 && 0.25 <= fabs(y_rel) && fabs(y_rel) <= 0.8) {
-                double yb = 0.8 - fabs(fabs(y_rel) - 0.525);
-                yb = yb < 0.0 ? 0.0 : yb;
-                r_flank = 0.1 * (x_rel / 1.8) * (yb / 0.8);
-            }
-        }
-        const double total = r_prog + r_alive + r_lead + r_lat + r_wall + r_opp + r_flank;
-        if (out64) out64[env] = total;
-        if (out32) out32[env] = (float)total;
-    }
+// the CTA-per-env kernel on a set of centerlines: each env on the line of its slot
+__global__ void __launch_bounds__(RW_THREADS) shaped_reward_set_kernel(RewardView base, RewardSetView rs, const float* __restrict__ obs,
+                                                                       const uint8_t* __restrict__ reset_mask,
+                                                                       double* __restrict__ out64, float* __restrict__ out32) {
+#define F110_REWARD_SET 1
+#include "f110_reward_cta_body.cuh"
+#undef F110_REWARD_SET
 }
 
 
@@ -645,257 +467,53 @@ __device__ __forceinline__ size_t reward_warp_smem_bytes(int B) { return sizeof(
 __global__ void __launch_bounds__(RWW_MAX * 32) shaped_reward_warp_kernel(RewardView v, const float* __restrict__ obs,
                                                                           const uint8_t* __restrict__ reset_mask,
                                                                           double* __restrict__ out64, float* __restrict__ out32) {
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    const int env = blockIdx.x * (blockDim.x >> 5) + wid;
-    if (env >= v.p.num_envs) return;
-    const int B = v.p.num_beams;
-    extern __shared__ __align__(16) unsigned char s_raw[];
-    unsigned char* mine = s_raw + (size_t)wid * ((reward_warp_smem_bytes(B) + 15) & ~size_t(15));
-    double* s_lb = reinterpret_cast<double*>(mine);                       // [256] lower bound of every midpoint block
-    unsigned* s_bits = reinterpret_cast<unsigned*>(s_lb + 256);           // [B] lidar as order-preserving unsigned
-    unsigned* s_hist = s_bits + B;                                        // [256]
-    int* s_cblk = reinterpret_cast<int*>(s_hist + 256);                   // [256]
-    int* s_knn = s_cblk + 256;                                            // [2][KNN]
-    const float* ob = obs + (size_t)env * (B + 8);
-    // the env's progress state lives in lane 0's registers for the duration of the kernel: one load of the record and one
-    // store, instead of a dependent global access per field of the state machine
-    RewardState r;
-    memset(&r, 0, sizeof(r));
+#define F110_REWARD_SET 0
+#include "f110_reward_warp_body.cuh"
+#undef F110_REWARD_SET
+}
 
-    double pose[5] = {0., 0., 0., 0., 0.};                                // ex, ey, ox, oy, oth
-    int early = 0, steps = 0, do_wall = 0;
-    if (lane == 0) {
-        if (reset_mask && reset_mask[env]) {        // reward_fn.reset() (rewards.py:262-264, _Prog.reset :98-106)
-            r.flip = +1.0;                          // everything else zero
-        } else {
-            r = v.st[env];
-        }
-        // parse_flat_obs :11-39 (the float32 fields are widened by float())
-        pose[0] = (double)ob[B + 0]; pose[1] = (double)ob[B + 1];
-        pose[2] = (double)ob[B + 4]; pose[3] = (double)ob[B + 5];
-        double th = (double)ob[B + 6] + 3.141592653589793;
-        double m = fmod(th, 2 * 3.141592653589793);
-        if (m != 0.0) { if (m < 0.0) m += 2 * 3.141592653589793; } else m = 0.0;
-        pose[4] = m - 3.141592653589793;
-        const bool ego_col = ob[B + 3] != 0.0f, opp_col = ob[B + 7] != 0.0f;
-        r.steps += 1;                                                   // :299
-        steps = r.steps;
-        if (ego_col) { early = 1; if (out64) out64[env] = -v.p.ego_crash_penalty; if (out32) out32[env] = (float)-v.p.ego_crash_penalty; }
-        else if (opp_col && v.p.opp_crash_bonus > 0.0) { early = 1; if (out64) out64[env] = v.p.opp_crash_bonus; if (out32) out32[env] = (float)v.p.opp_crash_bonus; }
-        do_wall = r.steps >= v.p.grace_steps_wall;
-        if (early) v.st[env] = r;
-    }
-    early = __shfl_sync(0xffffffffu, early, 0);
-    if (early) return;
-    steps = __shfl_sync(0xffffffffu, steps, 0);
-    do_wall = __shfl_sync(0xffffffffu, do_wall, 0);
-#pragma unroll
-    for (int k = 0; k < 5; ++k) pose[k] = __shfl_sync(0xffffffffu, pose[k], 0);
-
-    // ---- 5 nearest midpoints of both cars, exactly (see the CTA kernel for the bounding-circle argument)
-    for (int who = 0; who < 2; ++who) {
-        const double px = pose[2 * who], py = pose[2 * who + 1];
-        double ub = INFINITY;
-        for (int k = lane; k < v.nblk; k += 32) {
-            const double dx = v.blk[3 * k] - px, dy = v.blk[3 * k + 1] - py, R = v.blk[3 * k + 2];
-            const double d = sqrt(dx * dx + dy * dy);
-            s_lb[k] = d - R;
-            const int cnt = min(MID_BLOCK, v.n - 1 - k * MID_BLOCK);
-            if (cnt >= KNN) ub = fmin(ub, d + R);
-        }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) ub = fmin(ub, __shfl_xor_sync(0xffffffffu, ub, o));
-        const double tau = ub * (1.0 + 1e-12) + 1e-12;                  // slack for the rounding of the bounds
-        __syncwarp();
-        int ncand = 0;
-        for (int k0 = 0; k0 < v.nblk; k0 += 32) {
-            const int k = k0 + lane;
-            const bool keep = k < v.nblk && (!(tau < INFINITY) || s_lb[k] <= tau);
-            const unsigned m = __ballot_sync(0xffffffffu, keep);
-            if (keep) s_cblk[ncand + __popc(m & ((1u << lane) - 1u))] = k;
-            ncand += __popc(m);
-        }
-        __syncwarp();
-        Cand best[KNN];
-#pragma unroll
-        for (int k = 0; k < KNN; ++k) { best[k].d2 = INFINITY; best[k].idx = 0x7fffffff; }
-        for (int j = 0; j < ncand; ++j) {
-            const int base = s_cblk[j] * MID_BLOCK;
-#pragma unroll
-            for (int t = 0; t < MID_BLOCK / 32; ++t) {
-                const int i = base + 32 * t + lane;
-                if (i < v.n - 1) {
-                    const double dx = v.mid[2 * i] - px, dy = v.mid[2 * i + 1] - py;
-                    topk_insert(best, dx * dx + dy * dy, i);
-                }
-            }
-        }
-        // the warp's KNN smallest (d2, idx): every round the lanes offer the head of their sorted private lists
-        int head = 0;
-        for (int round = 0; round < KNN; ++round) {
-            Cand cnd;
-            cnd.d2 = INFINITY; cnd.idx = 0x7fffffff;
-#pragma unroll
-            for (int k = 0; k < KNN; ++k) if (k == head) cnd = best[k];
-            const unsigned long long bits = (unsigned long long)__double_as_longlong(cnd.d2);     // d2 >= 0: bits order like the value
-            const unsigned hi = (unsigned)(bits >> 32), lo = (unsigned)bits;
-            const unsigned mhi = __reduce_min_sync(0xffffffffu, hi);
-            const unsigned mlo = __reduce_min_sync(0xffffffffu, hi == mhi ? lo : 0xFFFFFFFFu);
-            const unsigned midx = __reduce_min_sync(0xffffffffu, (hi == mhi && lo == mlo) ? (unsigned)cnd.idx : 0x7FFFFFFFu);
-            if ((int)midx == cnd.idx && cnd.idx != 0x7fffffff) ++head;      // a midpoint index belongs to exactly one lane
-            if (lane == 0) s_knn[who * KNN + round] = midx == 0x7FFFFFFFu ? -1 : (int)midx;
-        }
-        __syncwarp();
-    }
-    // projections: lane 0 the ego, lane 1 the opponent (same code, different data: no divergence)
-    double p_s = 0., p_t = 0.;
-    int p_seg = 0;
-    if (lane < 2) p_seg = project_on_candidates(v, s_knn + lane * KNN, KNN, pose[2 * lane], pose[2 * lane + 1], p_s, p_t);
-    const double o_s = __shfl_sync(0xffffffffu, p_s, 1), o_t = __shfl_sync(0xffffffffu, p_t, 1);
-    const int seg1 = __shfl_sync(0xffffffffu, p_seg, 1);
-
-    // ---- np.quantile(rng, wall_q) of the float32 lidar (rewards.py:335-339): radix select of the two order statistics
-    float q_wall = 0.f;
-    if (do_wall) {
-        const float lm = (float)v.p.lidar_max;
-        for (int i = lane; i < B; i += 32) {
-            float x = ob[i];
-            if (x <= 0.0f || !isfinite(x)) x = lm;                      // zeros / NaNs count as far
-            x = x < 0.0f ? 0.0f : (x > lm ? lm : x);
-            s_bits[i] = __float_as_uint(x);                             // x >= 0: unsigned order == float order
-        }
-        const float vi = (float)(B - 1) * (float)v.p.wall_quantile;     // numpy forms the virtual index in float32
-        const int lo = (int)floorf(vi);
-        unsigned prefix = 0u, rank = (unsigned)lo;
-        for (int shift = 24; shift >= 0; shift -= 8) {
-#pragma unroll
-            for (int j = 0; j < 8; ++j) s_hist[8 * lane + j] = 0u;
-            __syncwarp();
-            const unsigned himask = shift == 24 ? 0u : (0xFFFFFFFFu << (shift + 8));
-            for (int i = lane; i < B; i += 32) {
-                const unsigned u = s_bits[i];
-                if ((u & himask) == prefix) atomicAdd(&s_hist[(u >> shift) & 0xFFu], 1u);
-            }
-            __syncwarp();
-            // which of the 256 bins holds the rank?  lane l owns bins 8l..8l+7: warp scan of the lane sums, then the owning
-            // lane walks its own 8 bins
-            unsigned c[8], sum = 0;
-#pragma unroll
-            for (int j = 0; j < 8; ++j) { c[j] = s_hist[8 * lane + j]; sum += c[j]; }
-            unsigned incl = sum;
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) { const unsigned t = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += t; }
-            const unsigned excl = incl - sum;
-            const bool own = rank >= excl && rank < incl;
-            const int owner = __ffs(__ballot_sync(0xffffffffu, own)) - 1;    // counts sum to >= rank + 1: exists
-            unsigned np = 0, nr = 0;
-            if (lane == owner) {
-                unsigned rem = rank - excl, b = 0;
-#pragma unroll
-                for (int j = 0; j < 7; ++j) if (b == (unsigned)j && rem >= c[j]) { rem -= c[j]; ++b; }
-                np = prefix | ((8u * lane + b) << shift);
-                nr = rem;
-            }
-            prefix = __shfl_sync(0xffffffffu, np, owner);
-            rank = __shfl_sync(0xffffffffu, nr, owner);
-            __syncwarp();
-        }
-        const unsigned vk = prefix;                                     // bits of sorted[lo]
-        unsigned cnt = 0, mn = 0xFFFFFFFFu;
-        for (int i = lane; i < B; i += 32) {
-            const unsigned u = s_bits[i];
-            if (u <= vk) ++cnt; else mn = u < mn ? u : mn;
-        }
-        cnt = __reduce_add_sync(0xffffffffu, cnt);
-        mn = __reduce_min_sync(0xffffffffu, mn);
-        const int hi = lo + 1 < B ? lo + 1 : B - 1;
-        const float a = __uint_as_float(vk);
-        const float b = (hi == lo || cnt >= (unsigned)(lo + 2)) ? a : __uint_as_float(mn);
-        const float g = __fsub_rn(vi, (float)lo);
-        const float d = __fsub_rn(b, a);
-        // _lerp in float32: b - (b-a)*(1-g) for g >= 0.5, else a + (b-a)*g
-        q_wall = g >= 0.5f ? __fsub_rn(b, __fmul_rn(d, __fsub_rn(1.0f, g))) : __fadd_rn(a, __fmul_rn(d, g));
-    }
-
-    if (lane == 0) {
-        const double ex = pose[0], ey = pose[1], ox = pose[2], oy = pose[3], oth = pose[4];
-        const double e_s = p_s, e_t = p_t;
-        const int seg0 = p_seg;
-        // _Prog.update :129-167
-        if (!r.has_s_prev[0]) { r.has_s_prev[0] = 1; r.s_prev[0] = e_s; }
-        if (!r.has_s_prev[1]) { r.has_s_prev[1] = 1; r.s_prev[1] = o_s; }
-        double de = signed_step(v, r, 0, ex, ey, e_s, r.s_prev[0], seg0);
-        double dop = signed_step(v, r, 1, ox, oy, o_s, r.s_prev[1], seg1);
-        r.s_prev[0] = e_s; r.s_prev[1] = o_s;
-        if (r.buf_n < 20) {
-            r.buf_sum += de; r.buf_n += 1;
-            if (r.buf_n == 20 && r.buf_sum / 20 < 0.0) r.flip = -1.0;
-        }
-        de *= r.flip; dop *= r.flip;
-        r.cum[0] += de; r.cum[1] += dop;
-        r.ema_abs = 0.8 * r.ema_abs + (1.0 - 0.8) * fabs(de);
-        r.t_last[0] = e_t; r.t_last[1] = o_t;
-        double dego = de;
-        if (steps < 10 && dego < 0.0) dego = 0.0;                        // :311-312
-        const double r_prog = v.p.w_prog * v.p.forward_sign * dego;
-        const double r_alive = v.p.alive_bonus;
-        double r_lead = 0.0;
-        if (v.p.w_rel_lead != 0.0) {
-            double lead = r.cum[0] - r.cum[1];
-            lead = lead < -v.p.lead_clip ? -v.p.lead_clip : (lead > v.p.lead_clip ? v.p.lead_clip : lead);
-            r_lead = v.p.w_rel_lead * (lead / v.p.lead_clip);
-        }
-        const int idx = seg_index_at_s(v, e_s, seg0);                    // lateral :323-333
-        double wR = v.p.default_half_width, wL = v.p.default_half_width;
-        if (v.wR && v.wL) { wR = v.wR[idx]; wL = v.wL[idx]; }
-        double w_eff = e_t >= 0.0 ? wL : wR;
-        w_eff = w_eff < 0.2 ? 0.2 : w_eff;
-        const double lat_norm = fabs(e_t) / w_eff;
-        const double lat_sq = lat_norm * lat_norm;
-        const double r_lat = -v.p.w_lat * (lat_sq < v.p.lat_cap ? lat_sq : v.p.lat_cap);
-        double r_wall = 0.0;                                             // :335-343
-        if (do_wall) {
-            const double dmin = (double)q_wall;
-            if (dmin < v.p.near_wall_dist) {
-                const double x = (v.p.near_wall_dist - dmin) / (v.p.near_wall_dist > 1e-6 ? v.p.near_wall_dist : 1e-6);
-                r_wall = -v.p.w_wall * (x * x);
-            }
-        }
-        double r_opp = 0.0;                                              // :345-352
-        if (steps >= v.p.grace_steps_opp) {
-            const double rho = hypot(ex - ox, ey - oy);
-            if (rho < v.p.opp_safe_dist) {
-                const double y = (v.p.opp_safe_dist - rho) / (v.p.opp_safe_dist > 1e-6 ? v.p.opp_safe_dist : 1e-6);
-                r_opp = -v.p.w_opp * (y * y);
-            }
-        }
-        double r_flank = 0.0;                                            // :353-358
-        {
-            const double dx = ex - ox, dy = ey - oy;
-            double sn, cs;
-            sincos(-oth, &sn, &cs);
-            const double x_rel = cs * dx - sn * dy, y_rel = sn * dx + cs * dy;
-            if (0.2 <= x_rel && x_rel <= 1.8 && 0.25 <= fabs(y_rel) && fabs(y_rel) <= 0.8) {
-                double yb = 0.8 - fabs(fabs(y_rel) - 0.525);
-                yb = yb < 0.0 ? 0.0 : yb;
-                r_flank = 0.1 * (x_rel / 1.8) * (yb / 0.8);
-            }
-        }
-        const double total = r_prog + r_alive + r_lead + r_lat + r_wall + r_opp + r_flank;
-        if (out64) out64[env] = total;
-        if (out32) out32[env] = (float)total;
-        v.st[env] = r;
-    }
+// the warp-per-env kernel on a set of centerlines: each env on the line of its slot
+__global__ void __launch_bounds__(RWW_MAX * 32) shaped_reward_set_warp_kernel(RewardView v, RewardSetView rs, const float* __restrict__ obs,
+                                                                              const uint8_t* __restrict__ reset_mask,
+                                                                              double* __restrict__ out64, float* __restrict__ out32) {
+#define F110_REWARD_SET 1
+#include "f110_reward_warp_body.cuh"
+#undef F110_REWARD_SET
 }
 
 }  // namespace
 
-extern "C" int f110_reward_create(const F110RewardConfig* cfg, const double* xy, const double* wR, const double* wL,
-                                  F110Reward** out) {
-    if (!cfg || !xy || !out || cfg->num_envs < 1 || cfg->num_points < 2 || cfg->num_beams < 1 || cfg->num_beams > 8192)
-        return f110_set_error(F110_ERR_INVALID, "f110_reward_create: need num_envs >= 1, num_points >= 2, 1 <= num_beams <= 8192");
-    if ((cfg->num_points - 1 + MID_BLOCK - 1) / MID_BLOCK > 256)
-        return f110_set_error(F110_ERR_INVALID, "f110_reward_create: at most 16385 centerline points");
+namespace {
+
+// Checks every line against the limits before anything is allocated; the message names the failing line and its limit.
+int check_lines(const char* who, const F110RewardConfig* cfg, const F110Centerline* lines, int32_t count, F110Reward** out) {
+    char msg[256];
+    if (!cfg || !lines || !out || cfg->num_envs < 1 || cfg->num_beams < 1 || cfg->num_beams > 8192) {
+        snprintf(msg, sizeof(msg), "%s: need non-null arguments, num_envs >= 1, 1 <= num_beams <= 8192", who);
+        return f110_set_error(F110_ERR_INVALID, msg);
+    }
+    if (count < 1 || count > F110_MAX_MAPS) {
+        snprintf(msg, sizeof(msg), "%s: %d centerlines; 1 to %d allowed", who, (int)count, F110_MAX_MAPS);
+        return f110_set_error(F110_ERR_INVALID, msg);
+    }
+    for (int k = 0; k < count; ++k) {
+        const int n = lines[k].num_points;
+        if (!lines[k].xy) {
+            snprintf(msg, sizeof(msg), "%s: centerline %d has no points (xy is NULL)", who, k);
+            return f110_set_error(F110_ERR_INVALID, msg);
+        }
+        if (n < 2 || (n - 1 + MID_BLOCK - 1) / MID_BLOCK > 256) {
+            snprintf(msg, sizeof(msg), "%s: centerline %d has %d points; 2 to 16385 allowed (at most 256 blocks of %d midpoints)",
+                     who, k, n, MID_BLOCK);
+            return f110_set_error(F110_ERR_INVALID, msg);
+        }
+    }
+    return F110_OK;
+}
+
+int reward_create(const char* who, const F110RewardConfig* cfg, const F110Centerline* lines, int32_t count, F110Reward** out) {
+    const int rc = check_lines(who, cfg, lines, count, out);
+    if (rc != F110_OK) return rc;
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
         cudaGetLastError();
@@ -905,76 +523,123 @@ extern "C" int f110_reward_create(const F110RewardConfig* cfg, const double* xy,
     cudaGetDevice(&prev);
     if (cudaSetDevice(cfg->device) != cudaSuccess) return F110_ERR_CUDA;
     F110Reward* r = new F110Reward();
-    r->cfg = *cfg; r->n = cfg->num_points; r->device = cfg->device;
-    const int n = r->n;
-    // CenterlineProgress.__init__, track_progress.py:33-49 (host, once)
-    double* s = new double[n];
-    double* tan = new double[2 * (n - 1)];
-    double* nrm = new double[2 * (n - 1)];
-    double* mid = new double[2 * (n - 1)];
-    s[0] = 0.0;
-    for (int i = 0; i < n - 1; ++i) {
-        const double sx = xy[2 * i + 2] - xy[2 * i], sy = xy[2 * i + 3] - xy[2 * i + 1];
-        const double len = sqrt(sx * sx + sy * sy);
-        s[i + 1] = s[i] + len;
-        const double den = len > 1e-12 ? len : 1e-12;
-        tan[2 * i] = sx / den; tan[2 * i + 1] = sy / den;
-        nrm[2 * i] = -tan[2 * i + 1]; nrm[2 * i + 1] = tan[2 * i];
-        mid[2 * i] = (xy[2 * i] + xy[2 * i + 2]) * 0.5; mid[2 * i + 1] = (xy[2 * i + 1] + xy[2 * i + 3]) * 0.5;
+    r->cfg = *cfg; r->device = cfg->device; r->count = count;
+    if (count == 1) { r->cfg.num_points = lines[0].num_points; r->cfg.closed = lines[0].closed; }
+    // the lines back to back: line k's points from off[k] on, its blocks from boff[k] on
+    std::vector<RewardLine> table(count);
+    size_t total = 0, total_blk = 0;
+    bool widths = false;
+    for (int k = 0; k < count; ++k) {
+        RewardLine& t = table[k];
+        t.off = (int)total; t.n = lines[k].num_points; t.boff = (int)total_blk;
+        t.nblk = (t.n - 1 + MID_BLOCK - 1) / MID_BLOCK;
+        t.closed = lines[k].closed; t.has_widths = lines[k].wR && lines[k].wL;
+        widths = widths || t.has_widths;
+        total += t.n; total_blk += t.nblk;
     }
-    r->L = s[n - 1];
-    auto up = [](const double* h, size_t cnt, double** d) {
-        if (cudaMalloc(d, cnt * sizeof(double)) != cudaSuccess) return false;
-        return cudaMemcpy(*d, h, cnt * sizeof(double), cudaMemcpyHostToDevice) == cudaSuccess;
-    };
-    bool ok = up(xy, 2 * (size_t)n, &r->xy) && up(s, n, &r->s) && up(tan, 2 * (size_t)(n - 1), &r->tan) &&
-              up(nrm, 2 * (size_t)(n - 1), &r->nrm) && up(mid, 2 * (size_t)(n - 1), &r->mid);
-    r->wR = r->wL = nullptr;
-    if (ok && wR && wL) ok = up(wR, n, &r->wR) && up(wL, n, &r->wL);
-    {   // bounding circles of MID_BLOCK consecutive midpoints
-        r->nblk = (n - 1 + MID_BLOCK - 1) / MID_BLOCK;
-        std::vector<double> blk(3 * (size_t)r->nblk);
-        for (int k = 0; k < r->nblk; ++k) {
-            const int i0 = k * MID_BLOCK, i1 = (k + 1) * MID_BLOCK < n - 1 ? (k + 1) * MID_BLOCK : n - 1;
+    std::vector<double> xy(2 * total), s(total), tan(2 * total), nrm(2 * total), mid(2 * total), blk(3 * total_blk);
+    std::vector<double> wR(widths ? total : 0), wL(widths ? total : 0);
+    for (int k = 0; k < count; ++k) {
+        RewardLine& t = table[k];
+        const int n = t.n;
+        const double* src = lines[k].xy;
+        double *pxy = &xy[2 * (size_t)t.off], *ps = &s[t.off], *ptan = &tan[2 * (size_t)t.off], *pnrm = &nrm[2 * (size_t)t.off];
+        double* pmid = &mid[2 * (size_t)t.off];
+        memcpy(pxy, src, 2 * (size_t)n * sizeof(double));
+        if (t.has_widths) {
+            memcpy(&wR[t.off], lines[k].wR, (size_t)n * sizeof(double));
+            memcpy(&wL[t.off], lines[k].wL, (size_t)n * sizeof(double));
+        }
+        // CenterlineProgress.__init__, track_progress.py:33-49 (host, once)
+        ps[0] = 0.0;
+        for (int i = 0; i < n - 1; ++i) {
+            const double sx = src[2 * i + 2] - src[2 * i], sy = src[2 * i + 3] - src[2 * i + 1];
+            const double len = sqrt(sx * sx + sy * sy);
+            ps[i + 1] = ps[i] + len;
+            const double den = len > 1e-12 ? len : 1e-12;
+            ptan[2 * i] = sx / den; ptan[2 * i + 1] = sy / den;
+            pnrm[2 * i] = -ptan[2 * i + 1]; pnrm[2 * i + 1] = ptan[2 * i];
+            pmid[2 * i] = (src[2 * i] + src[2 * i + 2]) * 0.5; pmid[2 * i + 1] = (src[2 * i + 1] + src[2 * i + 3]) * 0.5;
+        }
+        t.L = ps[n - 1];
+        for (int b = 0; b < t.nblk; ++b) {      // bounding circles of MID_BLOCK consecutive midpoints
+            const int i0 = b * MID_BLOCK, i1 = (b + 1) * MID_BLOCK < n - 1 ? (b + 1) * MID_BLOCK : n - 1;
             double cx = 0, cy = 0;
-            for (int i = i0; i < i1; ++i) { cx += mid[2 * i]; cy += mid[2 * i + 1]; }
+            for (int i = i0; i < i1; ++i) { cx += pmid[2 * i]; cy += pmid[2 * i + 1]; }
             cx /= (i1 - i0); cy /= (i1 - i0);
             double R = 0;
-            for (int i = i0; i < i1; ++i) { const double d = sqrt((mid[2 * i] - cx) * (mid[2 * i] - cx) + (mid[2 * i + 1] - cy) * (mid[2 * i + 1] - cy)); R = d > R ? d : R; }
-            blk[3 * k] = cx; blk[3 * k + 1] = cy; blk[3 * k + 2] = R * (1.0 + 1e-12) + 1e-12;
+            for (int i = i0; i < i1; ++i) { const double d = sqrt((pmid[2 * i] - cx) * (pmid[2 * i] - cx) + (pmid[2 * i + 1] - cy) * (pmid[2 * i + 1] - cy)); R = d > R ? d : R; }
+            double* pb = &blk[3 * ((size_t)t.boff + b)];
+            pb[0] = cx; pb[1] = cy; pb[2] = R * (1.0 + 1e-12) + 1e-12;
         }
-        r->blk = nullptr;
-        if (ok) ok = r->nblk <= 256 && up(blk.data(), blk.size(), &r->blk);
     }
-    delete[] s; delete[] tan; delete[] nrm; delete[] mid;
+    r->n = table[0].n; r->L = table[0].L; r->nblk = table[0].nblk;
+    auto up = [](const void* h, size_t bytes, void** d) {
+        if (cudaMalloc(d, bytes) != cudaSuccess) return false;
+        return cudaMemcpy(*d, h, bytes, cudaMemcpyHostToDevice) == cudaSuccess;
+    };
+    auto upd = [&](const std::vector<double>& h, double** d) { return up(h.data(), h.size() * sizeof(double), reinterpret_cast<void**>(d)); };
+    bool ok = upd(xy, &r->xy) && upd(s, &r->s) && upd(tan, &r->tan) && upd(nrm, &r->nrm) && upd(mid, &r->mid) && upd(blk, &r->blk);
+    if (ok && widths) ok = upd(wR, &r->wR) && upd(wL, &r->wL);
+    if (ok && count > 1) {
+        std::vector<int> minus1(cfg->num_envs, -1);
+        ok = up(table.data(), table.size() * sizeof(RewardLine), &r->lines) &&
+             up(minus1.data(), minus1.size() * sizeof(int), reinterpret_cast<void**>(&r->prev_slot));
+    }
     if (ok) {
         std::vector<RewardState> init(cfg->num_envs);
         memset(init.data(), 0, sizeof(RewardState) * init.size());
         for (auto& st : init) st.flip = +1.0;
-        ok = cudaMalloc(&r->state, sizeof(RewardState) * init.size()) == cudaSuccess &&
-             cudaMemcpy(r->state, init.data(), sizeof(RewardState) * init.size(), cudaMemcpyHostToDevice) == cudaSuccess;
+        ok = up(init.data(), sizeof(RewardState) * init.size(), &r->state);
     }
     cudaSetDevice(prev);
-    if (!ok) { f110_reward_destroy(r); cudaGetLastError(); return f110_set_error(F110_ERR_CUDA, "f110_reward_create: device allocation / upload failed"); }
+    if (!ok) {
+        f110_reward_destroy(r);
+        cudaGetLastError();
+        char msg[128];
+        snprintf(msg, sizeof(msg), "%s: device allocation / upload failed", who);
+        return f110_set_error(F110_ERR_CUDA, msg);
+    }
     *out = r;
     return F110_OK;
 }
 
+}  // namespace
+
+extern "C" int f110_reward_create_set(const F110RewardConfig* cfg, const F110Centerline* lines, int32_t count, F110Reward** out) {
+    return reward_create("f110_reward_create_set", cfg, lines, count, out);
+}
+
+extern "C" int f110_reward_create(const F110RewardConfig* cfg, const double* xy, const double* wR, const double* wL,
+                                  F110Reward** out) {
+    if (!cfg || !xy || !out) return f110_set_error(F110_ERR_INVALID, "f110_reward_create: null config, centerline or handle");
+    F110Centerline line;
+    line.xy = xy; line.wR = wR; line.wL = wL; line.num_points = cfg->num_points; line.closed = cfg->closed;
+    return reward_create("f110_reward_create", cfg, &line, 1, out);
+}
+
+extern "C" int32_t f110_reward_count(const F110Reward* r) { return r ? r->count : 0; }
+
 extern "C" void f110_reward_destroy(F110Reward* r) {
     if (!r) return;
     cudaFree(r->xy); cudaFree(r->s); cudaFree(r->tan); cudaFree(r->nrm); cudaFree(r->mid); cudaFree(r->wR); cudaFree(r->wL);
-    cudaFree(r->blk); cudaFree(r->state);
+    cudaFree(r->blk); cudaFree(r->state); cudaFree(r->lines); cudaFree(r->prev_slot);
     delete r;
 }
 
-extern "C" int f110_reward_compute(F110Reward* r, const float* obs, const uint8_t* reset_mask, double* out_f64, float* out_f32,
-                                   void* stream) {
+extern "C" int f110_reward_compute_slots(F110Reward* r, const float* obs, const uint8_t* reset_mask, const int32_t* slots,
+                                         double* out_f64, float* out_f32, void* stream) {
     if (!r || !obs || (!out_f64 && !out_f32)) return f110_set_error(F110_ERR_INVALID, "f110_reward_compute: null handle, obs or outputs");
+    if (r->count > 1 && !slots)
+        return f110_set_error(F110_ERR_INVALID, "f110_reward_compute_slots: a set of centerlines needs the envs' slots");
     RewardView v;
     v.p = r->cfg; v.n = r->n; v.L = r->L;
     v.blk = r->blk; v.nblk = r->nblk;
     v.xy = r->xy; v.s = r->s; v.tan = r->tan; v.nrm = r->nrm; v.mid = r->mid; v.wR = r->wR; v.wL = r->wL;
     v.st = static_cast<RewardState*>(r->state);
+    RewardSetView rs;
+    rs.lines = static_cast<const RewardLine*>(r->lines); rs.slots = slots; rs.prev = r->prev_slot; rs.count = r->count;
+    const bool set = r->count > 1;       // a set of one runs the single-line kernels and reads no slot
     // a warp per env where a warp's scratch (the scan as sortable words, a histogram, the block bounds) fits the 48 KB of
     // shared memory that need no opt-in; else (scans of more than ~11 000 beams) the CTA-per-env form
     const int B = r->cfg.num_beams;
@@ -983,11 +648,21 @@ extern "C" int f110_reward_compute(F110Reward* r, const float* obs, const uint8_
     if (per_warp <= 48 * 1024 && !(force_cta && force_cta[0] == '1')) {
         int warps = (int)((48 * 1024) / per_warp);
         warps = warps > RWW_MAX ? RWW_MAX : warps;
-        shaped_reward_warp_kernel<<<(r->cfg.num_envs + warps - 1) / warps, warps * 32, per_warp * warps, (cudaStream_t)stream>>>(
-            v, obs, reset_mask, out_f64, out_f32);
+        const dim3 grid((r->cfg.num_envs + warps - 1) / warps), block(warps * 32);
+        if (set) shaped_reward_set_warp_kernel<<<grid, block, per_warp * warps, (cudaStream_t)stream>>>(v, rs, obs, reset_mask, out_f64, out_f32);
+        else shaped_reward_warp_kernel<<<grid, block, per_warp * warps, (cudaStream_t)stream>>>(v, obs, reset_mask, out_f64, out_f32);
     } else {
-        shaped_reward_kernel<<<r->cfg.num_envs, RW_THREADS, sizeof(unsigned) * r->cfg.num_beams, (cudaStream_t)stream>>>(
-            v, obs, reset_mask, out_f64, out_f32);
+        const size_t smem = sizeof(unsigned) * r->cfg.num_beams;
+        if (set) shaped_reward_set_kernel<<<r->cfg.num_envs, RW_THREADS, smem, (cudaStream_t)stream>>>(v, rs, obs, reset_mask, out_f64, out_f32);
+        else shaped_reward_kernel<<<r->cfg.num_envs, RW_THREADS, smem, (cudaStream_t)stream>>>(v, obs, reset_mask, out_f64, out_f32);
     }
     return cudaPeekAtLastError() == cudaSuccess ? F110_OK : F110_ERR_CUDA;
+}
+
+extern "C" int f110_reward_compute(F110Reward* r, const float* obs, const uint8_t* reset_mask, double* out_f64, float* out_f32,
+                                   void* stream) {
+    if (r && r->count > 1)
+        return f110_set_error(F110_ERR_INVALID, "f110_reward_compute: this reward holds a set of centerlines; call "
+                                                "f110_reward_compute_slots with the envs' slots");
+    return f110_reward_compute_slots(r, obs, reset_mask, nullptr, out_f64, out_f32, stream);
 }

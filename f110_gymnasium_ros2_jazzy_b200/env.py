@@ -222,7 +222,8 @@ class F110VecEnv(object):
 
     ``maps=[spec, ...]`` instead of ``map=`` / ``map_arrays=`` installs a map set (BatchSim.set_maps): every env drives on
     the map of its slot, env e on slot floor(e * K / N) unless ``env_maps`` (int [N]) says otherwise; ``reassign`` moves envs
-    to other maps at their next reset.  The shaped reward (ShapedReward, DeviceRollout) stays single-centerline.
+    to other maps at their next reset.  ShapedReward(centerlines=[...]) with one centerline per map, in slot order, scores
+    each env on its own map's centerline (DeviceRollout passes it the slots).
     """
 
     def __init__(self, num_envs, map_dir=None, map=None, map_ext='.png', num_agents=2, params=None, seed=42,

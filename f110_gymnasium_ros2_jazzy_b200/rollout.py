@@ -63,8 +63,9 @@ class Actor(torch.nn.Module):
 class DeviceRollout(object):
     """ego = policy(obs), opponent = gap-follow on its own scan, env.step -- no host round trip per step.
 
-    ``reward_fn`` (optional, e.g. ShapedReward) replaces the env's constant reward, as train_ddpg.py:179 does.  Its
-    centerline is one track's: with a map set (F110VecEnv(maps=...)) the reward does not follow the envs' slots.
+    ``reward_fn`` (optional, e.g. ShapedReward) replaces the env's constant reward, as train_ddpg.py:179 does.  A reward
+    with K > 1 centerlines needs a map set of K maps (F110VecEnv(maps=...)): every step it is passed the envs' slots, so
+    each env is scored on its own map's centerline, whatever moved it there (set_env_maps, reassign, load_state_dict).
     ``replay`` (optional, e.g. DeviceReplayBuffer) receives every transition (obs, ego action, reward, next obs, done)
     except the auto-reset steps (see step).
     ``env`` is an F110VecEnv with num_agents == 2 and 'scans_f32' among its outputs; ``policy`` maps the observation
@@ -83,6 +84,13 @@ class DeviceRollout(object):
             self.actions[:, 1, 1] = float(opponent[1])
         self.obs = None
         self.reward_fn = reward_fn          # e.g. ShapedReward: train_ddpg.py:179 discards the env's reward for it
+        self._slots = None
+        k = getattr(reward_fn, 'num_centerlines', 1)
+        if k > 1:
+            if env.backend.num_maps != k:
+                raise ValueError("a reward with %d centerlines needs a map set of %d maps (the env has %d)"
+                                 % (k, k, env.backend.num_maps))
+            self._slots = torch.zeros(env.num_envs, dtype=torch.int32, device=env.device)   # refreshed every step
         self.reward = None
         self.replay = replay                # e.g. DeviceReplayBuffer: agent.remember(obs, ego_action, r, next_obs, done), :185
         self._prev_obs = None if replay is None else torch.zeros((env.num_envs,) + tuple(env.single_observation_shape),
@@ -116,7 +124,10 @@ class DeviceRollout(object):
         if self.reward_fn is not None:
             # reward object restarted on the reset step itself (its value there is discarded) and again on the first real step
             torch.maximum(self._resetting, self._first, out=self._fresh)
-            reward = self.reward_fn(self.obs, self._fresh)
+            if self._slots is None:
+                reward = self.reward_fn(self.obs, self._fresh)
+            else:
+                reward = self.reward_fn(self.obs, self._fresh, slots=self.env.backend.env_maps(out=self._slots))
             reward.masked_fill_(self._resetting.bool(), 0.0)
         self.reward = reward
         if self.replay is not None:
@@ -240,47 +251,73 @@ REWARD_DEFAULTS = dict(dt=0.01, w_prog=1.2, forward_sign=+1.0, alive_bonus=0.02,
 class ShapedReward(object):
     """Batched CenterlineSafetyProgressReward (rewards.py:185-355) on a CenterlineProgress (track_progress.py): one
     independent reward object per env, evaluated by ``f110_reward_compute`` straight from the observation tensor.
-    One centerline for all envs: under a map set (F110VecEnv(maps=...)) it is the centerline of one of the maps only.
 
     ``centerline``: [n, 2] (x_m, y_m) or [n, 4] (+ w_tr_right_m, w_tr_left_m), the CSV train_ddpg.py loads.  Keyword
     arguments are the reference constructor's.  ``__call__(obs, reset_mask=None)`` returns a float64 CUDA tensor [N];
     ``reset_mask`` plays the role of ``reward_fn.reset()`` per env.
+
+    ``centerlines=[cl_0, ..., cl_{K-1}]`` instead of ``centerline`` (1 <= K <= 256, each [n, 2] or [n, 4] with
+    2 <= n <= 16385) holds one centerline per map of a map set, in slot order; ``closed`` is then one flag for all or a
+    list of K.  ``__call__`` then needs ``slots`` (CUDA int32 [N], e.g. BatchSim.env_maps()): env e is scored exactly as a
+    reward on ``centerlines[slots[e]]`` alone would score it.  A changed slot restarts that env's record, as its reset mask
+    does; a slot outside [0, K) gives NaN and leaves the env's record alone.  Parameters are shared by the whole set.
     """
 
-    def __init__(self, num_envs, centerline, num_beams=1080, closed=True, device=None, **kw):
+    def __init__(self, num_envs, centerline=None, num_beams=1080, closed=True, device=None, centerlines=None, **kw):
         unknown = set(kw) - set(REWARD_DEFAULTS)
         if unknown:
             raise TypeError("unknown reward arguments: %s" % sorted(unknown))
+        if (centerline is None) == (centerlines is None):
+            raise ValueError("give either centerline= or centerlines=, not both and not neither")
+        lines = _check_centerlines(centerlines, closed) if centerlines is not None else None
         p = dict(REWARD_DEFAULTS)
         p.update(kw)
         self.lib = _lib.load()
         self.device = torch.device('cuda', torch.cuda.current_device() if device is None else device)
-        cl = np.ascontiguousarray(centerline, np.float64)
-        xy = np.ascontiguousarray(cl[:, :2])
-        wR = np.ascontiguousarray(cl[:, 2]) if cl.shape[1] >= 4 else None
-        wL = np.ascontiguousarray(cl[:, 3]) if cl.shape[1] >= 4 else None
-        cfg = _lib.F110RewardConfig(num_envs=num_envs, num_points=len(xy), num_beams=num_beams, device=self.device.index,
-                                    closed=int(closed), grace_steps_wall=int(p['grace_steps_wall']),
-                                    grace_steps_opp=int(p['grace_steps_opp']),
+        cfg = _lib.F110RewardConfig(num_envs=num_envs, num_beams=num_beams, device=self.device.index,
+                                    grace_steps_wall=int(p['grace_steps_wall']), grace_steps_opp=int(p['grace_steps_opp']),
                                     **{k: float(v) for k, v in p.items() if not k.startswith('grace_')})
         h = C.c_void_p()
-        _lib.check(self.lib.f110_reward_create(C.byref(cfg), xy.ctypes.data_as(C.c_void_p),
-                                               None if wR is None else wR.ctypes.data_as(C.c_void_p),
-                                               None if wL is None else wL.ctypes.data_as(C.c_void_p), C.byref(h)))
+        if lines is None:
+            cl = np.ascontiguousarray(centerline, np.float64)
+            xy = np.ascontiguousarray(cl[:, :2])
+            wR = np.ascontiguousarray(cl[:, 2]) if cl.shape[1] >= 4 else None
+            wL = np.ascontiguousarray(cl[:, 3]) if cl.shape[1] >= 4 else None
+            cfg.num_points, cfg.closed = len(xy), int(closed)
+            _lib.check(self.lib.f110_reward_create(C.byref(cfg), xy.ctypes.data_as(C.c_void_p),
+                                                   None if wR is None else wR.ctypes.data_as(C.c_void_p),
+                                                   None if wL is None else wL.ctypes.data_as(C.c_void_p), C.byref(h)))
+            self.num_centerlines = 1
+        else:
+            descs = (_lib.F110Centerline * len(lines))()
+            for d, (xy, wR, wL, c) in zip(descs, lines):
+                d.xy = xy.ctypes.data
+                d.wR = None if wR is None else wR.ctypes.data
+                d.wL = None if wL is None else wL.ctypes.data
+                d.num_points, d.closed = len(xy), int(c)
+            _lib.check(self.lib.f110_reward_create_set(C.byref(cfg), descs, len(lines), C.byref(h)))
+            self.num_centerlines = len(lines)
         self.h = h
         self.N, self.B = num_envs, num_beams
         self.out = torch.zeros(num_envs, dtype=torch.float64, device=self.device)
 
-    def __call__(self, obs, reset_mask=None):
+    def __call__(self, obs, reset_mask=None, slots=None):
         if not (obs.is_cuda and obs.dtype == torch.float32 and obs.is_contiguous() and obs.numel() == self.N * (self.B + 8)):
             raise ValueError("obs must be a contiguous CUDA float32 tensor [N, B+8]")
-        rm = None
+        if slots is None and self.num_centerlines > 1:
+            raise ValueError("a reward with %d centerlines needs each env's slot (slots=)" % self.num_centerlines)
+        rm = sl = None
         if reset_mask is not None:
             rm = reset_mask.to(device=self.device, dtype=torch.uint8).contiguous()
             self._keep = rm
+        if slots is not None:
+            if not (torch.is_tensor(slots) and slots.is_cuda and slots.dtype == torch.int32 and slots.is_contiguous()
+                    and slots.numel() == self.N):
+                raise ValueError("slots must be a contiguous CUDA int32 tensor [N]")
+            sl = slots
         stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
-        _lib.check(self.lib.f110_reward_compute(self.h, C.c_void_p(obs.data_ptr()), None if rm is None else C.c_void_p(rm.data_ptr()),
-                                                C.c_void_p(self.out.data_ptr()), None, stream))
+        ptr = lambda t: None if t is None else C.c_void_p(t.data_ptr())
+        _lib.check(self.lib.f110_reward_compute_slots(self.h, ptr(obs), ptr(rm), ptr(sl), ptr(self.out), None, stream))
         return self.out
 
     def close(self):
@@ -293,3 +330,28 @@ class ShapedReward(object):
             self.close()
         except Exception:
             pass
+
+
+def _check_centerlines(centerlines, closed):
+    """-> [(xy [n, 2], wR [n] or None, wL [n] or None, closed)] per line, or ValueError naming the first bad line; no
+    library call, so the checks hold without a device."""
+    lines = list(centerlines)
+    if not 1 <= len(lines) <= _lib.F110_MAX_MAPS:
+        raise ValueError("centerlines: %d given; 1 to %d allowed" % (len(lines), _lib.F110_MAX_MAPS))
+    if isinstance(closed, (list, tuple, np.ndarray)):
+        flags = [bool(c) for c in closed]
+        if len(flags) != len(lines):
+            raise ValueError("closed: %d flags for %d centerlines" % (len(flags), len(lines)))
+    else:
+        flags = [bool(closed)] * len(lines)
+    out = []
+    for k, (cl, c) in enumerate(zip(lines, flags)):
+        cl = np.asarray(cl, np.float64)
+        if cl.ndim != 2 or cl.shape[1] not in (2, 4):
+            raise ValueError("centerline %d: shape %s; [n, 2] (x, y) or [n, 4] (+ w_right, w_left) expected" % (k, cl.shape))
+        if not 2 <= len(cl) <= 16385:
+            raise ValueError("centerline %d has %d points; 2 to 16385 allowed" % (k, len(cl)))
+        wide = cl.shape[1] == 4
+        out.append((np.ascontiguousarray(cl[:, :2]), np.ascontiguousarray(cl[:, 2]) if wide else None,
+                    np.ascontiguousarray(cl[:, 3]) if wide else None, c))
+    return out

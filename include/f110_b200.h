@@ -163,7 +163,8 @@ int f110_get_map(F110Sim* sim, double* dt_host, int64_t capacity_cells);
  * alone (see f110_set_map), and lie back to back in one allocation: each member costs as much device memory as the largest
  * would.  A set that contains one 8000 x 8000 map pads every member to 8208 x 8192 cells = 538 MB.  The set's padded cells
  * in all must stay below 2^31 (31 maps when the largest is 8000^2, 127 at 4000^2, 508 at 2000^2).
- * The shaped reward (f110_reward_*) keeps one centerline per reward object: it does not know about slots. */
+ * The shaped reward follows the slots through a set of centerlines, one per map (f110_reward_create_set,
+ * f110_reward_compute_slots with the slots f110_get_env_maps returns). */
 #define F110_MAX_MAPS 256
 typedef struct F110MapDesc {
     const double*  dt;         /* HOST [height][width] fp64 as f110_set_map takes it, or NULL */
@@ -293,6 +294,26 @@ void f110_reward_destroy(F110Reward* r);
 /* obs: DEVICE float [num_envs][num_beams + 8] (F110StepIO.obs); reset_mask: DEVICE [num_envs] or NULL, non-zero =
  * reward_fn.reset() before this call; out_f64 / out_f32: DEVICE [num_envs], either may be NULL. */
 int f110_reward_compute(F110Reward* r, const float* obs, const uint8_t* reset_mask, double* out_f64, float* out_f32, void* stream);
+/* A set of centerlines in one reward object, one per map of a map set (DESIGN.md section 10): env e is scored on line
+ * slots[e], exactly as a reward object created from that line alone would score it, bit for bit.  Each line has its own
+ * points (2 to 16385), widths and closed flag; cfg->num_points and cfg->closed are ignored.  1 <= count <= F110_MAX_MAPS;
+ * every line is checked before anything is allocated, and an error names the failing line.  f110_reward_create is the set
+ * of one line.  f110_reward_compute on a set of more than one line returns F110_ERR_INVALID. */
+typedef struct F110Centerline {
+    const double* xy;           /* HOST [num_points][2] */
+    const double* wR;           /* HOST [num_points] or NULL; the widths are used when both wR and wL are given */
+    const double* wL;
+    int32_t num_points, closed;
+} F110Centerline;
+int f110_reward_create_set(const F110RewardConfig* cfg, const F110Centerline* lines, int32_t count, F110Reward** out);
+/* Number of centerlines (1 for f110_reward_create). */
+int32_t f110_reward_count(const F110Reward* r);
+/* f110_reward_compute with each env's slot.  slots: DEVICE int32 [num_envs], may be NULL only when the set holds one line
+ * (it is then not read and the single-line kernels run).  The set keeps each env's slot of its previous call (-1 at
+ * creation): an env whose slot differs is treated as if its reset_mask were set.  An env whose slot lies outside
+ * [0, count) gets NaN in both outputs, and its record and stored slot stay as they were. */
+int f110_reward_compute_slots(F110Reward* r, const float* obs, const uint8_t* reset_mask, const int32_t* slots,
+                              double* out_f64, float* out_f32, void* stream);
 
 /* ---- measurement utility: the empirical dependent-gather roofline (SURVEY 8d) ----
  * num_threads threads each chase `chain` dependent 8-byte loads through a power-of-two window of `window_cells`
