@@ -2,13 +2,12 @@
 // training loop (SURVEY 8f), so a rollout never leaves the GPU.  Paths are relative to /root/reference/.
 //
 //   gap_follow_kernel : rl_training/utils/gap_follow.py:3-58, the rule-based opponent train_ddpg.py:168 drives
-//                       from info["scans"][1].  One CTA per scan; float32 arithmetic in numpy's order, so the
+//                       from info["scans"][1].  One warp per scan; float32 arithmetic in numpy's order, so the
 //                       chosen beam index -- and with it (steer, speed) -- is identical to the reference's.
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdint.h>
 #include <stdio.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include <vector>
@@ -248,11 +247,11 @@ extern "C" int f110_gap_follow(const float* scans, int64_t num_scans, int64_t sc
 }
 
 // =====================================================================================================================
-//   shaped_reward_kernel : rl_training/utils/rewards.py:185-355 (CenterlineSafetyProgressReward, with _Prog :86-180 and
-//                          parse_flat_obs :11-39) over rl_training/utils/track_progress.py (CenterlineProgress.project_xy
+//   shaped_reward_warp_kernel : rl_training/utils/rewards.py:185-355 (CenterlineSafetyProgressReward, with _Prog :86-180
+//                          and parse_flat_obs :11-39) over rl_training/utils/track_progress.py (CenterlineProgress.project_xy
 //                          :58-95, delta_s :97-104) -- the reward train_ddpg.py:179 computes from the flat observation.
-//                          One CTA per env: brute-force 5-nearest segment midpoints for both cars (the reference's
-//                          cKDTree.query(k=5)), radix select for numpy's float32 quantile of the lidar, then one thread runs
+//                          One warp per env: exact 5-nearest segment midpoints for both cars (the reference's
+//                          cKDTree.query(k=5)), radix select for numpy's float32 quantile of the lidar, then lane 0 runs
 //                          the per-env progress state machine.  fp64 in the reference's order; results agree to ~1e-15.
 // =====================================================================================================================
 struct F110Reward {
@@ -287,8 +286,8 @@ struct RewardView {
 };
 
 // A set of K centerlines: the lines lie back to back in one allocation per array, line k's points from `off` on (xy, s,
-// wR, wL; tan, nrm, mid likewise, one entry short), its bounding circles from block `boff` on.  The set kernels read the
-// env's slot, then the slot's record, and point a RewardView at that line; from there on they are the single-line kernels.
+// wR, wL; tan, nrm, mid likewise, one entry short), its bounding circles from block `boff` on.  The set kernel reads the
+// env's slot, then the slot's record, and points a RewardView at that line; from there on it is the single-line kernel.
 struct RewardLine {
     int off, n, nblk, boff;
     double L;
@@ -302,7 +301,7 @@ struct RewardSetView {
     int count;
 };
 
-constexpr int RW_THREADS = 128;
+constexpr int RW_MAX_BEAMS = 8192;   // the longest scan a reward object accepts
 constexpr int KNN = 5;
 constexpr int MID_BLOCK = 64;   // midpoints per pruning block
 
@@ -321,45 +320,6 @@ __device__ __forceinline__ void topk_insert(Cand (&best)[KNN], double d2, int id
     for (int j = KNN - 1; j > 0; --j) {
         if (cand_less(best[j], best[j - 1])) { const Cand t = best[j]; best[j] = best[j - 1]; best[j - 1] = t; }
     }
-}
-
-// The KNN smallest (d2, idx) over the whole CTA.  Each warp pops its KNN best with shuffles (no barrier), the four
-// warps' lists meet in shared memory, thread 0 merges them.  `best` is this thread's sorted private list.
-__device__ void block_topk(const Cand (&best)[KNN], Cand* s_cand /*[4][KNN]*/, int* s_out /*[KNN]*/) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    int head = 0;
-    for (int round = 0; round < KNN; ++round) {
-        Cand c;
-        c.d2 = INFINITY; c.idx = 0x7fffffff;
-#pragma unroll
-        for (int k = 0; k < KNN; ++k) if (k == head) c = best[k];
-        // warp-wide lexicographic min of (d2, idx) with three REDUX: d2 >= 0, so its bit pattern orders like the value
-        const unsigned long long bits = (unsigned long long)__double_as_longlong(c.d2);
-        const unsigned hi = (unsigned)(bits >> 32), lo = (unsigned)bits;
-        const unsigned mhi = __reduce_min_sync(0xffffffffu, hi);
-        const unsigned mlo = __reduce_min_sync(0xffffffffu, hi == mhi ? lo : 0xFFFFFFFFu);
-        const unsigned midx = __reduce_min_sync(0xffffffffu, (hi == mhi && lo == mlo) ? (unsigned)c.idx : 0x7FFFFFFFu);
-        Cand w;
-        w.d2 = __longlong_as_double((long long)(((unsigned long long)mhi << 32) | mlo));
-        w.idx = (int)midx;
-        if (w.idx == c.idx && c.idx != 0x7fffffff) ++head;      // a midpoint index belongs to exactly one thread
-        if (lane == 0) s_cand[warp * KNN + round] = w;
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        int h[RW_THREADS / 32] = { 0, 0, 0, 0 };
-        for (int round = 0; round < KNN; ++round) {
-            int bw = -1;
-            Cand bc;
-            bc.d2 = INFINITY; bc.idx = 0x7fffffff;
-            for (int w = 0; w < RW_THREADS / 32; ++w) {
-                if (h[w] < KNN && cand_less(s_cand[w * KNN + h[w]], bc)) { bc = s_cand[w * KNN + h[w]]; bw = w; }
-            }
-            if (bw >= 0) ++h[bw];
-            s_out[round] = bc.idx == 0x7fffffff ? -1 : bc.idx;
-        }
-    }
-    __syncthreads();
 }
 
 // np.searchsorted(P.s, s, side="right") - 1 clamped to [0, n-2] (rewards.py:108-110, :272-274).  s is non-decreasing and the
@@ -437,32 +397,19 @@ __device__ __forceinline__ void write_nan(double* out64, float* out32, int env) 
     if (out32) out32[env] = __int_as_float(0x7fc00000);
 }
 
-__global__ void __launch_bounds__(RW_THREADS) shaped_reward_kernel(RewardView v, const float* __restrict__ obs,
-                                                                   const uint8_t* __restrict__ reset_mask,
-                                                                   double* __restrict__ out64, float* __restrict__ out32) {
-#define F110_REWARD_SET 0
-#include "f110_reward_cta_body.cuh"
-#undef F110_REWARD_SET
-}
-
-// the CTA-per-env kernel on a set of centerlines: each env on the line of its slot
-__global__ void __launch_bounds__(RW_THREADS) shaped_reward_set_kernel(RewardView base, RewardSetView rs, const float* __restrict__ obs,
-                                                                       const uint8_t* __restrict__ reset_mask,
-                                                                       double* __restrict__ out64, float* __restrict__ out32) {
-#define F110_REWARD_SET 1
-#include "f110_reward_cta_body.cuh"
-#undef F110_REWARD_SET
-}
-
-
-// The same reward with ONE WARP per env (round 2; the CTA-per-env kernel above stays as the form for scans too long for a
-// warp's share of shared memory).  Nothing about the arithmetic changes: the one-thread sections (observation parsing,
-// projections, the progress state machine) are the same statements run by lane 0 (lanes 0 and 1 for the two projections),
-// the 5-nearest search and the quantile's radix select produce the same discrete answers with warp-wide instead of
-// CTA-wide steps -- and no barrier: a third of the CTA kernel's stall samples were barriers around one-thread sections.
+// ONE WARP per env: the one-thread sections (observation parsing, projections, the progress state machine) are lane 0's
+// (lanes 0 and 1 for the two projections), the 5-nearest search and the quantile's radix select take warp-wide steps, and
+// nothing waits at a barrier -- with a CTA per env (round 1), a third of the stall samples were barriers around the
+// one-thread sections.
 constexpr int RWW_MAX = 4;      // envs per CTA
 
-__device__ __forceinline__ size_t reward_warp_smem_bytes(int B) { return sizeof(unsigned) * ((size_t)B + 256) + sizeof(double) * 256 + sizeof(int) * (256 + 2 * KNN + 2); }
+// a warp's share of shared memory: the scan as sortable words, a histogram, the block bounds and the candidates, rounded
+// to 16 bytes so that the next warp's doubles stay aligned
+__host__ __device__ constexpr size_t reward_warp_smem_bytes(int B) {
+    return (sizeof(unsigned) * ((size_t)B + 256) + sizeof(double) * 256 + sizeof(int) * (256 + 2 * KNN + 2) + 15) & ~size_t(15);
+}
+// so every scan check_lines accepts runs with a warp per env in the 48 KB that need no opt-in
+static_assert(reward_warp_smem_bytes(RW_MAX_BEAMS) <= 48 * 1024, "a warp's reward scratch must fit 48 KB at the longest scan");
 
 __global__ void __launch_bounds__(RWW_MAX * 32) shaped_reward_warp_kernel(RewardView v, const float* __restrict__ obs,
                                                                           const uint8_t* __restrict__ reset_mask,
@@ -488,8 +435,8 @@ namespace {
 // Checks every line against the limits before anything is allocated; the message names the failing line and its limit.
 int check_lines(const char* who, const F110RewardConfig* cfg, const F110Centerline* lines, int32_t count, F110Reward** out) {
     char msg[256];
-    if (!cfg || !lines || !out || cfg->num_envs < 1 || cfg->num_beams < 1 || cfg->num_beams > 8192) {
-        snprintf(msg, sizeof(msg), "%s: need non-null arguments, num_envs >= 1, 1 <= num_beams <= 8192", who);
+    if (!cfg || !lines || !out || cfg->num_envs < 1 || cfg->num_beams < 1 || cfg->num_beams > RW_MAX_BEAMS) {
+        snprintf(msg, sizeof(msg), "%s: need non-null arguments, num_envs >= 1, 1 <= num_beams <= %d", who, RW_MAX_BEAMS);
         return f110_set_error(F110_ERR_INVALID, msg);
     }
     if (count < 1 || count > F110_MAX_MAPS) {
@@ -640,22 +587,13 @@ extern "C" int f110_reward_compute_slots(F110Reward* r, const float* obs, const 
     RewardSetView rs;
     rs.lines = static_cast<const RewardLine*>(r->lines); rs.slots = slots; rs.prev = r->prev_slot; rs.count = r->count;
     const bool set = r->count > 1;       // a set of one runs the single-line kernels and reads no slot
-    // a warp per env where a warp's scratch (the scan as sortable words, a histogram, the block bounds) fits the 48 KB of
-    // shared memory that need no opt-in; else (scans of more than ~11 000 beams) the CTA-per-env form
-    const int B = r->cfg.num_beams;
-    const size_t per_warp = ((sizeof(unsigned) * ((size_t)B + 256) + sizeof(double) * 256 + sizeof(int) * (256 + 2 * KNN + 2)) + 15) & ~size_t(15);
-    const char* force_cta = getenv("F110_REWARD_CTA");      // test switch: the round-1 kernel
-    if (per_warp <= 48 * 1024 && !(force_cta && force_cta[0] == '1')) {
-        int warps = (int)((48 * 1024) / per_warp);
-        warps = warps > RWW_MAX ? RWW_MAX : warps;
-        const dim3 grid((r->cfg.num_envs + warps - 1) / warps), block(warps * 32);
-        if (set) shaped_reward_set_warp_kernel<<<grid, block, per_warp * warps, (cudaStream_t)stream>>>(v, rs, obs, reset_mask, out_f64, out_f32);
-        else shaped_reward_warp_kernel<<<grid, block, per_warp * warps, (cudaStream_t)stream>>>(v, obs, reset_mask, out_f64, out_f32);
-    } else {
-        const size_t smem = sizeof(unsigned) * r->cfg.num_beams;
-        if (set) shaped_reward_set_kernel<<<r->cfg.num_envs, RW_THREADS, smem, (cudaStream_t)stream>>>(v, rs, obs, reset_mask, out_f64, out_f32);
-        else shaped_reward_kernel<<<r->cfg.num_envs, RW_THREADS, smem, (cudaStream_t)stream>>>(v, obs, reset_mask, out_f64, out_f32);
-    }
+    // as many warps per CTA as the 48 KB of shared memory that need no opt-in hold, at least one (the static_assert above)
+    const size_t per_warp = reward_warp_smem_bytes(r->cfg.num_beams);
+    int warps = (int)((48 * 1024) / per_warp);
+    warps = warps > RWW_MAX ? RWW_MAX : warps;
+    const dim3 grid((r->cfg.num_envs + warps - 1) / warps), block(warps * 32);
+    if (set) shaped_reward_set_warp_kernel<<<grid, block, per_warp * warps, (cudaStream_t)stream>>>(v, rs, obs, reset_mask, out_f64, out_f32);
+    else shaped_reward_warp_kernel<<<grid, block, per_warp * warps, (cudaStream_t)stream>>>(v, obs, reset_mask, out_f64, out_f32);
     return cudaPeekAtLastError() == cudaSuccess ? F110_OK : F110_ERR_CUDA;
 }
 

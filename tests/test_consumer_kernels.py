@@ -4,11 +4,11 @@ gap_follow_kernel: over the parameter grid of test_consumer_model.py (every wind
 count up to 8192 with the shared-memory opt-in, the speed band boundaries, non-finite beams), through strided [N, 3, n]
 views, agent 0 and agent 2, with the other slots asserted untouched.
 
-shaped_reward_warp_kernel and shaped_reward_kernel: the reward is built with -fmad=false, and every operation in it is
+shaped_reward_warp_kernel: the reward is built with -fmad=false, and every operation in it is
 IEEE-exact except hypot (the opponent bubble) and sincos (the flank).  The expected value is the oracle's breakdown with
 those two terms recomputed in numpy from the device's own hypot and sincos (f110_hypot_probe, f110_trig_probe), summed
-in the kernel's order: it must equal out_f64 exactly, and out_f32 must equal its float32 rounding.  Both kernel forms run
-every case of reward_cases() (the CTA-per-env form through the F110_REWARD_CTA switch).
+in the kernel's order: it must equal out_f64 exactly, and out_f32 must equal its float32 rounding, on every case of
+reward_cases().
 """
 import ctypes as C
 
@@ -134,49 +134,47 @@ def _same(a, b):
     return np.array_equal(a, b, equal_nan=True)
 
 
-@pytest.mark.parametrize('form', ['warp', 'cta'])
-def test_shaped_reward_kernels_equal_oracle(form, monkeypatch):
-    monkeypatch.setenv('F110_REWARD_CTA', '1' if form == 'cta' else '0')
+@pytest.mark.parametrize('c', reward_cases(), ids=lambda c: c.name)
+def test_shaped_reward_kernels_equal_oracle(c):
     torch = _torch()
     from f110_gymnasium_ros2_jazzy_b200 import ShapedReward, _lib
     from oracle.f110_oracle import RewardOracle
     dm = DeviceMath()
     L = _lib.load()
+    Tn, N, _ = c.obs.shape
+    rw = ShapedReward(N, c.centerline, num_beams=c.num_beams, closed=c.closed, **c.kw)
+    orc = RewardOracle(N, c.centerline, num_beams=c.num_beams, closed=c.closed, **c.kw)
+    o64 = torch.full((N,), -123.0, dtype=torch.float64, device='cuda')
+    o32 = torch.full((N,), -123.0, dtype=torch.float32, device='cuda')
+    breakdown = []
     libm_differs = 0
-    for c in reward_cases():
-        Tn, N, _ = c.obs.shape
-        rw = ShapedReward(N, c.centerline, num_beams=c.num_beams, closed=c.closed, **c.kw)
-        orc = RewardOracle(N, c.centerline, num_beams=c.num_beams, closed=c.closed, **c.kw)
-        o64 = torch.full((N,), -123.0, dtype=torch.float64, device='cuda')
-        o32 = torch.full((N,), -123.0, dtype=torch.float32, device='cuda')
-        breakdown = []
-        for t in range(Tn):
-            ob = torch.from_numpy(c.obs[t]).cuda()
-            mask = None if c.masks is None else torch.from_numpy(c.masks[t]).cuda()
-            mode = t % 3                                  # f64 and f32, f64 only, f32 only
-            p64 = C.c_void_p(o64.data_ptr()) if mode in (0, 1) else None
-            p32 = C.c_void_p(o32.data_ptr()) if mode in (0, 2) else None
-            o64.fill_(-123.0); o32.fill_(-123.0)
-            _lib.check(L.f110_reward_compute(rw.h, C.c_void_p(ob.data_ptr()), None if mask is None else C.c_void_p(mask.data_ptr()),
-                                             p64, p32, None))
-            torch.cuda.synchronize()
-            tot, terms = orc.compute_terms(c.obs[t], None if c.masks is None else c.masks[t])
-            breakdown.append(terms)
-            want, nd = expected_reward(dm, c.obs[t], tot, terms, c.num_beams, c.kw)
-            libm_differs += nd
-            g64, g32 = o64.cpu().numpy(), o32.cpu().numpy()
-            if mode in (0, 1):
-                bad = np.nonzero(~((g64 == want) | (np.isnan(g64) & np.isnan(want))))[0]
-                assert len(bad) == 0, (c.name, form, t, bad[:5], g64[bad[:5]], want[bad[:5]])
-            else:
-                assert (g64 == -123.0).all()
-            if mode in (0, 2):
-                assert _same(g32, want.astype(np.float32)), (c.name, form, t)
-            else:
-                assert (g32 == -123.0).all()
-        rw.close()
-        check_branches(c, np.stack(breakdown))          # the case reached what it was built for
-    print('reward terms where the device hypot / sincos differ from glibc:', libm_differs)
+    for t in range(Tn):
+        ob = torch.from_numpy(c.obs[t]).cuda()
+        mask = None if c.masks is None else torch.from_numpy(c.masks[t]).cuda()
+        mode = t % 3                                  # f64 and f32, f64 only, f32 only
+        p64 = C.c_void_p(o64.data_ptr()) if mode in (0, 1) else None
+        p32 = C.c_void_p(o32.data_ptr()) if mode in (0, 2) else None
+        o64.fill_(-123.0); o32.fill_(-123.0)
+        _lib.check(L.f110_reward_compute(rw.h, C.c_void_p(ob.data_ptr()), None if mask is None else C.c_void_p(mask.data_ptr()),
+                                         p64, p32, None))
+        torch.cuda.synchronize()
+        tot, terms = orc.compute_terms(c.obs[t], None if c.masks is None else c.masks[t])
+        breakdown.append(terms)
+        want, nd = expected_reward(dm, c.obs[t], tot, terms, c.num_beams, c.kw)
+        libm_differs += nd
+        g64, g32 = o64.cpu().numpy(), o32.cpu().numpy()
+        if mode in (0, 1):
+            bad = np.nonzero(~((g64 == want) | (np.isnan(g64) & np.isnan(want))))[0]
+            assert len(bad) == 0, (c.name, t, bad[:5], g64[bad[:5]], want[bad[:5]])
+        else:
+            assert (g64 == -123.0).all()
+        if mode in (0, 2):
+            assert _same(g32, want.astype(np.float32)), (c.name, t)
+        else:
+            assert (g32 == -123.0).all()
+    rw.close()
+    check_branches(c, np.stack(breakdown))          # the case reached what it was built for
+    print(c.name, 'reward terms where the device hypot / sincos differ from glibc:', libm_differs)
 
 
 def test_reward_centerline_point_limit():

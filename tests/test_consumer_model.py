@@ -11,7 +11,7 @@ NaN-blind argmin part from the reference.
 Reward: the float32 wall quantile against np.quantile, the lateral segment lookup against np.searchsorted, the 5 nearest
 midpoints against scipy's cKDTree.  reward_cases() builds seeded centerlines and episodes, each aimed at a branch of the
 reward; test_reward_cases_reach_their_branches checks on the oracle's per-env breakdown that each one gets there.  The GPU
-tests (test_consumer_kernels.py) hold both reward kernels to the oracle on the same cases.
+tests (test_consumer_kernels.py) hold the reward kernel to the oracle on the same cases.
 """
 import numpy as np
 import pytest

@@ -1086,13 +1086,12 @@ def test_c4_full_size_sharded_properties():
     sim.close()
 
 
-@pytest.mark.parametrize('form', ['warp', 'cta'])
-def test_shaped_reward_kernel_matches_reference_and_oracle(form, monkeypatch):
+@pytest.mark.parametrize('key', ['reward', 'reward_alt'])
+def test_shaped_reward_kernel_matches_reference_and_oracle(key):
     """f110_reward_compute: (a) the recorded reference episodes, each replayed in its own env slot of one batch, within
     1e-9 of the reference (numpy, BLAS and glibc there), (b) the oracle on the same batch of independent envs, exactly,
-    once its opponent and flank terms are recomputed with the device's hypot and sincos.  Both forms of the kernel: a warp
-    per env (the default) and a CTA per env (scans too long for a warp's shared memory; forced)."""
-    monkeypatch.setenv('F110_REWARD_CTA', '1' if form == 'cta' else '0')
+    once its opponent and flank terms are recomputed with the device's hypot and sincos.  `key` names the recording and
+    its reward parameters: the defaults of the reference's training run, or the alternative set."""
     torch = _torch()
     from f110_gymnasium_ros2_jazzy_b200 import ShapedReward
     from oracle.f110_oracle import RewardOracle
@@ -1102,20 +1101,20 @@ def test_shaped_reward_kernel_matches_reference_and_oracle(form, monkeypatch):
     g = H.reward_recording()
     obs, starts = g['obs'], g['episode_start']
     T = len(obs)
-    for kw, key in ((REWARD_KW, 'reward'), (REWARD_ALT_KW, 'reward_alt')):
-        # env slot 0 replays the recording; slots 1..3 replay it shifted in time (independent state per env)
-        N = 4
-        rw = ShapedReward(N, g['centerline'], **kw)
-        orc = RewardOracle(N, g['centerline'], **kw)
-        for t in range(T):
-            batch = np.stack([obs[(t + 37 * k) % T] for k in range(N)])
-            mask = np.array([starts[(t + 37 * k) % T] or t == 0 for k in range(N)], np.uint8)
-            got = rw(torch.from_numpy(batch).cuda(), torch.from_numpy(mask).cuda()).cpu().numpy()
-            tot, terms = orc.compute_terms(batch, mask)
-            want, _ = expected_reward(dm, batch, tot, terms, 1080, kw)
-            assert np.array_equal(got, want), (key, t, got, want)
-            assert abs(got[0] - g[key][t]) < 1e-9, (key, t, got[0], g[key][t])
-        rw.close()
+    kw = {'reward': REWARD_KW, 'reward_alt': REWARD_ALT_KW}[key]
+    # env slot 0 replays the recording; slots 1..3 replay it shifted in time (independent state per env)
+    N = 4
+    rw = ShapedReward(N, g['centerline'], **kw)
+    orc = RewardOracle(N, g['centerline'], **kw)
+    for t in range(T):
+        batch = np.stack([obs[(t + 37 * k) % T] for k in range(N)])
+        mask = np.array([starts[(t + 37 * k) % T] or t == 0 for k in range(N)], np.uint8)
+        got = rw(torch.from_numpy(batch).cuda(), torch.from_numpy(mask).cuda()).cpu().numpy()
+        tot, terms = orc.compute_terms(batch, mask)
+        want, _ = expected_reward(dm, batch, tot, terms, 1080, kw)
+        assert np.array_equal(got, want), (key, t, got, want)
+        assert abs(got[0] - g[key][t]) < 1e-9, (key, t, got[0], g[key][t])
+    rw.close()
 
 
 def test_device_edt_bit_identical_to_scipy():

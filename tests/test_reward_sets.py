@@ -4,10 +4,11 @@ DeviceRollout on a map set; DESIGN.md section 10).
 The expected value throughout: K single-centerline references, each run over all N envs, env e read from reference
 slots[e], each reference given reset_mask | slot changed.  The references are the oracle (with the device's hypot and
 sincos, as test_consumer_kernels.py holds the single-line kernels to it) or single-line ShapedReward objects, which that
-file holds to the oracle bit for bit.  GPU tests run both kernel forms (the CTA-per-env one through F110_REWARD_CTA).
+file holds to the oracle bit for bit.  The GPU tests run at a short scan, where four envs share a CTA, and at the
+longest, 8192 beams, where a warp's scratch leaves room for only one env per CTA.
 
 CPU: the argument checks of ShapedReward(centerlines=...) and of f110_reward_create_set (both refuse before any device
-call), and a static guard on the set kernels' stack frames in the built library.
+call), and a static guard on the reward kernels' stack frames in the built library.
 """
 import ctypes as C
 import re
@@ -77,9 +78,9 @@ def test_create_set_validates_every_line_before_allocating():
     assert 'centerline 1 has no points' in L.f110_last_error().decode()
 
 
-def test_set_kernels_stack_frames():
-    """Both set kernels exist, and their local memory is at most 16 bytes above the single-line kernels' stack frames
-    (80 bytes warp form, 64 bytes CTA form): the line's view (pointers, L, closed) does not go to local memory."""
+def test_reward_kernels_stack_frames():
+    """Exactly the two reward kernels exist, and the set kernel's local memory is at most 16 bytes above the single-line
+    kernel's 80-byte stack frame: the line's view (pointers, L, closed) does not go to local memory."""
     from tests.test_kernel_shape import CUOBJDUMP, _functions
     if not CUOBJDUMP:
         pytest.skip("cuobjdump neither on PATH nor under CUDA_HOME")
@@ -89,11 +90,9 @@ def test_set_kernels_stack_frames():
         m = re.search(r"(shaped_reward_(?:set_)?(?:warp_)?kernel)", name)
         if m:
             local[m.group(1)] = int(re.search(r"LOCAL:(\d+)", " ".join(lines)).group(1))
-    assert set(local) == {'shaped_reward_kernel', 'shaped_reward_warp_kernel', 'shaped_reward_set_kernel',
-                          'shaped_reward_set_warp_kernel'}, local
-    assert local['shaped_reward_warp_kernel'] <= 80 and local['shaped_reward_kernel'] <= 64, local
+    assert set(local) == {'shaped_reward_warp_kernel', 'shaped_reward_set_warp_kernel'}, local
+    assert local['shaped_reward_warp_kernel'] <= 80, local
     assert local['shaped_reward_set_warp_kernel'] <= 80 + 16, local
-    assert local['shaped_reward_set_kernel'] <= 64 + 16, local
 
 
 # ----------------------------------------------------------------------------------------------------- GPU
@@ -191,36 +190,35 @@ def _check_step(g64, g32, want, where):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize('form', ['warp', 'cta'])
-def test_set_equals_oracle(form, monkeypatch):
-    """Six lines, 1080 beams, envs in blocks and interleaved, reset masks from the episodes: out_f64 equals the oracle of
-    each env's line bit for bit, out_f32 is its rounding.  Then the longest scan, 8192 beams (the CTA form's case)."""
-    monkeypatch.setenv('F110_REWARD_CTA', '1' if form == 'cta' else '0')
+@pytest.mark.parametrize('B', [1080, 8192])
+def test_set_equals_oracle(B):
+    """Envs in blocks and interleaved, reset masks from the episodes: out_f64 equals the oracle of each env's line bit
+    for bit, out_f32 is its rounding.  1080 beams on six lines; the longest scan, 8192 beams (one warp per CTA), on two."""
     _torch()
     from oracle.f110_oracle import RewardOracle
     from tests.test_consumer_kernels import DeviceMath, expected_reward
     dm = DeviceMath()
     rng = np.random.default_rng(31)
     lines = _lines()
-    for B, per_line, T, sub in ((1080, 5, 30, lines), (8192, 2, 6, [lines[0], lines[3]])):
-        K = len(sub)
-        for slots in (np.repeat(np.arange(K), per_line), np.arange(K * per_line) % K):       # blocks, interleaved
-            N = len(slots)
-            slots_t = np.broadcast_to(slots, (T, N)).copy()
-            obs, masks = _assemble(rng, sub, slots_t, T, B)
-            run = SetRun(N, sub, B, **KW)
-            orcs = [RewardOracle(N, cl, num_beams=B, closed=c, **KW) for cl, c in sub]
-            chg = _changed(slots_t)
-            for t in range(T):
-                g64, g32 = run(obs[t], masks[t], slots_t[t])
-                m = (masks[t] != 0) | chg[t]
-                want = np.zeros(N)
-                for k, o in enumerate(orcs):
-                    tot, terms = o.compute_terms(obs[t], m.astype(np.uint8))
-                    wk, _ = expected_reward(dm, obs[t], tot, terms, B, KW)
-                    want[slots == k] = wk[slots == k]
-                _check_step(g64, g32, want, (form, B, t))
-            run.rw.close()
+    per_line, T, sub = (5, 30, lines) if B == 1080 else (2, 6, [lines[0], lines[3]])
+    K = len(sub)
+    for slots in (np.repeat(np.arange(K), per_line), np.arange(K * per_line) % K):       # blocks, interleaved
+        N = len(slots)
+        slots_t = np.broadcast_to(slots, (T, N)).copy()
+        obs, masks = _assemble(rng, sub, slots_t, T, B)
+        run = SetRun(N, sub, B, **KW)
+        orcs = [RewardOracle(N, cl, num_beams=B, closed=c, **KW) for cl, c in sub]
+        chg = _changed(slots_t)
+        for t in range(T):
+            g64, g32 = run(obs[t], masks[t], slots_t[t])
+            m = (masks[t] != 0) | chg[t]
+            want = np.zeros(N)
+            for k, o in enumerate(orcs):
+                tot, terms = o.compute_terms(obs[t], m.astype(np.uint8))
+                wk, _ = expected_reward(dm, obs[t], tot, terms, B, KW)
+                want[slots == k] = wk[slots == k]
+            _check_step(g64, g32, want, (B, t))
+        run.rw.close()
 
 
 def _three_lines():
@@ -229,15 +227,14 @@ def _three_lines():
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize('form', ['warp', 'cta'])
-def test_slot_change_restarts_only_the_moved_envs(form, monkeypatch):
+@pytest.mark.parametrize('B', [64, 8192])
+def test_slot_change_restarts_only_the_moved_envs(B):
     """At step 15 a third of the envs move to another line with no reset mask: they restart (their value is a fresh
     reward object's first), the others go on; every step equals the single-line references."""
-    monkeypatch.setenv('F110_REWARD_CTA', '1' if form == 'cta' else '0')
     torch = _torch()
     from f110_gymnasium_ros2_jazzy_b200 import ShapedReward
     lines = _three_lines()
-    K, N, T, B, tc = len(lines), 12, 30, 64, 15
+    K, N, T, tc = len(lines), 12, 30, 15
     rng = np.random.default_rng(5)
     slots = np.arange(N) % K
     moved = np.arange(N) % 3 == 1
@@ -248,7 +245,7 @@ def test_slot_change_restarts_only_the_moved_envs(form, monkeypatch):
     want = _single_refs(lines, N, B, obs, None, slots_t, **KW)
     for t in range(T):
         g64, g32 = run(obs[t], None, slots_t[t])
-        _check_step(g64, g32, want[t], (form, t))
+        _check_step(g64, g32, want[t], t)
         if t == tc:
             fresh = [ShapedReward(N, cl, num_beams=B, closed=c, **KW) for cl, c in lines]
             first = np.choose(slots_t[t], [f(torch.from_numpy(obs[t]).cuda()).cpu().numpy() for f in fresh])
@@ -260,14 +257,13 @@ def test_slot_change_restarts_only_the_moved_envs(form, monkeypatch):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize('form', ['warp', 'cta'])
-def test_out_of_range_slot_leaves_the_record(form, monkeypatch):
+@pytest.mark.parametrize('B', [64, 8192])
+def test_out_of_range_slot_leaves_the_record(B):
     """At step 8 every env has a slot outside [0, K) (-1, K, INT32_MAX): NaN in both outputs.  Back on a valid slot, each
     env goes on exactly as a set that never saw that call -- which counts a return to another line as a slot change."""
-    monkeypatch.setenv('F110_REWARD_CTA', '1' if form == 'cta' else '0')
     _torch()
     lines = _three_lines()
-    K, N, T, B, tb = len(lines), 12, 20, 64, 8
+    K, N, T, tb = len(lines), 12, 20, 8
     rng = np.random.default_rng(8)
     slots = np.arange(N) % K
     slots_t = np.broadcast_to(slots, (T, N)).copy()
@@ -284,24 +280,23 @@ def test_out_of_range_slot_leaves_the_record(form, monkeypatch):
             assert np.isnan(ga64).all() and np.isnan(ga32).all()
             continue
         gb64, gb32 = b(obs[t], masks[t], slots_t[t])
-        assert np.array_equal(ga64.view(np.int64), gb64.view(np.int64)) and np.array_equal(ga32.view(np.int32), gb32.view(np.int32)), (form, t)
-        _check_step(gb64, gb32, want[j], (form, t))
+        assert np.array_equal(ga64.view(np.int64), gb64.view(np.int64)) and np.array_equal(ga32.view(np.int32), gb32.view(np.int32)), t
+        _check_step(gb64, gb32, want[j], t)
         j += 1
     a.rw.close(); b.rw.close()
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize('form', ['warp', 'cta'])
-def test_set_of_one_is_the_single_reward(form, monkeypatch):
+@pytest.mark.parametrize('B', [1080, 8192])
+def test_set_of_one_is_the_single_reward(B):
     """f110_reward_create_set with one line equals f110_reward_create bit for bit, through f110_reward_compute_slots with
     no slots and with slots that would be out of range (a set of one does not read them).  On a set of two,
     f110_reward_compute and f110_reward_compute_slots without slots refuse."""
-    monkeypatch.setenv('F110_REWARD_CTA', '1' if form == 'cta' else '0')
     torch = _torch()
     from f110_gymnasium_ros2_jazzy_b200 import ShapedReward, _lib
     L = _lib.load()
     sh = H.load('reward')['centerline']
-    N, T, B = 8, 12, 1080
+    N, T = 8, 12
     obs, masks = episodes(np.random.default_rng(2), sh[:, :2], True, N, T, B)
     one = ShapedReward(N, sh, num_beams=B, **KW)
     sets = [ShapedReward(N, centerlines=[sh], num_beams=B, **KW) for _ in range(2)]
