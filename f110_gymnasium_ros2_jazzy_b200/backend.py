@@ -108,23 +108,13 @@ class BatchSim(object):
                                                  s.ctypes.data_as(C.c_void_p)))
 
     def set_map_arrays(self, dt, resolution, origin):
-        dt = np.ascontiguousarray(dt, np.float64)
-        # orig_s / orig_c are numpy-evaluated on the host like laser_models.py:421-422
-        _lib.check(self.lib.f110_set_map(self.h, dt.ctypes.data_as(C.c_void_p), dt.shape[0], dt.shape[1],
-                                         float(resolution), float(origin[0]), float(origin[1]),
-                                         float(np.cos(origin[2])), float(np.sin(origin[2]))))
-        self.map_shape = dt.shape
-        self.map_shapes = None
+        """One map from its distance transform (any dtype, converted to float64): the set of one."""
+        self.set_maps([(np.asarray(dt, np.float64), resolution, origin)])
 
     def set_map_image(self, free_mask, resolution, origin):
         """Map from the binarised image (non-zero = free, row 0 = bottom row): the EDT runs on the device
         (f110_set_map_image) and reproduces resolution * scipy.ndimage.distance_transform_edt(img) bit for bit."""
-        m = np.ascontiguousarray(np.asarray(free_mask) != 0, np.uint8)
-        _lib.check(self.lib.f110_set_map_image(self.h, m.ctypes.data_as(C.c_void_p), m.shape[0], m.shape[1],
-                                               float(resolution), float(origin[0]), float(origin[1]),
-                                               float(np.cos(origin[2])), float(np.sin(origin[2]))))
-        self.map_shape = m.shape
-        self.map_shapes = None
+        self.set_maps([(np.asarray(free_mask) != 0, resolution, origin)])
 
     def edt_kernel_ms(self):
         """Device time of the EDT kernels of the last set_map_image call (CUDA events)."""
@@ -132,8 +122,7 @@ class BatchSim(object):
 
     def get_map(self, slot=0):
         """The fp64 map of `slot` (0 for a single map) as the device holds it."""
-        shape = self.map_shapes[slot] if getattr(self, 'map_shapes', None) else self.map_shape
-        dt = np.empty(shape, np.float64)
+        dt = np.empty(self.map_shapes[slot], np.float64)
         _lib.check(self.lib.f110_get_map_slot(self.h, int(slot), dt.ctypes.data_as(C.c_void_p), dt.size))
         return dt
 
@@ -146,7 +135,8 @@ class BatchSim(object):
         """Installs a map set (f110_set_maps): env e then drives on map floor(e * K / N) until set_env_maps says otherwise.
         Each spec is a yaml path (loaded like set_map: scipy's EDT on the host, or the device EDT with edt='device'), a
         (dt float64 [H, W], resolution, origin) tuple, or a (free_mask bool / uint8 [H, W], resolution, origin) tuple (device
-        EDT).  ShapedReward(centerlines=[...]) with one centerline per map scores each env on the line of its slot."""
+        EDT).  ShapedReward(centerlines=[...]) with one centerline per map scores each env on the line of its slot.
+        Every other map setter installs the set of one map through here."""
         from .maps import load_map_image
         descs, keep, shapes = (_lib.F110MapDesc * len(specs))(), [], []
         for k, spec in enumerate(specs):
@@ -161,7 +151,8 @@ class BatchSim(object):
                 a = np.ascontiguousarray(arr)
                 d.dt = a.ctypes.data
             elif arr.dtype in (np.bool_, np.uint8):
-                a = np.ascontiguousarray(arr != 0, np.uint8)
+                # numpy stores a bool as one byte 0 / 1: a bool mask goes to the library as it is, without another pass
+                a = np.ascontiguousarray(arr if arr.dtype == np.bool_ else arr != 0).view(np.uint8)
                 d.free_mask = a.ctypes.data
             else:
                 raise ValueError("map %d: a distance transform must be float64, a free mask bool or uint8 (got %s)" % (k, arr.dtype))
@@ -173,7 +164,6 @@ class BatchSim(object):
             shapes.append(a.shape)
         _lib.check(self.lib.f110_set_maps(self.h, descs, len(specs)))
         self.map_shapes = shapes
-        self.map_shape = shapes[0]
 
     def set_env_maps(self, slots, env_mask=None):
         """Each (masked) env's map slot.  numpy / list input: validated on the host first -- a slot outside
@@ -207,12 +197,8 @@ class BatchSim(object):
         return out
 
     def set_map(self, map_path, map_ext, edt='host'):
-        """edt='host': scipy on the host, as the reference; edt='device': f110_set_map_image."""
-        if edt == 'device':
-            from .maps import load_map_image
-            self.set_map_image(*load_map_image(map_path, map_ext))
-        else:
-            self.set_map_arrays(*load_map(map_path, map_ext))
+        """edt='host': scipy on the host, as the reference; edt='device': the device EDT, as set_map_image."""
+        self.set_maps([map_path], edt=edt, map_ext=map_ext)
 
     def update_params(self, params, agent_idx=-1):
         pv = params_vector(params)

@@ -57,12 +57,10 @@ struct F110Sim {
     SimConst c;
     SimState st;
     StepScratch sc;
-    MapView map;
-    bool map_set = false;
+    MapView map;                  // the maps' common view: slot 0's, with min_positive over all of them
     int64_t map_generation = 0;   // bumped by every set_map / set_maps: a CUDA graph captured before holds the old map by value
-    int32_t map_count = 0;        // maps installed: 0 before any, 1 for a single map, K for a set
-    bool maps_mode = false;       // a set of K >= 2 maps is installed: the *_maps kernels run, `map` is the set's common view
-    MapSet ms;                    // the set's device descriptors (valid while maps_mode)
+    int32_t map_count = 0;        // maps installed, 0 before any; the *_maps kernels run for K >= 2, the single-map ones for 1
+    MapSet ms;                    // the maps' device descriptors (passed to the kernels for K >= 2)
     std::vector<MapView> h_views; // [K] host copies of ms.views: the direction tables are rebuilt from them
     bool count_lookups = false;
     bool narrow_fraction = false;
@@ -71,12 +69,12 @@ struct F110Sim {
     char* state_blob = nullptr;   size_t state_bytes = 0;    // checkpointable
     char* scratch_blob = nullptr; size_t scratch_bytes = 0;
     double* d_tables = nullptr;   // params[A][18], sim_params[18], sines, cosines, scan_angles, beam_cos, side_dist
-    double* d_map = nullptr;      // the padded map, or the K padded maps of a set back to back
-    double2* d_lidar_tables = nullptr;   // beam_tt[B], dir_fx[theta_dis]
-    MapView* d_views = nullptr;   // [K] a set's per-slot views
-    double2* d_map_dir = nullptr; // [K][theta_dis] a set's direction tables
-    int32_t* d_env_map = nullptr; // [N] slot of each env (all 0 unless a set is installed)
-    std::vector<double> h_sines, h_cosines;   // host copies: dir_fx is rebuilt from them whenever the map changes
+    double* d_map = nullptr;      // the K padded maps back to back
+    double2* d_beam_tt = nullptr; // [B] beam_tt
+    MapView* d_views = nullptr;   // [K] per-slot views
+    double2* d_map_dir = nullptr; // [K][theta_dis] direction tables; slot 0's is c.dir_fx
+    int32_t* d_env_map = nullptr; // [N] slot of each env (all 0 for one map)
+    std::vector<double> h_sines, h_cosines;   // host copies: the direction tables are rebuilt from them whenever a map changes
     // host-buffer path (f110_step_host)
     cudaStream_t host_stream = nullptr;
     char* io_blob = nullptr; size_t io_bytes = 0;
@@ -151,7 +149,7 @@ struct Guard {   // selects the handle's device for the duration of a call
 
 int check_step_io(const F110Sim* sim, const F110StepIO* io) {
     if (!sim || !io) return fail(F110_ERR_INVALID, "null handle or io");
-    if (!sim->map_set) return fail(F110_ERR_MAP_NOT_SET, "Map is not set for scan simulator.");
+    if (sim->map_count == 0) return fail(F110_ERR_MAP_NOT_SET, "Map is not set for scan simulator.");
     if (io->reset_mask && !io->reset_poses) return fail(F110_ERR_INVALID, "reset_mask given without reset_poses");
     return F110_OK;
 }
@@ -174,7 +172,7 @@ int run_step(F110Sim* sim, const F110StepIO& io, cudaStream_t s) {
         const cudaError_t de = cudaStreamSynchronize(s);                                                           \
         if (de != cudaSuccess) return fail(F110_ERR_CUDA, "%s: %s", name, cudaGetErrorString(de));                 \
     }
-    const MapSet* ms = sim->maps_mode ? &sim->ms : nullptr;
+    const MapSet* ms = sim->map_count >= 2 ? &sim->ms : nullptr;
     CUDA_TRY(launch_dynamics(sim->c, sim->map, sim->st, sim->sc, io, ms, s));
     DEBUG_SYNC("dynamics_kernel")
     if (sim->timing) CUDA_TRY(cudaEventRecord(e[1], s));
@@ -265,8 +263,8 @@ int f110_create(const F110Config* cfg, const double* params, F110Sim** out) {
     if (e == cudaSuccess) e = cudaMemset(sim->state_blob, 0, sim->state_bytes);
     if (e == cudaSuccess) e = cudaMemset(sim->scratch_blob, 0, sim->scratch_bytes);
     if (e == cudaSuccess) e = cudaMemset(sim->d_tables, 0, ntab * sizeof(double));
-    if (e == cudaSuccess) e = cudaMalloc(&sim->d_lidar_tables, ((size_t)B + cfg->theta_dis) * sizeof(double2));
-    if (e == cudaSuccess) e = cudaMemset(sim->d_lidar_tables, 0, ((size_t)B + cfg->theta_dis) * sizeof(double2));
+    if (e == cudaSuccess) e = cudaMalloc(&sim->d_beam_tt, (size_t)B * sizeof(double2));
+    if (e == cudaSuccess) e = cudaMemset(sim->d_beam_tt, 0, (size_t)B * sizeof(double2));
     if (e == cudaSuccess) e = cudaMalloc(&sim->d_env_map, (size_t)N * sizeof(int32_t));
     if (e == cudaSuccess) e = cudaMemset(sim->d_env_map, 0, (size_t)N * sizeof(int32_t));
     if (e == cudaSuccess) {
@@ -327,9 +325,8 @@ int f110_create(const F110Config* cfg, const double* params, F110Sim** out) {
     c.scan_angles = t; t += B;
     c.beam_cos = t; t += B;
     c.side_dist = t; t += B;
-    c.beam_tt = sim->d_lidar_tables;
+    c.beam_tt = sim->d_beam_tt;
     c.ttc_side_max = INFINITY; c.ttc_cos_max = INFINITY;
-    c.dir_fx = sim->d_lidar_tables + B;
     sim->h_sines.assign(cfg->theta_dis, 0.0); sim->h_cosines.assign(cfg->theta_dis, 1.0);
 
     std::vector<double> hp((size_t)(A + 1) * F110_NUM_PARAMS);
@@ -351,7 +348,7 @@ void f110_destroy(F110Sim* sim) {
     if (!sim) return;
     Guard g(sim->cfg.device);
     if (sim->host_stream) { cudaStreamSynchronize(sim->host_stream); cudaStreamDestroy(sim->host_stream); }
-    cudaFree(sim->state_blob); cudaFree(sim->scratch_blob); cudaFree(sim->d_tables); cudaFree(sim->d_map); cudaFree(sim->d_lidar_tables);
+    cudaFree(sim->state_blob); cudaFree(sim->scratch_blob); cudaFree(sim->d_tables); cudaFree(sim->d_map); cudaFree(sim->d_beam_tt);
     cudaFree(sim->d_views); cudaFree(sim->d_map_dir); cudaFree(sim->d_env_map);
     cudaFree(sim->io_blob);
     edt_scratch_free(&sim->edt);
@@ -359,31 +356,20 @@ void f110_destroy(F110Sim* sim) {
     delete sim;
 }
 
-// The lidar kernel's direction table of one map: table direction k rotated into the map frame and scaled to fixed-point
-// cells per metre.  Depends on the sin / cos tables and on the map (origin yaw, resolution, fraction bits).
-static void direction_table(const F110Sim* sim, const MapView& m, double2* dir) {
+// The lidar kernel's direction tables [K][theta_dis] of the maps `views`: table direction k rotated into each map's frame and
+// scaled to fixed-point cells per metre.  Depend on the sin / cos tables and on each map (origin yaw, resolution, fraction bits).
+static std::vector<double2> direction_tables(const F110Sim* sim, const std::vector<MapView>& views) {
     const size_t n = sim->h_sines.size();
-    for (size_t k = 0; k < n; ++k) {
-        const double cs = sim->h_cosines[k], sn = sim->h_sines[k];
-        dir[k].x = (cs * m.oc + sn * m.os) * m.inv_fx;
-        dir[k].y = (-cs * m.os + sn * m.oc) * m.inv_fx;
+    std::vector<double2> dir(n * views.size());
+    for (size_t v = 0; v < views.size(); ++v) {
+        const MapView& m = views[v];
+        for (size_t k = 0; k < n; ++k) {
+            const double cs = sim->h_cosines[k], sn = sim->h_sines[k];
+            dir[v * n + k].x = (cs * m.oc + sn * m.os) * m.inv_fx;
+            dir[v * n + k].y = (-cs * m.os + sn * m.oc) * m.inv_fx;
+        }
     }
-}
-
-// Rebuilds the direction table of the map, or of every map of a set (both setters call it).
-static int refresh_direction_table(F110Sim* sim) {
-    if (!sim->map_set) return F110_OK;
-    const size_t n = sim->h_sines.size();
-    if (sim->maps_mode) {
-        std::vector<double2> dir(n * sim->h_views.size());
-        for (size_t k = 0; k < sim->h_views.size(); ++k) direction_table(sim, sim->h_views[k], dir.data() + k * n);
-        CUDA_TRY(cudaMemcpy(sim->d_map_dir, dir.data(), dir.size() * sizeof(double2), cudaMemcpyHostToDevice));
-        return F110_OK;
-    }
-    std::vector<double2> dir(n);
-    direction_table(sim, sim->map, dir.data());
-    CUDA_TRY(cudaMemcpy(const_cast<double2*>(sim->c.dir_fx), dir.data(), n * sizeof(double2), cudaMemcpyHostToDevice));
-    return F110_OK;
+    return dir;
 }
 
 // Fixed-point format of the lidar kernel's fast march for a map whose larger side is `side_cells`: as many fraction bits as
@@ -411,60 +397,6 @@ static void place_map(MapView& m, double* padded, int height, int width, double 
     m.wres = width * resolution; m.hres = height * resolution;   // laser_models.py:79
 }
 
-// Leaves set mode (after a single map replaced the set): frees the set's descriptors, every env back on slot 0
-static void drop_map_set(F110Sim* sim) {
-    cudaFree(sim->d_views); sim->d_views = nullptr;
-    cudaFree(sim->d_map_dir); sim->d_map_dir = nullptr;
-    sim->h_views.clear();
-    memset(&sim->ms, 0, sizeof(sim->ms));
-    if (sim->maps_mode) cudaMemset(sim->d_env_map, 0, (size_t)sim->c.N * sizeof(int32_t));
-    sim->maps_mode = false;
-}
-
-// Installs a DENSE device map [H][W] as the handle's padded map (see MapView) and frees `dense`.
-static int install_map(F110Sim* sim, double* dense, int height, int width, double resolution,
-                       double orig_x, double orig_y, double orig_cos, double orig_sin) {
-    MapView m;
-    memset(&m, 0, sizeof(m));
-    fixed_point_format(sim, (unsigned)(width > height ? width : height), m);
-    const size_t prows = (size_t)m.prows, pitch = (size_t)m.pitch;
-    if ((double)prows * (double)pitch >= 2147483648.0) { cudaFree(dense); return fail(F110_ERR_INVALID, "map too large once padded (%zu x %zu cells)", prows, pitch); }
-    if (map_min_positive(dense, (size_t)height * width, &m.min_positive, sim->host_stream) != cudaSuccess) {
-        cudaFree(dense); cudaGetLastError();
-        return fail(F110_ERR_CUDA, "map scan failed");
-    }
-    double* padded = nullptr;
-    cudaError_t e = cudaMalloc(&padded, prows * pitch * sizeof(double));
-    if (e == cudaSuccess) e = launch_pad_map(dense, height, width, padded, (int)prows, (int)pitch, sim->host_stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(sim->host_stream);
-    cudaFree(dense);
-    if (e != cudaSuccess) { cudaFree(padded); cudaGetLastError(); return fail(F110_ERR_CUDA, "map padding: %s", cudaGetErrorString(e)); }
-    cudaFree(sim->d_map);
-    sim->d_map = padded;
-    drop_map_set(sim);
-    place_map(m, padded, height, width, resolution, orig_x, orig_y, orig_cos, orig_sin);
-    sim->map = m;
-    sim->map_set = true;
-    sim->map_count = 1;
-    sim->map_generation += 1;
-    return refresh_direction_table(sim);
-}
-
-int f110_set_map(F110Sim* sim, const double* dt, int32_t height, int32_t width, double resolution,
-                 double orig_x, double orig_y, double orig_cos, double orig_sin) {
-    if (!sim || !dt || height < 1 || width < 1 || !(resolution > 0)) return fail(F110_ERR_INVALID, "bad map arguments");
-    if ((double)height * width >= 2147483648.0 || height >= 65536 || width >= 65536)
-        return fail(F110_ERR_INVALID, "map too large (need H*W < 2^31 and H, W < 65536)");
-    Guard g(sim->cfg.device);
-    CUDA_TRY(cudaDeviceSynchronize());
-    double* d = nullptr;
-    const size_t bytes = (size_t)height * width * sizeof(double);
-    CUDA_TRY(cudaMalloc(&d, bytes));
-    cudaError_t e = cudaMemcpy(d, dt, bytes, cudaMemcpyHostToDevice);
-    if (e != cudaSuccess) { cudaFree(d); return fail(F110_ERR_CUDA, "map upload: %s", cudaGetErrorString(e)); }
-    return install_map(sim, d, height, width, resolution, orig_x, orig_y, orig_cos, orig_sin);
-}
-
 // The dense fp64 map of a mask through the device EDT: DEVICE [H][W] in *out (caller frees), or an error code
 static int dense_from_mask(F110Sim* sim, const uint8_t* free_mask, int32_t height, int32_t width, double resolution, double** out) {
     const size_t cells = (size_t)height * width;
@@ -482,21 +414,22 @@ static int dense_from_mask(F110Sim* sim, const uint8_t* free_mask, int32_t heigh
     return F110_OK;
 }
 
+int f110_set_map(F110Sim* sim, const double* dt, int32_t height, int32_t width, double resolution,
+                 double orig_x, double orig_y, double orig_cos, double orig_sin) {
+    const F110MapDesc d = { dt, nullptr, height, width, resolution, orig_x, orig_y, orig_cos, orig_sin };
+    return f110_set_maps(sim, &d, 1);
+}
+
 int f110_set_map_image(F110Sim* sim, const uint8_t* free_mask, int32_t height, int32_t width, double resolution,
                        double orig_x, double orig_y, double orig_cos, double orig_sin) {
-    if (!sim || !free_mask || height < 1 || width < 1 || !(resolution > 0)) return fail(F110_ERR_INVALID, "bad map arguments");
-    if ((double)height * width >= 2147483648.0 || height >= 65536 || width >= 65536)
-        return fail(F110_ERR_INVALID, "map too large (need H*W < 2^31 and H, W < 65536)");
-    Guard g(sim->cfg.device);
-    CUDA_TRY(cudaDeviceSynchronize());
-    double* d = nullptr;
-    const int rc = dense_from_mask(sim, free_mask, height, width, resolution, &d);
-    if (rc != F110_OK) return rc;
-    return install_map(sim, d, height, width, resolution, orig_x, orig_y, orig_cos, orig_sin);
+    const F110MapDesc d = { nullptr, free_mask, height, width, resolution, orig_x, orig_y, orig_cos, orig_sin };
+    return f110_set_maps(sim, &d, 1);
 }
 
 float f110_edt_kernel_ms(const F110Sim* sim) { return sim ? sim->edt.kernel_ms : -1.f; }
 
+// The one map installer: a single map is the set of one.  Everything is built aside and committed at the end, so a failure
+// leaves the handle's maps as they were.
 int f110_set_maps(F110Sim* sim, const F110MapDesc* maps, int32_t count) {
     if (!sim || !maps) return fail(F110_ERR_INVALID, "null argument");
     if (count < 1 || count > F110_MAX_MAPS) return fail(F110_ERR_INVALID, "a map set holds 1 to %d maps, not %d", F110_MAX_MAPS, count);
@@ -504,24 +437,19 @@ int f110_set_maps(F110Sim* sim, const F110MapDesc* maps, int32_t count) {
     for (int k = 0; k < count; ++k) {
         const F110MapDesc& d = maps[k];
         if ((!d.dt && !d.free_mask) || d.height < 1 || d.width < 1 || !(d.resolution > 0))
-            return fail(F110_ERR_INVALID, "bad arguments for map %d of the set", k);
+            return fail(F110_ERR_INVALID, "bad arguments for map %d", k);
         if ((double)d.height * d.width >= 2147483648.0 || d.height >= 65536 || d.width >= 65536)
             return fail(F110_ERR_INVALID, "map %d too large (need H*W < 2^31 and H, W < 65536)", k);
         const unsigned s = (unsigned)(d.width > d.height ? d.width : d.height);
         side = s > side ? s : side;
     }
-    if (count == 1) {   // a set of one map is that map
-        const F110MapDesc& d = maps[0];
-        return d.dt ? f110_set_map(sim, d.dt, d.height, d.width, d.resolution, d.orig_x, d.orig_y, d.orig_cos, d.orig_sin)
-                    : f110_set_map_image(sim, d.free_mask, d.height, d.width, d.resolution, d.orig_x, d.orig_y, d.orig_cos, d.orig_sin);
-    }
-    // one fixed-point format for the whole set, that of its largest side; every map padded to it, at a fixed stride
+    // one fixed-point format for all maps, that of the largest side; every map padded to it, at a fixed stride
     MapView common;
     memset(&common, 0, sizeof(common));
     fixed_point_format(sim, side, common);
     const size_t stride = (size_t)common.prows * (size_t)common.pitch;
     if ((double)stride * count >= 2147483648.0)
-        return fail(F110_ERR_INVALID, "map set too large: %d maps padded to %d x %d cells each (the largest side is %u) exceed 2^31 cells",
+        return fail(F110_ERR_INVALID, "maps too large: %d padded to %d x %d cells each (the largest side is %u) reach 2^31 cells",
                     count, common.prows, common.pitch, side);
     Guard g(sim->cfg.device);
     CUDA_TRY(cudaDeviceSynchronize());
@@ -533,7 +461,7 @@ int f110_set_maps(F110Sim* sim, const F110MapDesc* maps, int32_t count) {
     if (e == cudaSuccess) e = cudaMalloc(&d_views, (size_t)count * sizeof(MapView));
     if (e == cudaSuccess) e = cudaMalloc(&d_dir, (size_t)count * nt * sizeof(double2));
     auto undo = [&]() { cudaFree(padded); cudaFree(d_views); cudaFree(d_dir); cudaGetLastError(); };
-    if (e != cudaSuccess) { undo(); return fail(F110_ERR_CUDA, "map set allocation (%d x %zu cells): %s", count, stride, cudaGetErrorString(e)); }
+    if (e != cudaSuccess) { undo(); return fail(F110_ERR_CUDA, "map allocation (%d x %zu cells): %s", count, stride, cudaGetErrorString(e)); }
     std::vector<MapView> views(count, common);
     double min_positive = INFINITY;
     for (int k = 0; k < count; ++k) {
@@ -558,27 +486,25 @@ int f110_set_maps(F110Sim* sim, const F110MapDesc* maps, int32_t count) {
         place_map(v, block, d.height, d.width, d.resolution, d.orig_x, d.orig_y, d.orig_cos, d.orig_sin);
         min_positive = v.min_positive < min_positive ? v.min_positive : min_positive;
     }
-    std::vector<double2> dir(nt * count);
-    for (int k = 0; k < count; ++k) direction_table(sim, views[k], dir.data() + (size_t)k * nt);
+    const std::vector<double2> dir = direction_tables(sim, views);
     e = cudaMemcpy(d_views, views.data(), views.size() * sizeof(MapView), cudaMemcpyHostToDevice);
     if (e == cudaSuccess) e = cudaMemcpy(d_dir, dir.data(), dir.size() * sizeof(double2), cudaMemcpyHostToDevice);
     // every env to its contiguous block: env e drives on slot floor(e K / N)
     std::vector<int32_t> slots(sim->c.N);
     for (int n = 0; n < sim->c.N; ++n) slots[n] = (int32_t)((int64_t)n * count / sim->c.N);
     if (e == cudaSuccess) e = cudaMemcpy(sim->d_env_map, slots.data(), slots.size() * sizeof(int32_t), cudaMemcpyHostToDevice);
-    if (e != cudaSuccess) { undo(); return fail(F110_ERR_CUDA, "map set upload: %s", cudaGetErrorString(e)); }
+    if (e != cudaSuccess) { undo(); return fail(F110_ERR_CUDA, "map upload: %s", cudaGetErrorString(e)); }
     // commit
     cudaFree(sim->d_map); cudaFree(sim->d_views); cudaFree(sim->d_map_dir);
     sim->d_map = padded; sim->d_views = d_views; sim->d_map_dir = d_dir;
     sim->h_views = views;
     sim->map = views[0];
     sim->map.min_positive = min_positive;
+    sim->c.dir_fx = d_dir;   // slot 0's table, which the single-map kernels read
     sim->ms.env_map = sim->d_env_map;
     sim->ms.views = d_views;
     sim->ms.dir_fx = d_dir;
     sim->ms.stride = stride;
-    sim->maps_mode = true;
-    sim->map_set = true;
     sim->map_count = count;
     sim->map_generation += 1;
     return F110_OK;
@@ -588,9 +514,9 @@ int32_t f110_map_count(const F110Sim* sim) { return sim ? sim->map_count : 0; }
 
 int f110_get_map_slot(F110Sim* sim, int32_t slot, double* dt_host, int64_t capacity_cells) {
     if (!sim || !dt_host) return fail(F110_ERR_INVALID, "null argument");
-    if (!sim->map_set) return fail(F110_ERR_MAP_NOT_SET, "Map is not set for scan simulator.");
+    if (sim->map_count == 0) return fail(F110_ERR_MAP_NOT_SET, "Map is not set for scan simulator.");
     if (slot < 0 || slot >= sim->map_count) return fail(F110_ERR_INDEX, "map slot %d out of range (%d maps)", slot, sim->map_count);
-    const MapView& m = sim->maps_mode ? sim->h_views[slot] : sim->map;
+    const MapView& m = sim->h_views[slot];
     const size_t cells = (size_t)m.H * m.W;
     if ((size_t)capacity_cells < cells) return fail(F110_ERR_INVALID, "buffer too small for %d x %d cells", m.H, m.W);
     Guard g(sim->cfg.device);
@@ -647,7 +573,9 @@ int f110_set_tables(F110Sim* sim, const double* sines, const double* cosines) {
     CUDA_TRY(cudaMemcpy(const_cast<double*>(sim->c.cosines), cosines, n, cudaMemcpyHostToDevice));
     sim->h_sines.assign(sines, sines + sim->cfg.theta_dis);
     sim->h_cosines.assign(cosines, cosines + sim->cfg.theta_dis);
-    return refresh_direction_table(sim);
+    const std::vector<double2> dir = direction_tables(sim, sim->h_views);   // empty before any map
+    if (!dir.empty()) CUDA_TRY(cudaMemcpy(sim->d_map_dir, dir.data(), dir.size() * sizeof(double2), cudaMemcpyHostToDevice));
+    return F110_OK;
 }
 
 int f110_set_beam_tables(F110Sim* sim, const double* scan_angles, const double* beam_cosines, const double* side_distances) {

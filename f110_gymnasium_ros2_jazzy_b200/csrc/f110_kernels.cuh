@@ -43,7 +43,7 @@ struct MapView {
 struct MapSet {
     const int32_t* env_map;   // [N] slot of each env
     const MapView* views;     // [K] per-slot descriptors
-    const double2* dir_fx;    // [K][theta_dis] slot k's direction table (as SimConst::dir_fx for a single map)
+    const double2* dir_fx;    // [K][theta_dis] slot k's direction table (SimConst::dir_fx is slot 0's)
     size_t stride;            // cells between the blocks of two consecutive slots
 };
 
@@ -125,7 +125,8 @@ struct SimConst {
     const double2* beam_tt;    // [B] (beam_cos, side_dist) interleaved for the lidar kernel
     double ttc_side_max, ttc_cos_max;   // max side_dist, max |beam_cos| (+inf until the beam tables are set: nothing is pre-filtered)
     const double2* dir_fx;     // [theta_dis] table direction k rotated into the map frame and scaled to fixed point:
-                               //   ((cos*oc + sin*os) * inv_fx, (-cos*os + sin*oc) * inv_fy); rebuilt by set_map / set_tables
+                               //   ((cos*oc + sin*os) * inv_fx, (-cos*os + sin*oc) * inv_fy); slot 0's table of
+                               //   MapSet::dir_fx, rebuilt by set_map(s) / set_tables
 };
 
 // ms == nullptr: the handle holds one map (m); otherwise m is the set's common view (slot 0's, min_positive over the set)

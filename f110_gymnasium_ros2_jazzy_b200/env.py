@@ -212,6 +212,18 @@ class F110Env(gym.Env):
             self.sim.backend.close()
 
 
+def _map_specs(map_dir=None, map=None, map_arrays=None, maps=None):
+    """The vector envs' map arguments as one BatchSim.set_maps spec list: one map is the set of one."""
+    if maps is not None:
+        if map is not None or map_arrays is not None:
+            raise ValueError("give either maps= (a map set) or map= / map_arrays= (one map), not both")
+        return maps
+    if map_arrays is not None:
+        dt, resolution, origin = map_arrays
+        return [(np.asarray(dt, np.float64), resolution, origin)]
+    return [map_dir + map + '.yaml']
+
+
 class F110VecEnv(object):
     """N F110Envs stepped as one batch on one GPU; torch CUDA tensors in and out (zero-copy).
 
@@ -230,8 +242,7 @@ class F110VecEnv(object):
                  timestep=0.01, ego_idx=0, integrator=Integrator.RK4, lidar_dist=0.0, device=None, auto_reset=True,
                  outputs=FAST_OUTPUTS, noise_std=0.01, num_beams=1080, fov=4.7, count_lookups=False, map_arrays=None,
                  cuda_graph=False, maps=None, env_maps=None):
-        if maps is not None and (map is not None or map_arrays is not None):
-            raise ValueError("give either maps= (a map set) or map= / map_arrays= (one map), not both")
+        specs = _map_specs(map_dir, map, map_arrays, maps)
         self.num_envs, self.num_agents = num_envs, num_agents
         self.timestep = timestep
         self.auto_reset = auto_reset
@@ -239,14 +250,9 @@ class F110VecEnv(object):
         self.backend = BatchSim(num_envs, num_agents, params=params, seed=seed, timestep=timestep, integrator=integrator,
                                 ego_idx=ego_idx, lidar_dist=lidar_dist, noise_std=noise_std, device=device, outputs=outs,
                                 num_beams=num_beams, fov=fov, count_lookups=count_lookups)
-        if maps is not None:
-            self.backend.set_maps(maps, map_ext=map_ext)
-            if env_maps is not None:
-                self.backend.set_env_maps(env_maps)
-        elif map_arrays is not None:
-            self.backend.set_map_arrays(*map_arrays)
-        else:
-            self.backend.set_map(map_dir + map + '.yaml', map_ext)
+        self.backend.set_maps(specs, map_ext=map_ext)
+        if maps is not None and env_maps is not None:
+            self.backend.set_env_maps(env_maps)
         self.device = self.backend.device
         self.start_poses = None
         self.truncated = torch.zeros(num_envs, dtype=torch.uint8, device=self.device)
@@ -273,7 +279,7 @@ class F110VecEnv(object):
     def step(self, actions, noise=None):
         o = self.backend.out
         if self._graph is not None and self._map_generation != self.backend.map_generation:
-            self._drop_graph()      # the map was changed behind the env's back (backend.set_map*): see set_map
+            self._drop_graph()      # the map was changed behind the env's back (backend.set_map*): see set_maps
         if self.cuda_graph and noise is None and self.auto_reset and self.start_poses is not None:
             self._act.copy_(torch.as_tensor(actions, device=self.device).reshape(self._act.shape))
             if self._graph is None and self._steps_eager >= 1:
@@ -300,18 +306,15 @@ class F110VecEnv(object):
         return o['obs'], o['reward'], o['terminated'], self.truncated, o
 
     def set_map(self, map_path, map_ext, edt='host'):
-        """update_map for the whole batch.  The step kernels receive the map descriptor by value, so a captured CUDA graph
-        still holds the previous (freed) map: it is dropped here and re-captured by the next steps."""
-        self.backend.set_map(map_path, map_ext, edt=edt)
-        self._drop_graph()
+        """update_map for the whole batch: the set of one map (set_maps)."""
+        self.set_maps([map_path], edt=edt, map_ext=map_ext)
 
     def set_map_arrays(self, dt, resolution, origin):
-        self.backend.set_map_arrays(dt, resolution, origin)
-        self._drop_graph()
+        self.set_maps(_map_specs(map_arrays=(dt, resolution, origin)))
 
     def set_maps(self, specs, edt='host', map_ext='.png'):
-        """Installs a map set for the whole batch (BatchSim.set_maps; env e on slot floor(e * K / N)); like set_map it drops a
-        captured CUDA graph."""
+        """Installs a map set for the whole batch (BatchSim.set_maps; env e on slot floor(e * K / N)).  A captured CUDA graph
+        holds the previous (freed) map by value: it is dropped here and re-captured by the next steps."""
         self.backend.set_maps(specs, edt=edt, map_ext=map_ext)
         self._drop_graph()
 
@@ -380,8 +383,7 @@ class F110HostVecEnv(object):
 
     def __init__(self, num_envs, chunks=2, map_arrays=None, map_dir=None, map=None, map_ext='.png', num_agents=1,
                  seed=42, device=None, outputs=FAST_OUTPUTS, num_beams=1080, maps=None, env_maps=None, **kw):
-        if maps is not None and (map is not None or map_arrays is not None):
-            raise ValueError("give either maps= (a map set) or map= / map_arrays= (one map), not both")
+        specs = _map_specs(map_dir, map, map_arrays, maps)
         self.num_envs, self.num_agents, self.num_beams = num_envs, num_agents, num_beams
         if maps is not None:
             # the whole batch's assignment (F110VecEnv's default: env e on slot floor(e K / N)); each chunk gets its slice
@@ -398,13 +400,9 @@ class F110HostVecEnv(object):
             n = self.bounds[k + 1] - self.bounds[k]
             b = BatchSim(n, num_agents, seed=seed + 7919 * k, device=device, outputs=('obs',), num_beams=num_beams,
                          host_stream_rank=k + 1, **kw)
+            b.set_maps(specs, map_ext=map_ext)
             if maps is not None:
-                b.set_maps(maps, map_ext=map_ext)
                 b.set_env_maps(slots[self.bounds[k]:self.bounds[k + 1]])
-            elif map_arrays is not None:
-                b.set_map_arrays(*map_arrays)
-            else:
-                b.set_map(map_dir + map + '.yaml', map_ext)
             self.parts.append(b)
         outs = tuple(dict.fromkeys(tuple(outputs) + ('obs', 'reward', 'terminated')))
         from .backend import _OUT_SPECS

@@ -144,7 +144,9 @@ int f110_create(const F110Config* cfg, const double* params, F110Sim** out);
 void f110_destroy(F110Sim* sim);
 
 /* dt: HOST [height][width] fp64 = resolution * EDT(binarised, bottom-up image) exactly as
- * laser_models.py:398-425 builds it; orig_cos/orig_sin = cos/sin(origin yaw) as computed by the host. */
+ * laser_models.py:398-425 builds it; orig_cos/orig_sin = cos/sin(origin yaw) as computed by the host.
+ * The map set of this one map (f110_set_maps with count 1), and so atomic like it: it replaces whatever map or set the
+ * handle held, and afterwards every env is on slot 0. */
 int f110_set_map(F110Sim* sim, const double* dt, int32_t height, int32_t width, double resolution,
                  double orig_x, double orig_y, double orig_cos, double orig_sin);
 /* The same from the binarised image itself: free_mask HOST uint8 [height][width], non-zero = free (pixel > 128), row 0 =
@@ -175,10 +177,10 @@ typedef struct F110MapDesc {
 /* Installs `count` (1 .. F110_MAX_MAPS) maps at once; maps may differ in size, resolution and origin.  Afterwards env e
  * drives on slot floor(e * count / N) (contiguous blocks, which keep the lidar kernel's home-segment locality).  Atomic: on
  * any failure (F110_ERR_INVALID for bad arguments or a set too large, F110_ERR_CUDA for out of memory) the handle keeps
- * the map or maps it had.  Bumps f110_map_generation.  A set of one map is f110_set_map / f110_set_map_image of that map,
- * and f110_set_map / f110_set_map_image on a handle holding a set replace the set with that one map. */
+ * the map or maps it had.  Bumps f110_map_generation.  f110_set_map and f110_set_map_image install the set of one map;
+ * a step on one map runs the single-map kernels (f110_get_lidar_variant reports out[3] = 0). */
 int f110_set_maps(F110Sim* sim, const F110MapDesc* maps, int32_t count);
-/* Maps installed: 1 for a single map, 0 before any. */
+/* Maps installed by the last f110_set_map / f110_set_map_image / f110_set_maps: 1 for a single map, 0 before any. */
 int32_t f110_map_count(const F110Sim* sim);
 /* Reads map `slot` back like f110_get_map; slot outside [0, f110_map_count) -> F110_ERR_INDEX. */
 int f110_get_map_slot(F110Sim* sim, int32_t slot, double* dt_host, int64_t capacity_cells);

@@ -337,9 +337,11 @@ def test_set_construction_limits_and_slots():
     gen = sim.map_generation
     tiny = (np.full((4, 4), 0.5), 0.05, [0.0, 0.0, 0.0])
     wide = (np.full((1, 4096), 0.5), 0.05, [0.0, 0.0, 0.0])   # pads every member to 8192 x 8208 cells: 32 exceed 2^31
-    for specs in ([], [tiny] * (_lib.F110_MAX_MAPS + 1), [wide] * 32):
+    huge = (np.full((1, 40000), 0.5), 0.05, [0.0, 0.0, 0.0])  # pads to 65536 x 65552 cells: alone beyond 2^31
+    for install in (lambda: sim.set_maps([]), lambda: sim.set_maps([tiny] * (_lib.F110_MAX_MAPS + 1)),
+                    lambda: sim.set_maps([wide] * 32), lambda: sim.set_maps([huge]), lambda: sim.set_map_arrays(*huge)):
         with pytest.raises(ValueError):
-            sim.set_maps(specs)
+            install()
         assert sim.num_maps == 1 and sim.map_generation == gen
         assert np.array_equal(_scan_once(sim, poses), first)
     # back to one map: f110_set_map after a set gives what a fresh single-map handle gives
@@ -349,6 +351,59 @@ def test_set_construction_limits_and_slots():
     assert sim.num_maps == 1 and np.array_equal(sim.env_maps().cpu().numpy(), np.zeros(len(poses)))
     assert np.array_equal(_scan_once(sim, poses), first)
     sim.close()
+
+
+@pytest.mark.gpu
+def test_a_set_of_one_is_the_single_map():
+    """The rotated-origin Shanghai map installed four ways -- set_maps of its dt, set_map_arrays, set_map_image and set_maps
+    of its free mask -- gives one map_generation bump, one map, all slots 0, the same map and the single-map kernel each, and
+    bit-identical outputs over a 40-step rollout.  set_tables after a set of one rebuilds its direction table: the scans then
+    equal those of a fresh handle given the same tables before its map."""
+    torch = _torch()
+    free, res, _ = _golden_free('Shanghai_map')
+    dt = H.golden_map('Shanghai_map')[0]
+    gr = H.load('scans_rotated')
+    origin = [float(v) for v in gr['origin']]
+    N = len(gr['poses'])
+    poses = torch.as_tensor(gr['poses'][:, None, :], device='cuda')
+    installs = {'set_maps(dt)': lambda s: s.set_maps([(dt, res, origin)]),
+                'set_map_arrays': lambda s: s.set_map_arrays(dt, res, origin),
+                'set_map_image': lambda s: s.set_map_image(free, res, origin),
+                'set_maps(mask)': lambda s: s.set_maps([(free, res, origin)])}
+    gen = torch.Generator(device='cuda').manual_seed(6)
+    acts = [torch.rand((N, 1, 2), generator=gen, device='cuda') * torch.tensor([0.8, 6.0], device='cuda')
+            + torch.tensor([-0.4, 0.0], device='cuda') for _ in range(40)]
+    want = None
+    for name, install in installs.items():
+        sim = _sim(N)
+        gen0 = sim.map_generation
+        install(sim)
+        assert sim.map_generation == gen0 + 1 and sim.num_maps == 1, name
+        assert np.array_equal(sim.get_map(0), dt), name
+        assert not sim.env_maps().cpu().numpy().any(), name
+        outs = [{k: v.clone() for k, v in sim.reset(poses).items()}]
+        for a in acts:
+            sim.step(a, None, reset_mask=sim.out['terminated'], reset_poses=poses)
+            outs.append({k: v.clone() for k, v in sim.out.items()})
+        assert sim.lidar_variant()['maps'] == 0, name
+        want = outs if want is None else want
+        for t, (o, w) in enumerate(zip(outs, want)):
+            for k in o:
+                assert _eq(o[k], w[k]), (name, t, k)
+        sim.close()
+    s, c = H.tables()[:2]
+    s2, c2 = np.roll(s, 100), np.roll(c, 100)      # every table direction turned by 100 entries
+    sim = _sim(N)
+    sim.set_maps([(dt, res, origin)])
+    before = _scan_once(sim, gr['poses'])
+    sim.set_tables(s2, c2)
+    fresh = _sim(N)
+    fresh.set_tables(s2, c2)
+    fresh.set_maps([(dt, res, origin)])
+    after = _scan_once(sim, gr['poses'])
+    assert np.array_equal(after, _scan_once(fresh, gr['poses']))
+    assert not np.array_equal(after, before)
+    sim.close(); fresh.close()
 
 
 @pytest.mark.gpu
